@@ -33,6 +33,7 @@ sys.path.insert(0, ROOT)
 LEVELS = os.path.join(ROOT, "tests", "levels")
 ENVS_PER_GPU = int(os.environ.get("MJB_BENCH_ENVS", "4096"))
 SETTLE = int(os.environ.get("MJB_BENCH_SETTLE", "300"))
+DUMP_LIMIT = 64 << 20   # bytes of --dump-outputs files in all
 WORKLOAD = "C2: MultiAgentModel.xml, 2 agents, Language + tag-distance reward + done, ctrl mode, skipFrames=1"
 L2_NOTE = "flushed between steps (256 MiB write, outside the per-step events)"
 
@@ -76,6 +77,22 @@ def literal_bytes_per_env_step(nq, nv, nu, nsens, n_agents, act_dim, obs_dim, np
     read = 4 * (nq + nv + nu + nsens + n_agents * act_dim + 4 * nprobe + 1) + store
     write = 4 * (n_agents * obs_dim + (nv if free_joint else nu) + n_agents + 1) + 2 * (n_agents + 1) + store
     return read + write
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """Writes `arrays` ({name: array with one row per env}) as out_dir/<name>.npy, float64 kept, everything else as
+    float32, plus env_index.npy, the envs the rows belong to.  When all envs would take more than `limit` bytes, a
+    fixed seeded sample of envs is written, the same for every build, so that two builds compare row for row."""
+    import numpy as np
+    arrays = {k: np.asarray(v, dtype=np.float64 if np.asarray(v).dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    per_env = 8 + sum(a.nbytes for a in arrays.values()) // n
+    keep = (limit - 4096 * (len(arrays) + 1)) // per_env   # leaves room for each file's .npy header (128 bytes)
+    rows = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), rows.astype(np.float64))
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a[rows])
 
 
 # ------------------------------------------------------------------------------------------------
@@ -315,6 +332,9 @@ def run_ours(args):
     step_ms, kern_ms = timed_steps(env, pool, args.steps, warm)
     t_wall = time.perf_counter() - t_wall0
     launches = b.launch_count - launches0 - warm
+    if args.dump_outputs:   # what the last timed step returned (the end-to-end arm below steps on)
+        obs_dim = max(env._spec.obs_dim[a] for a in range(A))
+        last = {"obs": b.obs[:, :, :obs_dim].cpu(), "reward": b.reward.cpu(), "term": b.term.cpu(), "trunc": b.trunc.cpu()}
 
     # ---- end-to-end arm: C-ABI host-buffer call, pinned H2D / D2H inside the timed region
     h_act, h_obs, h_rew, h_term, h_trunc = b.host_arrays()
@@ -434,6 +454,8 @@ def run_ours(args):
             out["cpu_baseline"] = {"value": v, "unit": "agent-steps/s", "cores": cores, "kind": "port",
                                    "sample": f"{cores} processes x 1 env x 12 s of the same workload ({n} env-steps), fp64 oracle + reference-order host loop"}
         print(json.dumps(out))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {k: v.numpy() for k, v in last.items()})
     if world > 1:
         torch.distributed.barrier()
         torch.distributed.destroy_process_group()
@@ -447,7 +469,11 @@ if __name__ == "__main__":
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-configs", action="store_true", help="headline config only")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write obs / reward / term / trunc of the last timed headline step as "
+                    "DIR/<name>.npy (rank 0's envs), to compare two builds on the same inputs")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if a.impl == "reference":
         run_reference(a)
     else:
