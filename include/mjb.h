@@ -194,7 +194,7 @@ int mjb_sync(mjb_batch* b);
  * When all five arrays are page-locked (cudaHostAlloc / torch pin_memory) the kernel writes obs / reward / term /
  * trunc straight into them (zero-copy) and the DEVICE copies buffers.obs / reward / term / trunc are NOT updated by
  * that call: read the results from the host arrays.  State buffers (qpos, qvel, store, timestep ...) are always
- * updated.  MJB_HOST_ZEROCOPY=0 restores "device buffers written, then copied". */
+ * updated. */
 int mjb_step_host(mjb_batch* b, const float* actions, float* obs, float* reward, uint8_t* term, uint8_t* trunc);
 /* number of kernel launches issued so far by this handle */
 int64_t mjb_launch_count(const mjb_batch* b);
@@ -202,10 +202,6 @@ int64_t mjb_launch_count(const mjb_batch* b);
  * recorded around each launch when enabled with mjb_set_timing(b, 1) */
 int mjb_set_timing(mjb_batch* b, int32_t enable);
 int mjb_kernel_time_ms(mjb_batch* b, double* total_ms, int64_t* launches);
-/* Optional scheduling hint: a device permutation of [0, num_envs) (NULL = identity).  Consecutive entries
- * share an SM round, so ordering envs by their last solver cost (buffers.niter) evens the rounds out.
- * Results do not depend on it (envs are independent). */
-int mjb_set_env_order(mjb_batch* b, const int32_t* order_dev);
 /* Level variants (the reference's `xmlPath` list, mujoco_parent.py:88-91,351-356): several batch handles, one
  * per level, are created over the SAME caller-owned buffers; each then steps / resets only the envs currently
  * assigned to its level.  `env_ids_dev` lists `count` distinct env indices in [0, num_envs) (device memory,

@@ -110,7 +110,6 @@ def load(build_if_missing=True):
     lib.mjb_launch_count.argtypes = [vp]
     lib.mjb_set_timing.argtypes = [vp, i32]
     lib.mjb_kernel_time_ms.argtypes = [vp, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(i64)]
-    lib.mjb_set_env_order.argtypes = [vp, vp]
     lib.mjb_set_env_subset.argtypes = [vp, vp, ctypes.c_int32]
     lib.mjb_render.argtypes = [vp, ctypes.POINTER(ctypes.c_int32), ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, vp]
     lib.mjb_batch_geometry.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(i32), ctypes.POINTER(i64)]

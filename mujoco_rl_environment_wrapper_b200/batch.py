@@ -5,7 +5,6 @@ CUDA tensors owned here (row-major, env-major, rows 16 B aligned); the library o
 pointers.  There is no CPU fallback: constructing a Batch without a CUDA device raises.
 """
 import ctypes
-import os
 
 import numpy as np
 import torch
@@ -34,21 +33,12 @@ class Batch:
         A, N, dev = spec.n_agents, self.num_envs, self.device
         f32, i32, u8 = torch.float32, torch.int32, torch.uint8
         z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=dev)
-        # the step's results (obs, reward, term, trunc) live back to back in ONE allocation so that the host-buffer
-        # entry point can return them with a single device-to-host copy
-        nb = [N * max(1, A) * lay.obs_stride * 4, N * max(1, A) * 4, N * (A + 1), N * (A + 1)]
-        self._out_block = share._out_block if share is not None else torch.zeros(sum((b + 15) // 16 * 16 for b in nb) , dtype=u8, device=dev)
-        offs, o = [], 0
-        for b in nb:
-            offs.append(o)
-            o += (b + 15) // 16 * 16
-        view = lambda k, dt, shape: self._out_block[offs[k]:offs[k] + nb[k]].view(dt).view(shape)
         self.buf = share.buf if share is not None else {
             "qpos": z((N, lay.qpos_stride), f32), "qvel": z((N, lay.qvel_stride), f32),
             "ctrl": z((N, lay.ctrl_stride), f32), "warmstart": z((N, lay.qvel_stride), f32),
             "sensordata": z((N, lay.sensor_stride), f32), "probe": z((N, max(1, lay.probe_count), 4), f32),
-            "actions": z((N, max(1, A), lay.act_stride), f32), "obs": view(0, f32, (N, max(1, A), lay.obs_stride)),
-            "reward": view(1, f32, (N, max(1, A))), "term": view(2, u8, (N, A + 1)), "trunc": view(3, u8, (N, A + 1)),
+            "actions": z((N, max(1, A), lay.act_stride), f32), "obs": z((N, max(1, A), lay.obs_stride), f32),
+            "reward": z((N, max(1, A)), f32), "term": z((N, A + 1), u8), "trunc": z((N, A + 1), u8),
             "timestep": z((N,), i32), "store_i": z((N, max(1, A), lay.store_i32), i32),
             "store_f": z((N, max(1, A), lay.store_f32), f32), "ncon": z((N,), i32),
             "contact_geom": z((N, lay.maxcon, 2), i32), "contact_dist": z((N, lay.maxcon), f32), "niter": z((N,), i32), "nreset": z((N,), i32), "ncon_dropped": z((N,), i32),
@@ -68,7 +58,6 @@ class Batch:
                                                ctypes.c_void_p(self.stream.cuda_stream), ctypes.byref(B), ctypes.byref(h)),
                     "batch create")
         self._h = h
-        self.balance_every = int(os.environ.get("MJB_BALANCE_EVERY", "0"))
 
     def __del__(self):
         try:
@@ -94,19 +83,6 @@ class Batch:
 
     def step(self):
         L.check(self._lib.mjb_step(self._h), "step")
-        self._steps = getattr(self, "_steps", 0) + 1
-        if self.balance_every and self._steps % self.balance_every == 0:
-            self.rebalance()
-
-    def rebalance(self):
-        """Scheduling hint only: order envs by their last solver cost (Newton iterations, contacts) so that the
-        lock-step rounds of an SM hold envs of similar cost.  One device sort, no host sync.  (Measured in round 2, also
-        with the sorted groups dealt to the CTAs in snake order: <= 2 % under random actions, less than the sort costs;
-        off by default.)"""
-        key = self.buf["niter"] * 64 + self.buf["ncon"]
-        order = torch.argsort(key).to(torch.int32)
-        self._order = order.contiguous()
-        L.check(self._lib.mjb_set_env_order(self._h, ctypes.c_void_p(self._order.data_ptr())), "env order")
 
     def set_subset(self, env_ids=None):
         """Restrict this handle's launches to the listed env indices (int32 CUDA tensor; None = all envs)."""
@@ -152,21 +128,14 @@ class Batch:
 
     def host_arrays(self, pinned=True):
         """(actions, obs, reward, term, trunc) host arrays for step_host.  Page-locked by default: the library
-        then copies straight to / from them; pageable arrays work too (staged through pinned memory)."""
+        then copies the actions straight from them and the kernel writes the results into them; pageable arrays work
+        too (staged through pinned memory)."""
         lay, A, N = self.layout, self.spec.n_agents, self.num_envs
-        act = torch.zeros((N, A, lay.act_stride), dtype=torch.float32, pin_memory=pinned)
-        # results mirror the device block (same 16-byte aligned offsets): one D2H copy brings all four back
-        nb = [N * A * lay.obs_stride * 4, N * A * 4, N * (A + 1), N * (A + 1)]
-        block = torch.zeros(sum((b + 15) // 16 * 16 for b in nb), dtype=torch.uint8, pin_memory=pinned)
-        offs, o = [], 0
-        for b in nb:
-            offs.append(o)
-            o += (b + 15) // 16 * 16
-        views = [block[offs[0]:offs[0] + nb[0]].view(torch.float32).view(N, A, lay.obs_stride),
-                 block[offs[1]:offs[1] + nb[1]].view(torch.float32).view(N, A),
-                 block[offs[2]:offs[2] + nb[2]].view(N, A + 1), block[offs[3]:offs[3] + nb[3]].view(N, A + 1)]
-        self._host_keep = [act, block] + views
-        return (act.numpy(),) + tuple(v.numpy() for v in views)
+        z = lambda shape, dt: torch.zeros(shape, dtype=dt, pin_memory=pinned)
+        f32, u8 = torch.float32, torch.uint8
+        self._host_keep = [z((N, A, lay.act_stride), f32), z((N, A, lay.obs_stride), f32), z((N, A), f32),
+                           z((N, A + 1), u8), z((N, A + 1), u8)]
+        return tuple(t.numpy() for t in self._host_keep)
 
     @property
     def launch_count(self):

@@ -22,14 +22,13 @@
 namespace mjb {
 
 // One CTA per SM, `warps` environments in flight per CTA; each warp walks the env index space with a grid-wide
-// stride (envs are independent: the warps only meet at the staging of the model image and at the round barrier).
-// `active` envs are walked starting at `env_base` (range launches of the host-buffer step) or through `env_order`
-// (a scheduling permutation, or the env ids of one level: mjb_set_env_subset).
+// stride (envs are independent: the warps only meet at the staging of the model image and at the alignment points).
+// `active` envs are walked starting at `env_base` (range launches of the host-buffer step) or through `env_ids`
+// (the env ids of one level: mjb_set_env_subset).
 template <bool PHYS, bool PACKED>
 __global__ void __launch_bounds__(PHYS ? MJB_MAX_THREADS : 512, PHYS ? 1 : 4) k_env(const __grid_constant__ DevModel dm, const uint32_t* __restrict__ image, const mjb_buffers B,
-                      int num_envs, int mode, int skip_frames, const uint8_t* __restrict__ mask, int* __restrict__ next_env,
-                      int lockstep_groups, const int* __restrict__ env_order, int active, int env_base) {
-  const int lockstep = lockstep_groups & 0xff, groups = lockstep_groups >> 8;
+                      int num_envs, int mode, int skip_frames, const uint8_t* __restrict__ mask,
+                      const int* __restrict__ env_ids, int active, int env_base) {
   extern __shared__ __align__(128) uint32_t smem[];
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem);
   uint32_t* img = smem + 4;  // 16 B after the barrier
@@ -46,51 +45,33 @@ __global__ void __launch_bounds__(PHYS ? MJB_MAX_THREADS : 512, PHYS ? 1 : 4) k_
   }
   float* scratch = reinterpret_cast<float*>(img + dm.image_words) + (size_t)warp * (dm.env_words + 4 * ((dm.nprobe + 3) & ~3));
   float* probe = scratch + dm.env_words;
-  // MJB_LOCKSTEP: 2 rounds only, 1 rounds + every alignment point, 3 rounds replaced by a sync before the collision phase,
-  // 4 rounds + re-alignment after the Newton solve, 5 = 4 + before the collision phase, 6 = 4 + Newton iterations,
-  // 7 (default) re-alignment after the Newton solve ONLY: the env-warps leave it together and stay together through the
-  // tail of the step and the head of the next env without a barrier at the round boundary
-  Ctx c{&dm, img, scratch, lane, probe, 0, lockstep == 1 ? 7 : (lockstep == 3 ? 2 : ((lockstep == 4 || lockstep == 7) ? 4 : (lockstep == 5 ? 6 : (lockstep == 6 ? 5 : 0))))};
+  Ctx c{&dm, img, scratch, lane, probe, 0};
 #if defined(MJB_PHASE_PROF)
   long long t_last = clock64();
   c.t_last = &t_last;
 #endif
-  // Two scheduling modes share ONE call site of the step code:
-  //  * lock-step rounds (default): every env-warp of the CTA takes one env per round and the CTA re-aligns
-  //    at each round boundary, so the warps walk through the (large) step code together and share
-  //    instruction-cache lines (measured 2x at 65536 envs); costs waiting for the slowest env of the round;
-  //  * dynamic: each warp pulls its next env from a grid-wide counter (better balance, poor i-cache reuse).
+  // Lock-step rounds: every env-warp of the CTA takes one env per round, so the warps walk through the (large) step
+  // code together and share instruction-cache lines (measured 2x at 65536 envs against a grid-wide work counter).
+  // The physics step re-aligns the busy env-warps right after the Newton solve (step_kernel.cuh, forward): they leave
+  // it together and stay together through the tail of the step and the head of the next env, so there is no barrier
+  // at the round boundary.  The physics-free step has no alignment point inside and re-aligns at the end of each round.
   const int stride = gridDim.x * warps;
   const int pack = PACKED ? dm.pack : 1;
   const int nvirt = (active + pack - 1) / pack;   // virtual envs: `pack` real envs share a warp (active = envs this launch walks)
   const int rounds = (nvirt - blockIdx.x * warps + stride - 1) / stride;
   int env = blockIdx.x * warps + warp;
-  for (int r = 0;; r++) {
-    if (lockstep ? (r >= rounds) : (env >= nvirt)) break;
-    if (lockstep != 0 && lockstep != 2) {
+  for (int r = 0; r < rounds; r++) {
+    if (PHYS) {
       int busy = nvirt - (blockIdx.x * warps + r * stride);  // env-warps of this CTA with work in this round
       // (a masked reset lets warps skip their env, so intra-step alignment is off for it)
       c.cta_threads = (mask == nullptr ? 32 : 0) * (busy > warps ? warps : (busy < 0 ? 0 : busy));
     }
     c.img_bar = r == 0 ? bar : nullptr;
-    if (env < nvirt) run_env<PHYS, PACKED>(c, B, env_order ? env_order[env] : env + env_base, num_envs, mode, skip_frames, mask);
+    if (env < nvirt) run_env<PHYS, PACKED>(c, B, env_ids ? env_ids[env] : env + env_base, num_envs, mode, skip_frames, mask);
     if (r == 0) mbar_wait(bar, 0);   // warps that had nothing to do in the first round (or returned early) have not waited yet
-    if (lockstep) {
-      if (groups > 1) {
-        // the env-warps re-align in `groups` independent sets: fewer warps wait on the slowest env of a round,
-        // at the price of `groups` instruction streams per SM
-        const int gsz = (warps + groups - 1) / groups, g = warp / gsz;
-        const int cnt = 32 * (g * gsz + gsz <= warps ? gsz : warps - g * gsz);
-        asm volatile("bar.sync %0, %1;" ::"r"(2 + g), "r"(cnt) : "memory");
-      } else if (lockstep != 3 && lockstep != 7) __syncthreads();   // modes 3 / 7 align inside the step only (before the collision phase / after the solve)
-      MJB_PH(c, PH_BARRIER);
-      env += stride;
-    } else {
-      __syncwarp();
-      int nxt = 0;
-      if (lane == 0) nxt = atomicAdd(next_env, 1);
-      env = __shfl_sync(0xffffffffu, nxt, 0);
-    }
+    if (!PHYS) __syncthreads();
+    MJB_PH(c, PH_BARRIER);
+    env += stride;
   }
 }
 
@@ -113,23 +94,16 @@ struct mjb_batch {
   size_t smem_bytes = 0;
   cudaStream_t stream = nullptr;
   cudaStream_t stream2 = nullptr;            // host-buffer step: second half of the envs (copy / compute overlap)
-  cudaEvent_t ev_fork = nullptr, ev_k0 = nullptr, ev_join = nullptr;
-  int host_zero_copy = 1;                    // MJB_HOST_ZEROCOPY: 1 = the kernel writes page-locked result arrays itself
-  int host_split = 1;                        // MJB_HOST_SPLIT: 1 = pipeline the host-buffer step in two halves
+  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   uint32_t* d_image = nullptr;
-  int* d_next = nullptr;   // ring of work counters, one per in-flight launch
-  int next_slot = 0;
-  int lockstep = 0, groups = 1;
   mjb::DevImage rimg;     // camera rendering: one-env-per-CTA image + camera table (models with cameras only)
   uint32_t *d_rimage = nullptr, *d_rtab = nullptr;
-  const int* env_order = nullptr;   // scheduling permutation of all envs ...
-  const int* subset = nullptr;      // ... or the env ids of this handle's level
+  const int* subset = nullptr;      // the env ids of this handle's level (null: all envs)
   int subset_count = -1;
   int64_t launches = 0;
   bool timing = false;
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> events;
   // pinned staging for the host-buffer entry point
-  int* h_first = nullptr;  // pinned: initial value of the work counter (= grid * warps)
   float *h_act = nullptr, *h_obs = nullptr, *h_rew = nullptr;
   uint8_t *h_term = nullptr, *h_trunc = nullptr;
   const void* pin_cache[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -158,11 +132,6 @@ int launch(mjb_batch* b, int mode, int skip_frames, const uint8_t* mask, cudaStr
     CUDA_TRY(cudaEventCreate(&e1));
     CUDA_TRY(cudaEventRecord(e0, stream));
   }
-  // dynamic scheduler only: the first grid*warps envs are taken statically, the counter hands out the rest
-  int* counter = b->d_next + b->next_slot;
-  b->next_slot = (b->next_slot + 1) % 64;
-  if (b->lockstep == 0)  // only the dynamic scheduler consumes the counter
-    CUDA_TRY(cudaMemcpyAsync(counter, &b->h_first[0], sizeof(int), cudaMemcpyHostToDevice, stream));
   if (mode == mjb::MODE_STEP && b->has_lite && !b->subset) {
     // no physics in the step: the bandwidth-shaped tile kernel (lite_kernel.cuh) over the contiguous env range
     const int ntiles = (active + b->tile.tile - 1) / b->tile.tile;
@@ -190,15 +159,13 @@ int launch(mjb_batch* b, int mode, int skip_frames, const uint8_t* mask, cudaStr
   } else if (mode == mjb::MODE_STEP && b->has_lite) {
     // an env-id list (level variants) is not a contiguous range: the warp-per-env form of the same step
     mjb::k_env<false, false><<<b->lite_grid, b->lite_warps * 32, b->lite_smem, stream>>>(b->lite.dm, b->d_image, B, b->num_envs, mode,
-                                                                                   skip_frames, mask, counter, 2, b->subset, active, base);
+                                                                                   skip_frames, mask, b->subset, active, base);
   } else {
     auto kern = b->img.dm.pack > 1 ? mjb::k_env<true, true> : mjb::k_env<true, false>;
     const int pack = b->img.dm.pack;
-    const bool ranged = count >= 0 && !b->subset;   // a range launch walks env ids directly
     const int need = ((active + pack - 1) / pack + b->warps - 1) / b->warps;
     kern<<<std::min(b->grid, std::max(1, need)), b->warps * 32, b->smem_bytes, stream>>>(
-        b->img.dm, b->d_image, B, b->num_envs, mode, skip_frames, mask, counter, b->lockstep | (b->groups << 8),
-        b->subset ? b->subset : ((b->lockstep && pack == 1 && !ranged) ? b->env_order : nullptr), active, base / pack);
+        b->img.dm, b->d_image, B, b->num_envs, mode, skip_frames, mask, b->subset, active, base / pack);
   }
   CUDA_TRY(cudaGetLastError());
   if (b->timing) {
@@ -267,16 +234,13 @@ int mjb_batch_create(const mjb_model* m, const mjb_env_spec* spec, int32_t num_e
   size_t max_smem = prop.sharedMemPerBlockOptin;
   size_t fixed = 16 + (size_t)dm.image_words * 4;
   size_t per_env = ((size_t)dm.env_words + 4 * ((dm.nprobe + 3) & ~3)) * 4;
-  // `ctas` lock-step groups per SM (each with its own copy of the model image and its own round barrier)
-  int ctas = std::max(1, mjb::env_int("MJB_CTAS_PER_SM", 1));
-  size_t sm_smem = prop.sharedMemPerMultiprocessor;
-  size_t cta_budget = std::min(max_smem, sm_smem / ctas - 1024);
+  size_t cta_budget = std::min(max_smem, prop.sharedMemPerMultiprocessor - 1024);
   int warps = cta_budget > fixed ? (int)((cta_budget - fixed) / per_env) : 0;
   int cap = std::min(MJB_MAX_THREADS / 32, mjb::env_int("MJB_WARPS", MJB_MAX_THREADS / 32));
   if (warps > cap) warps = cap;
   if (warps < 1) { mjb::set_error("model needs more shared memory per environment than one SM has"); return fail(MJB_ERR_LIMIT); }
   // even out the rounds: the fewest warps per CTA that keeps the same number of passes over the envs
-  int sms = prop.multiProcessorCount * ctas;
+  int sms = prop.multiProcessorCount;
   const int nvirt = (num_envs + dm.pack - 1) / dm.pack;
   int rounds = (nvirt + sms * warps - 1) / (sms * warps);
   int even = (nvirt + sms * rounds - 1) / (sms * rounds);
@@ -341,23 +305,12 @@ int mjb_batch_create(const mjb_model* m, const mjb_env_spec* spec, int32_t num_e
     mjb::set_error("device image upload failed");
     return fail(MJB_ERR_CUDA);
   }
-  if (cudaMalloc(&b->d_next, 64 * sizeof(int)) != cudaSuccess || cudaMallocHost(&b->h_first, sizeof(int)) != cudaSuccess) {
-    mjb::set_error("work counter allocation failed");
-    return fail(MJB_ERR_CUDA);
-  }
-  b->h_first[0] = b->grid * b->warps;
-  b->host_split = mjb::env_int("MJB_HOST_SPLIT", 1);
-  b->host_zero_copy = mjb::env_int("MJB_HOST_ZEROCOPY", 1);
   if (cudaStreamCreateWithFlags(&b->stream2, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreateWithFlags(&b->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
-      cudaEventCreateWithFlags(&b->ev_k0, cudaEventDisableTiming) != cudaSuccess ||
       cudaEventCreateWithFlags(&b->ev_join, cudaEventDisableTiming) != cudaSuccess) {
     mjb::set_error("mjb_batch_create: stream / event creation failed");
     return fail(MJB_ERR_CUDA);
   }
-  b->lockstep = mjb::env_int("MJB_LOCKSTEP", 7);
-  b->groups = mjb::env_int("MJB_GROUPS", 1);
-  if (b->groups < 1 || b->groups > 8 || b->lockstep != 2) b->groups = 1;
   const int A = dm.a1;
   if (cudaMallocHost(&b->h_act, sizeof(float) * (size_t)num_envs * A * dm.act_stride + 16) != cudaSuccess ||
       cudaMallocHost(&b->h_obs, sizeof(float) * (size_t)num_envs * A * dm.obs_stride + 16) != cudaSuccess ||
@@ -376,13 +329,11 @@ void mjb_batch_destroy(mjb_batch* b) {
   for (auto& ev : b->events) { cudaEventDestroy(ev.first); cudaEventDestroy(ev.second); }
   if (b->d_image) cudaFree(b->d_image);
   if (b->stream2) cudaStreamDestroy(b->stream2);
-  for (cudaEvent_t e : {b->ev_fork, b->ev_k0, b->ev_join}) if (e) cudaEventDestroy(e);
+  for (cudaEvent_t e : {b->ev_fork, b->ev_join}) if (e) cudaEventDestroy(e);
   if (b->d_rimage) cudaFree(b->d_rimage);
   if (b->d_rtab) cudaFree(b->d_rtab);
-  if (b->d_next) cudaFree(b->d_next);
   if (b->d_lite_tab) cudaFree(b->d_lite_tab);
   if (b->d_lite_dm) cudaFree(b->d_lite_dm);
-  if (b->h_first) cudaFreeHost(b->h_first);
   if (b->h_act) cudaFreeHost(b->h_act);
   if (b->h_obs) cudaFreeHost(b->h_obs);
   if (b->h_rew) cudaFreeHost(b->h_rew);
@@ -426,34 +377,24 @@ int mjb_step_host(mjb_batch* b, const float* actions, float* obs, float* reward,
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return false; }
     return at.type == cudaMemoryTypeHost;
   };
-  const bool direct = pinned(actions) && pinned(obs) && pinned(reward) && pinned(term) && pinned(trunc);
+  bool direct = pinned(actions) && pinned(obs) && pinned(reward) && pinned(term) && pinned(trunc);
   if (direct) {
     b->pin_cache[0] = actions; b->pin_cache[1] = obs; b->pin_cache[2] = reward; b->pin_cache[3] = term; b->pin_cache[4] = trunc;
-  } else {
-    memcpy(b->h_act, actions, nb_act);
   }
-  // when the four result arrays sit back to back (16-byte aligned) on both sides, one copy returns them all
-  auto r16 = [](size_t n) { return (n + 15) / 16 * 16; };
-  const char *d0 = (const char*)b->B.obs, *h0 = (const char*)obs;
-  const bool packed_out = direct && (const char*)b->B.reward == d0 + r16(nb_obs) && (const char*)reward == h0 + r16(nb_obs) &&
-                          (const char*)b->B.term == d0 + r16(nb_obs) + r16(nb_rew) && (const char*)term == h0 + r16(nb_obs) + r16(nb_rew) &&
-                          (const char*)b->B.trunc == d0 + r16(nb_obs) + r16(nb_rew) + r16(nb_flag) &&
-                          (const char*)trunc == h0 + r16(nb_obs) + r16(nb_rew) + r16(nb_flag);
   // Page-locked result arrays are written by the kernel itself (zero-copy: pinned host memory is device-addressable,
   // the stores are posted PCIe writes that overlap the rest of the step), so no device-to-host copy follows the
   // kernel.  The actions still go up by copy engine, in two halves on two streams so that the second half's upload
   // overlaps the first half's compute.  Same results (envs are independent).
-  const int pack = dm.pack;
-  int half = (int)((N / 2 + pack - 1) / pack * pack);
-  const bool split = b->host_split && !b->subset && b->lockstep != 0 && N >= (size_t)(4 * b->warps) && half > 0 && (size_t)half < N;
-  if (direct && b->host_zero_copy && !b->subset) {
+  if (direct && !b->subset) {
     mjb_buffers Bh = b->B;
     void *d_obs = nullptr, *d_rew = nullptr, *d_term = nullptr, *d_trunc = nullptr;
     if (cudaHostGetDevicePointer(&d_obs, obs, 0) == cudaSuccess && cudaHostGetDevicePointer(&d_rew, reward, 0) == cudaSuccess &&
         cudaHostGetDevicePointer(&d_term, term, 0) == cudaSuccess && cudaHostGetDevicePointer(&d_trunc, trunc, 0) == cudaSuccess) {
       Bh.obs = (float*)d_obs; Bh.reward = (float*)d_rew; Bh.term = (uint8_t*)d_term; Bh.trunc = (uint8_t*)d_trunc;
       const size_t act_row = sizeof(float) * A * dm.act_stride;
-      if (split) {
+      const int pack = dm.pack;
+      const int half = (int)((N / 2 + pack - 1) / pack * pack);
+      if (N >= (size_t)(4 * b->warps) && half > 0 && (size_t)half < N) {
         CUDA_TRY(cudaEventRecord(b->ev_fork, b->stream));
         CUDA_TRY(cudaStreamWaitEvent(b->stream2, b->ev_fork, 0));
         CUDA_TRY(cudaMemcpyAsync(b->B.actions, actions, act_row * half, cudaMemcpyHostToDevice, b->stream));
@@ -477,52 +418,18 @@ int mjb_step_host(mjb_batch* b, const float* actions, float* obs, float* reward,
     // memory): forget what was remembered and take the staged path for this call
     cudaGetLastError();
     for (auto& p : b->pin_cache) p = nullptr;
-    memcpy(b->h_act, actions, nb_act);
-    CUDA_TRY(cudaMemcpyAsync(b->B.actions, b->h_act, nb_act, cudaMemcpyHostToDevice, b->stream));
-    int rc = launch(b, mjb::MODE_STEP, dm.skip_frames, nullptr);
-    if (rc != MJB_OK) return rc;
-    CUDA_TRY(cudaMemcpyAsync(b->h_obs, b->B.obs, nb_obs, cudaMemcpyDeviceToHost, b->stream));
-    CUDA_TRY(cudaMemcpyAsync(b->h_rew, b->B.reward, nb_rew, cudaMemcpyDeviceToHost, b->stream));
-    CUDA_TRY(cudaMemcpyAsync(b->h_term, b->B.term, nb_flag, cudaMemcpyDeviceToHost, b->stream));
-    CUDA_TRY(cudaMemcpyAsync(b->h_trunc, b->B.trunc, nb_flag, cudaMemcpyDeviceToHost, b->stream));
-    CUDA_TRY(cudaStreamSynchronize(b->stream));
-    memcpy(obs, b->h_obs, nb_obs); memcpy(reward, b->h_rew, nb_rew); memcpy(term, b->h_term, nb_flag); memcpy(trunc, b->h_trunc, nb_flag);
-    return MJB_OK;
+    direct = false;
   }
-  // Two halves on two streams: the second half's actions go up while the first half computes, and the first
-  // half's observations come down while the second half computes.
-  if (split && packed_out) {
-    const size_t act_row = sizeof(float) * A * dm.act_stride, obs_row = sizeof(float) * A * dm.obs_stride;
-    CUDA_TRY(cudaEventRecord(b->ev_fork, b->stream));
-    CUDA_TRY(cudaStreamWaitEvent(b->stream2, b->ev_fork, 0));
-    CUDA_TRY(cudaMemcpyAsync(b->B.actions, actions, act_row * half, cudaMemcpyHostToDevice, b->stream));
-    CUDA_TRY(cudaMemcpyAsync((char*)b->B.actions + act_row * half, (const char*)actions + act_row * half, act_row * (N - half),
-                             cudaMemcpyHostToDevice, b->stream2));
-    int rc = launch(b, mjb::MODE_STEP, dm.skip_frames, nullptr, b->stream, 0, half);
-    if (rc != MJB_OK) return rc;
-    CUDA_TRY(cudaEventRecord(b->ev_k0, b->stream));
-    CUDA_TRY(cudaMemcpyAsync(obs, b->B.obs, obs_row * half, cudaMemcpyDeviceToHost, b->stream));
-    rc = launch(b, mjb::MODE_STEP, dm.skip_frames, nullptr, b->stream2, half, (int)N - half);
-    if (rc != MJB_OK) return rc;
-    CUDA_TRY(cudaStreamWaitEvent(b->stream2, b->ev_k0, 0));   // the tail copy also carries the first half's rewards / flags
-    CUDA_TRY(cudaMemcpyAsync((char*)obs + obs_row * half, (const char*)b->B.obs + obs_row * half,
-                             (r16(nb_obs) - obs_row * half) + r16(nb_rew) + r16(nb_flag) + nb_flag, cudaMemcpyDeviceToHost, b->stream2));
-    CUDA_TRY(cudaEventRecord(b->ev_join, b->stream2));
-    CUDA_TRY(cudaStreamWaitEvent(b->stream, b->ev_join, 0));
-    CUDA_TRY(cudaStreamSynchronize(b->stream));
-    return MJB_OK;
-  }
+  // Pageable arrays, a level subset, or arrays not device-addressable: upload the actions, step, copy the results back
+  // (page-locked arrays directly, others through the pinned staging area).
+  if (!direct) memcpy(b->h_act, actions, nb_act);
   CUDA_TRY(cudaMemcpyAsync(b->B.actions, direct ? actions : b->h_act, nb_act, cudaMemcpyHostToDevice, b->stream));
   int rc = launch(b, mjb::MODE_STEP, dm.skip_frames, nullptr);
   if (rc != MJB_OK) return rc;
-  if (packed_out) {
-    CUDA_TRY(cudaMemcpyAsync(obs, b->B.obs, r16(nb_obs) + r16(nb_rew) + r16(nb_flag) + nb_flag, cudaMemcpyDeviceToHost, b->stream));
-  } else {
-    CUDA_TRY(cudaMemcpyAsync(direct ? obs : b->h_obs, b->B.obs, nb_obs, cudaMemcpyDeviceToHost, b->stream));
-    CUDA_TRY(cudaMemcpyAsync(direct ? reward : b->h_rew, b->B.reward, nb_rew, cudaMemcpyDeviceToHost, b->stream));
-    CUDA_TRY(cudaMemcpyAsync(direct ? term : b->h_term, b->B.term, nb_flag, cudaMemcpyDeviceToHost, b->stream));
-    CUDA_TRY(cudaMemcpyAsync(direct ? trunc : b->h_trunc, b->B.trunc, nb_flag, cudaMemcpyDeviceToHost, b->stream));
-  }
+  CUDA_TRY(cudaMemcpyAsync(direct ? obs : b->h_obs, b->B.obs, nb_obs, cudaMemcpyDeviceToHost, b->stream));
+  CUDA_TRY(cudaMemcpyAsync(direct ? reward : b->h_rew, b->B.reward, nb_rew, cudaMemcpyDeviceToHost, b->stream));
+  CUDA_TRY(cudaMemcpyAsync(direct ? term : b->h_term, b->B.term, nb_flag, cudaMemcpyDeviceToHost, b->stream));
+  CUDA_TRY(cudaMemcpyAsync(direct ? trunc : b->h_trunc, b->B.trunc, nb_flag, cudaMemcpyDeviceToHost, b->stream));
   CUDA_TRY(cudaStreamSynchronize(b->stream));
   if (!direct) {
     memcpy(obs, b->h_obs, nb_obs);
@@ -553,12 +460,6 @@ int mjb_kernel_time_ms(mjb_batch* b, double* total_ms, int64_t* launches) {
   }
   *total_ms = tot; *launches = (int64_t)b->events.size();
   b->events.clear();
-  return MJB_OK;
-}
-
-int mjb_set_env_order(mjb_batch* b, const int32_t* order_dev) {
-  if (!b) { mjb::set_error("mjb_set_env_order: null batch"); return MJB_ERR_ARG; }
-  b->env_order = order_dev;
   return MJB_OK;
 }
 

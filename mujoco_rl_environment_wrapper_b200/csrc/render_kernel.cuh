@@ -154,7 +154,7 @@ __global__ void __launch_bounds__(256) k_render(const __grid_constant__ DevModel
   for (int i = tid; i < dm.image_words; i += blockDim.x) img[i] = image[i];
   for (int i = tid; i < rh.words; i += blockDim.x) tab[i] = rtab[i];
   __syncthreads();
-  Ctx c{&dm, img, scratch, lane, nullptr, 0, 0};
+  Ctx c{&dm, img, scratch, lane, nullptr, 0};
   const float* rgba = reinterpret_cast<const float*>(tab + rh.off_rgba);
   const int tiles_x = (width + RENDER_TILE_W - 1) / RENDER_TILE_W, tiles_y = (height + RENDER_TILE_H - 1) / RENDER_TILE_H;
   const int tiles_cam = tiles_x * tiles_y, ntiles = tiles_cam * cams.n;

@@ -85,9 +85,7 @@ struct Ctx {
   float* s;             // this env's scratch (shared memory)
   int lane;
   float* probe;         // exported positions of this env (shared memory, 4 floats per probe)
-  int cta_threads;      // threads of the CTA busy in this lock-step round (0 / 32: no CTA-level alignment)
-  int align_all;        // CTA-level re-alignment points inside the step (bits): 1 constraints / Newton iterations, 2 before the
-                        // collision phase, 4 after the Newton solve (the data-dependent part): see k_env
+  int cta_threads;      // threads of the CTA busy in this lock-step round (0 / 32: no CTA-level alignment after the solve)
   float* probe_quat;    // this env's exported orientations in GLOBAL memory (4 floats per probe) or null
   uint64_t* img_bar;    // first round of a launch: barrier of the image's bulk copy, waited on at the first use of the image (else null)
 #if defined(MJB_PHASE_PROF)
@@ -1526,24 +1524,18 @@ MJB_DEV int newton(const Ctx& c, int ncon) {
   }
   MJB_PH(c, PH_NEWTON_INIT);
   int it = 0;
-  bool done = false;
   float last_step = 0.f;   // |alpha s| of the previous iteration (lane = dof)
   MJB_NOUNROLL
   for (;;) {
-    // Iterations can be aligned across the env-warps of the CTA (c.align_all: they then share instruction-cache
-    // lines); a warp whose env has converged idles at the barrier until every env of the round is done.
-    if (!done) {
-      const float qf = lane < nv ? qfrc[lane] : 0.f, ma = lane < nv ? tot[lane] + g : 0.f;   // M a = qfrc_smooth + J' f + g
-      // (four independent reductions in one stage: gradient and force norms, and the size of the previous step against
-      // the iterate for the stall test)
-      const float gn = wsum(g * g), fn = wsum(qf * qf + ma * ma);
-      const float amax = wmax(lane < nv ? fabsf(a[lane]) : 0.f), smax = wmax(last_step);
-      const bool stalled = it > 0 && smax <= 1e-7f * (1.f + amax);
-      if (gn <= dm.solver_tol * dm.solver_tol * (fn + 1e-12f) || it >= dm.solver_iterations || stalled) done = true;
-    }
+    const float qf = lane < nv ? qfrc[lane] : 0.f, ma = lane < nv ? tot[lane] + g : 0.f;   // M a = qfrc_smooth + J' f + g
+    // (four independent reductions in one stage: gradient and force norms, and the size of the previous step against
+    // the iterate for the stall test)
+    const float gn = wsum(g * g), fn = wsum(qf * qf + ma * ma);
+    const float amax = wmax(lane < nv ? fabsf(a[lane]) : 0.f), smax = wmax(last_step);
+    const bool stalled = it > 0 && smax <= 1e-7f * (1.f + amax);
+    const bool done = gn <= dm.solver_tol * dm.solver_tol * (fn + 1e-12f) || it >= dm.solver_iterations || stalled;
     MJB_PH(c, PH_NEWTON_GRAD);
-    if (!((c.align_all & 1) ? MJB_CTA_ANY(c.cta_threads, !done) : !done)) break;
-    if (done) continue;
+    if (done) break;
     it++;
     // Hessian H = M + J' diag(D active) J (packed lower triangle)
     {
@@ -1848,8 +1840,6 @@ MJB_DEV int forward(const Ctx& c, bool sensors, bool probes, int* iters_out, int
   MJB_PH(c, PH_FK);
   dyn_backward(c);
   MJB_PH(c, PH_RNE);
-  if (c.align_all & 2) MJB_CTA_SYNC(c.cta_threads);  // re-align the env-warps of the CTA before the data-dependent phases
-  MJB_PH(c, PH_ALIGN);
   int tot[MJB_MAX_PACK] = {0, 0, 0, 0};
   int ncon = collide(c, tot);
   MJB_PH(c, PH_COLLIDE);
@@ -1859,16 +1849,14 @@ MJB_DEV int forward(const Ctx& c, bool sensors, bool probes, int* iters_out, int
   }
   if (sensors) sensors_pos(c);
   MJB_PH(c, PH_SENS);
-  if (c.align_all & 1) MJB_CTA_SYNC(c.cta_threads);
   make_constraints(c, ncon);
   MJB_PH(c, PH_CONSTR);
-  if (c.align_all & 1) MJB_CTA_SYNC(c.cta_threads);
   int it = newton(c, ncon);
   // The Newton solve is where the envs of a round drift apart (1 .. 5 iterations).  Waiting for the slowest one HERE
   // instead of at the end of the round costs the same wait, and the rest of the step (sensors, integration, stores,
   // epilogue) then runs with the warps walking the code together: their instruction fetches hit lines a neighbour
   // has just brought in (the tail used to be the part with the most instruction-fetch stalls)
-  if (c.align_all & 5) MJB_CTA_SYNC(c.cta_threads);
+  MJB_CTA_SYNC(c.cta_threads);
   MJB_PH(c, PH_ALIGN);
   if (iters_out) *iters_out = it;
   if (sensors) sensors_acc(c, ncon);

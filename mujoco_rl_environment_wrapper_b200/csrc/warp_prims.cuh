@@ -26,7 +26,6 @@ inline uint32_t mjb_f2u(float x) { uint32_t u; memcpy(&u, &x, 4); return u; }
 #define MJB_G2S(dst, src) (*(dst) = *(src))
 #define MJB_G2S_WAIT() ((void)0)
 #define MJB_CTA_SYNC(nthreads) ((void)0)
-#define MJB_CTA_ANY(nthreads, pred) (pred)
 #else
 #define MJB_DEV __device__ __forceinline__
 #define MJB_DEV_NOINLINE __device__ __noinline__
@@ -52,23 +51,7 @@ __device__ __forceinline__ void mjb_g2s4(float* dst, const float* src) {
 __device__ __forceinline__ void mjb_cta_sync(int nthreads) {
   if (nthreads > 32) asm volatile("bar.sync 1, %0;" ::"r"(nthreads) : "memory");
 }
-__device__ __forceinline__ bool mjb_cta_any(int nthreads, bool pred) {
-  if (nthreads <= 32) return pred;
-  int out;
-  asm volatile(
-      "{\n"
-      ".reg .pred p, q;\n"
-      "setp.ne.s32 q, %2, 0;\n"
-      "bar.red.or.pred p, 1, %1, q;\n"
-      "selp.s32 %0, 1, 0, p;\n"
-      "}\n"
-      : "=r"(out)
-      : "r"(nthreads), "r"((int)pred)
-      : "memory");
-  return out != 0;
-}
 #define MJB_CTA_SYNC(nthreads) mjb_cta_sync(nthreads)
-#define MJB_CTA_ANY(nthreads, pred) mjb_cta_any((nthreads), (pred))
 #endif
 
 // block-placement hints: rarely taken paths move out of the straight-line instruction stream

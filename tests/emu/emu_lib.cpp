@@ -52,7 +52,7 @@ int emu_run(const void* blob, const mjb_env_spec* spec, int num_envs, const mjb_
     const int nvirt = (num_envs + K - 1) / K;
     for (int env = 0; env < nvirt; env++) {
       simt::run_warp([&]() {
-        mjb::Ctx c{&img.dm, img.words.data(), scratch.data(), simt::lane(), probe.data(), 0, 0};
+        mjb::Ctx c{&img.dm, img.words.data(), scratch.data(), simt::lane(), probe.data(), 0};
         mjb::run_env<true, true>(c, *B, env, num_envs, mode, skip_frames, mask);
       }, reverse != 0);
     }

@@ -593,20 +593,19 @@ def test_level_variants_reject_structural_mismatch(tmp_path):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("scene_xml,agents,n,pinned,split,zero_copy", [
-    ("two_ants.xml", ["sender", "receiver"], 100, True, "1", "1"), ("two_ants.xml", ["sender", "receiver"], 100, True, "0", "1"),
-    ("two_ants.xml", ["sender", "receiver"], 100, True, "1", "0"), ("two_ants.xml", ["sender", "receiver"], 100, True, "0", "0"),
-    ("two_ants.xml", ["sender", "receiver"], 37, False, "1", "1"), ("one_ant_arena.xml", ["sender"], 101, True, "1", "1"),
-    ("one_ant_arena.xml", ["sender"], 101, True, "1", "0"), ("ant_rk4.xml", ["torso"], 64, True, "1", "1")])
-def test_step_host_matches_device_step(monkeypatch, scene_xml, agents, n, pinned, split, zero_copy):
+@pytest.mark.parametrize("scene_xml,agents,n,pinned", [
+    ("two_ants.xml", ["sender", "receiver"], 100, True), ("two_ants.xml", ["sender", "receiver"], 3, True),
+    ("two_ants.xml", ["sender", "receiver"], 37, False), ("one_ant_arena.xml", ["sender"], 101, True),
+    ("one_ant_arena.xml", ["sender"], 3, True), ("one_ant_arena.xml", ["sender"], 101, False),
+    ("ant_rk4.xml", ["torso"], 64, True), ("ant_rk4.xml", ["torso"], 64, False)])
+def test_step_host_matches_device_step(scene_xml, agents, n, pinned):
     """mjb_step_host (host arrays in / out) returns exactly what mjb_step leaves in the device buffers: page-locked
-    arrays written by the kernel itself (zero-copy) or copied back in two pipelined halves, pageable arrays through
-    the staging area; also with several envs per warp (one_ant_arena) and a ragged split."""
+    arrays written by the kernel itself (zero-copy; two launches on two streams from 4 envs per env-warp on, one below:
+    n = 3), pageable arrays uploaded and copied back through the staging area; each also with several envs per warp
+    (one_ant_arena, a ragged split at 101) and with the no-physics tile kernel (ant_rk4)."""
     import os
     from mujoco_rl_environment_wrapper_b200 import plugins as P
     from mujoco_rl_environment_wrapper_b200.mujoco_rl import MuJoCoRL
-    monkeypatch.setenv("MJB_HOST_SPLIT", split)
-    monkeypatch.setenv("MJB_HOST_ZEROCOPY", zero_copy)
     lv = os.path.join(os.path.dirname(__file__), "levels")
     cfg = {"xmlPath": os.path.join(lv, scene_xml), "agents": agents, "num_envs": n, "seed": 11}
     if len(agents) == 2:
