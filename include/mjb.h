@@ -121,10 +121,20 @@ typedef struct mjb_env_spec {
   int32_t n_extra_probes;
   int32_t extra_objtype[MJB_MAX_EXTRA_PROBES];
   int32_t extra_objid[MJB_MAX_EXTRA_PROBES];
+  /* action-space bounds of action dimension d < act_dim, the same for every agent (as action_space.sample() sees
+   * them); read only with MJB_SPEC_AUTORESET, for the random action the dynamics are applied with at an auto-reset */
+  float act_low[64], act_high[64];
+  /* MJB_SPEC_AUTORESET (required then at mjb_batch_create, ignored otherwise): device buffer
+   * [N, n_agents, obs_stride] that receives the last observation of every episode mjb_step ends; rows of other envs
+   * are not written.  (A field of the spec, not of mjb_buffers, so that mjb_buffers keeps its layout.) */
+  float* final_obs;
 } mjb_env_spec;
 
 /* mjb_env_spec.flags */
-enum { MJB_SPEC_NO_PACK = 1 /* one env per warp even for small models (needed by mjb_set_env_subset) */ };
+enum {
+  MJB_SPEC_NO_PACK = 1,   /* one env per warp even for small models (needed by mjb_set_env_subset) */
+  MJB_SPEC_AUTORESET = 2  /* mjb_step resets every env whose step ends its episode, in the same launch (see mjb_step) */
+};
 
 /* Caller-owned device buffers (torch CUDA tensors on the Python side).  Row-major, env-major;
  * strides are in elements and come from mjb_batch_layout. Optional pointers may be NULL. */
@@ -181,16 +191,23 @@ int mjb_batch_create(const mjb_model* m, const mjb_env_spec* spec, int32_t num_e
 void mjb_batch_destroy(mjb_batch* b);
 /* reset envs whose mask byte is non-zero (NULL = all): qpos0, zero velocities, forward pass,
  * data_store wipe, timestep = 0, observations (dynamics applied once with `actions`, results discarded
- * from the store as mujoco_rl.py:322-328 does) */
+ * from the store as mujoco_rl.py:322-328 does), reward / term / trunc = 0.  Never auto-resets. */
 int mjb_reset(mjb_batch* b, const uint8_t* mask_dev);
-/* one MuJoCoRL.step for every env; reads buffers.actions, writes obs / reward / term / trunc */
+/* one MuJoCoRL.step for every env; reads buffers.actions, writes obs / reward / term / trunc.
+ * With MJB_SPEC_AUTORESET, every env whose step sets term[n_agents] | trunc[n_agents] (the "__all__" columns) then
+ * has its obs rows copied to spec.final_obs and is reset in the same launch, as mjb_reset with its mask byte set
+ * would reset it, with two differences: the dynamics are applied with the random action of mjb_reset_action (one
+ * draw per agent and action dimension, keyed by the env's rows as the finishing step left them) instead of
+ * buffers.actions, and reward / term / trunc keep the values of the finishing step.  buffers.obs then holds the
+ * new episode's first observation.  Refused at creation (MJB_ERR_ARG) with skip_frames = 0. */
 int mjb_step(mjb_batch* b);
 /* physics only (apply_action + skip_frames x mj_step), for stage-wise parity tests */
 int mjb_physics(mjb_batch* b, int32_t skip_frames);
 /* forward pass only (mj_forward): kinematics, collisions, sensors; no integration */
 int mjb_forward(mjb_batch* b);
 int mjb_sync(mjb_batch* b);
-/* host-buffer call: H2D actions, step, D2H obs/reward/flags, synchronises.  Layouts as above.
+/* host-buffer call: H2D actions, step, D2H obs/reward/flags, synchronises.  Layouts as above.  MJB_ERR_ARG on a
+ * batch created with MJB_SPEC_AUTORESET.
  * When all five arrays are page-locked (cudaHostAlloc / torch pin_memory) the kernel writes obs / reward / term /
  * trunc straight into them (zero-copy) and the DEVICE copies buffers.obs / reward / term / trunc are NOT updated by
  * that call: read the results from the host arrays.  State buffers (qpos, qvel, store, timestep ...) are always
@@ -206,7 +223,8 @@ int mjb_kernel_time_ms(mjb_batch* b, double* total_ms, int64_t* launches);
  * per level, are created over the SAME caller-owned buffers; each then steps / resets only the envs currently
  * assigned to its level.  `env_ids_dev` lists `count` distinct env indices in [0, num_envs) (device memory,
  * must stay valid until replaced); NULL restores "all envs".  Needs a batch created with MJB_SPEC_NO_PACK.
- * A reset mask stays indexed by env id. */
+ * A reset mask stays indexed by env id.  MJB_ERR_ARG on a batch created with MJB_SPEC_AUTORESET (a reset there
+ * cannot draw a new level). */
 int mjb_set_env_subset(mjb_batch* b, const int32_t* env_ids_dev, int32_t count);   /* (non-NULL, 0) = no env at all */
 /* Agent cameras (`get_camera_data`, mujoco_parent.py:518-556): renders `ncams` fixed cameras (model camera ids,
  * host array; mjb_name2id with MJB_OBJ_CAMERA) of every env from its current qpos into
@@ -221,6 +239,13 @@ int mjb_batch_geometry(const mjb_batch* b, int32_t* grid, int32_t* warps_per_cta
 int mjb_phase_cycles(uint64_t* out, int32_t n);
 /* counter-based draw used for target selection: exported so tests can reproduce the stream */
 uint32_t mjb_draw_u32(uint64_t seed, uint32_t env, uint32_t agent, uint32_t counter);
+/* the random action an auto-reset (MJB_SPEC_AUTORESET) applies the dynamics with, for action dimension `dim` of
+ * `agent` in `env`:
+ *   u = (mjb_draw_u32(seed ^ 0x5eedc0de, env, 0xC000 + agent * 64 + dim, ep) >> 8) * 2^-24
+ *   a = low + u * (high - low)     (fp32, each operation rounded to nearest, no fused multiply-add)
+ * ep = timestep ^ bits(qpos[0]) ^ (bits(qvel[0]) << 13) of the env's rows as the finishing step left them (the key
+ * reset_noise uses); low / high = act_low[dim] / act_high[dim] of the spec */
+float mjb_reset_action(uint64_t seed, uint32_t env, uint32_t agent, uint32_t dim, uint32_t ep, float low, float high);
 
 #ifdef __cplusplus
 }

@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MJB_LIB") or os.path.join(_HERE, "libmjb.so")
 
 MAX_AGENTS, MAX_PLUGINS, MAX_TARGETS, MAX_EXTRA_PROBES = 8, 4, 16, 48
-SPEC_NO_PACK = 1   # mjb_env_spec.flags
+SPEC_NO_PACK, SPEC_AUTORESET = 1, 2   # mjb_env_spec.flags
 OBJ_BODY, OBJ_JOINT, OBJ_GEOM, OBJ_SITE, OBJ_CAMERA, OBJ_ACTUATOR, OBJ_SENSOR = 1, 3, 5, 6, 7, 19, 20
 DYN_LANGUAGE, DYN_PICKUP = 1, 2
 REW_TAG_DISTANCE, REW_ANT = 1, 2
@@ -48,6 +48,7 @@ class EnvSpec(ctypes.Structure):
         ("seed", ctypes.c_uint64),
         ("solver_iterations", ctypes.c_int32), ("ls_iterations", ctypes.c_int32), ("flags", ctypes.c_int32), ("reset_noise", ctypes.c_float),
         ("n_extra_probes", ctypes.c_int32), ("extra_objtype", ctypes.c_int32 * MAX_EXTRA_PROBES), ("extra_objid", ctypes.c_int32 * MAX_EXTRA_PROBES),
+        ("act_low", ctypes.c_float * 64), ("act_high", ctypes.c_float * 64), ("final_obs", ctypes.c_void_p),
     ]
 
 
@@ -116,6 +117,9 @@ def load(build_if_missing=True):
     lib.mjb_phase_cycles.argtypes = [ctypes.POINTER(ctypes.c_uint64), i32]
     lib.mjb_draw_u32.restype = ctypes.c_uint32
     lib.mjb_draw_u32.argtypes = [ctypes.c_uint64, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32]
+    lib.mjb_reset_action.restype = ctypes.c_float
+    lib.mjb_reset_action.argtypes = [ctypes.c_uint64, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32,
+                                     ctypes.c_float, ctypes.c_float]
     _LIB = lib
     return lib
 

@@ -47,6 +47,11 @@ class Batch:
             q = z((N, lay.probe_count, 4), f32)
             q[:, :, 0] = 1.0
             self.buf["probe_quat"] = q
+        if spec.flags & L.SPEC_AUTORESET:
+            # last observation of every episode a step ended (include/mjb.h, mjb_env_spec.final_obs)
+            self.final_obs = z((N, max(1, A), lay.obs_stride), f32)
+            spec = L.EnvSpec.from_buffer_copy(spec)   # the caller's spec stays as it was
+            spec.final_obs = self.final_obs.data_ptr()
         B = L.Buffers()
         for k, v in self.buf.items():
             setattr(B, k, v.data_ptr())

@@ -153,6 +153,12 @@ struct DevModel {
   int env_words;          // scratch words per env (multiple of 4)
   // HBM strides
   int qpos_stride, qvel_stride, ctrl_stride, sensor_stride, act_stride, obs_stride, store_i32, store_f32;
+  // MJB_SPEC_AUTORESET: the step resets the envs it finishes; bounds of the one action slot each dynamic reads (act_lo:
+  // Language's utterance; the random action of the reset, mjb_reset_action).  Last, and 48 bytes in this order, so that
+  // the kernels without the flag address every other field and kernel parameter with the same 16-byte alignment as before.
+  float* final_obs;    // [N, A, obs_stride] (mjb_env_spec.final_obs)
+  int autoreset;
+  float dyn_act_low[4], dyn_act_high[4];
 };
 
 // ---- camera rendering (render_kernel.cuh): a second, small constant table next to the image -------------

@@ -428,6 +428,15 @@ inline void build_dev_model(const ModelView& m, const mjb_env_spec& spec, DevIma
     for (int i = 0; i < 4; i++) d.param[i] = s.param[i];
   };
   for (int i = 0; i < spec.n_dynamics; i++) cp(dm.dynamics[i], spec.dynamics[i]);
+  dm.autoreset = (spec.flags & MJB_SPEC_AUTORESET) ? 1 : 0;
+  dm.final_obs = dm.autoreset ? spec.final_obs : nullptr;
+  for (int i = 0; i < spec.n_dynamics; i++) {
+    const int d = spec.dynamics[i].act_lo;
+    if (dm.autoreset && spec.dynamics[i].act_hi > d) {
+      if (d < 0 || d >= spec.act_dim || d >= 64) throw std::runtime_error("dynamic action slot out of range");
+      dm.dyn_act_low[i] = spec.act_low[d]; dm.dyn_act_high[i] = spec.act_high[d];
+    }
+  }
   for (int i = 0; i < spec.n_rewards; i++) cp(dm.rewards[i], spec.rewards[i]);
   for (int i = 0; i < spec.n_dones; i++) cp(dm.dones[i], spec.dones[i]);
   std::vector<int> pk, pid;

@@ -33,6 +33,18 @@ MJB_HD uint32_t draw_u32(unsigned long long seed, uint32_t env, uint32_t agent, 
   return (uint32_t)(z >> 32);
 }
 
+// the random action of an auto-reset (include/mjb.h, mjb_reset_action): uniform in [low, high), keyed like reset_noise
+// by how the episode ended; each operation rounded on its own, so that a float32 host evaluation gives the same bits
+MJB_HD float reset_action(unsigned long long seed, uint32_t env, uint32_t agent, uint32_t dim, uint32_t ep, float low, float high) {
+  const float u = (float)(draw_u32(seed ^ 0x5eedc0deULL, env, 0xC000u + agent * 64u + dim, ep) >> 8) * (1.f / 16777216.f);
+#if defined(__CUDA_ARCH__)
+  return __fadd_rn(low, __fmul_rn(u, high - low));
+#else
+  volatile float span = u * (high - low);
+  return low + span;
+#endif
+}
+
 // Distances, the reward arithmetic and the done comparison run in fp64 on the fp32 positions (the reference computes
 // math.dist on float64 numpy views, mujoco_parent.py:428-449): given identical xipos the reward, cast to fp32, and the
 // done flag are those of the reference's own arithmetic.  The stored distance keeps its fp64 value in two store_f
@@ -67,9 +79,12 @@ MJB_DEV void st_dist(float* sfa, double d) {
 // shared memory), `ctrl` the env's ctrl row (read by the ant reward), `probe` its exported positions.
 // AMAX bounds the agent loops at compile time: with a small AMAX (the tile kernel uses 2) the per-agent accumulators
 // live in registers and the loops unroll; MJB_MAX_AGENTS is the general form.
+// A reset zeroes rew / term / trunc unless `keep_flags` (auto-reset: they stay those of the step that ended the episode).
+// Returns whether the step ended the episode (term[A] | trunc[A]); false for a reset.
 template <int AMAX>
-MJB_DEV void run_plugins(const DevModel& dm, const float* ctrl, float* obs, float* rew, uint8_t* term, uint8_t* trunc, int env, int copy,
-                         bool is_reset, const float* probe, int* si, float* sf, const float* act, int* ts_io, const double* dtab = nullptr) {
+MJB_DEV bool run_plugins(const DevModel& dm, const float* ctrl, float* obs, float* rew, uint8_t* term, uint8_t* trunc, int env, int copy,
+                         bool is_reset, const float* probe, int* si, float* sf, const float* act, int* ts_io, const double* dtab = nullptr,
+                         bool keep_flags = false) {
   // `env` is the REAL environment, `copy` its slot inside the (possibly packed) virtual env of this warp
   const int A = dm.a1, ab = copy * dm.a1, tb = copy * dm.t1, n_targets = dm.t1;
   // agent - target distance: from the table the warp filled lane-parallel (dist_table), or evaluated here
@@ -135,11 +150,11 @@ MJB_DEV void run_plugins(const DevModel& dm, const float* ctrl, float* obs, floa
       for (int k = 0; k < dm.store_i32; k++) if (k != MJB_STORE_I_DRAWS) si[a * dm.store_i32 + k] = 0;
       MJB_NOUNROLL
       for (int k = 0; k < dm.store_f32; k++) sf[a * dm.store_f32 + k] = 0.f;
-      rew[a] = 0.f; term[a] = 0; trunc[a] = 0;
+      if (!keep_flags) { rew[a] = 0.f; term[a] = 0; trunc[a] = 0; }
     }
-    term[A] = 0; trunc[A] = 0;
+    if (!keep_flags) { term[A] = 0; trunc[A] = 0; }
     *ts_io = 0;
-    return;
+    return false;
   }
   MJB_NOUNROLL
   for (int p = 0; p < dm.n_rewards; p++) {
@@ -194,6 +209,7 @@ MJB_DEV void run_plugins(const DevModel& dm, const float* ctrl, float* obs, floa
   for (int a = 0; a < AMAX; a++) if (a < A) { rew[a] = (float)reward[a]; term[a] = done[a] ? 1 : 0; }
   term[A] = all ? 1 : 0;
   *ts_io = ts + 1;
+  return all || tr;
 }
 
 // element i of a virtual per-copy array -> (copy, element); no division in the unpacked case
@@ -206,9 +222,17 @@ MJB_DEV void split_copy(int i, int n1, int K, int& k, int& j) {
 // environment of this warp: dm.pack real environments (venv * pack + copy) presented to the physics as one
 // model with `pack` independent copies (csrc/replicate.h); pack == 1 is the plain case.  Virtual state index i
 // of a per-copy array of length n1 maps to copy i / n1, element i % n1 of that real env's HBM row.
-template <bool PHYS, bool PACKED>
-MJB_DEV void run_env(const Ctx& c_in, const mjb_buffers& B, int venv, int num_envs, int mode, int skip_frames,
+// Auto-reset (MJB_SPEC_AUTORESET): after a step, the copies whose episode it ended run this body once more, in
+// MODE_RESET with `upd` = those copies, exactly as a masked reset of them would (same call sites: one forward pass in
+// the code, see DESIGN §4).  AUTO = false compiles the auto-reset out (the device kernels of batches without the flag);
+// with AUTO = true it follows dm.autoreset.
+template <bool PHYS, bool PACKED, bool AUTO = true>
+MJB_DEV void run_env(const Ctx& c_in, const mjb_buffers& B, int venv, int num_envs, int mode_in, int skip_frames,
                      const uint8_t* reset_mask) {
+  uint32_t fin = 0;   // 0: the pass the launch asked for; else the auto-reset pass over these copies (the step pass finished them)
+pass:
+  const bool auto_pass = fin != 0;
+  const int mode = auto_pass ? (int)MODE_RESET : mode_in;
   Ctx c = c_in;
   float* probe = c.probe;
   const DevModel& dm = *c.dm;
@@ -221,6 +245,10 @@ MJB_DEV void run_env(const Ctx& c_in, const mjb_buffers& B, int venv, int num_en
       live |= 1u << k;
       if (!(mode == MODE_RESET && reset_mask && !reset_mask[e0 + k])) upd |= 1u << k;
     }
+  if (auto_pass) {
+    upd = fin;
+    c.cta_threads = 0;   // no CTA-level alignment in forward(): the other warps do not run this pass
+  }
   if (!upd) return;
   // the loads below read the image only for copies that start from qpos0 or hold no env
   if (mode == MODE_RESET || live != (K >= 32 ? 0xffffffffu : (1u << K) - 1u)) MJB_IMG_WAIT(c);
@@ -289,6 +317,10 @@ MJB_DEV void run_env(const Ctx& c_in, const mjb_buffers& B, int venv, int num_en
     if (lane < dm.a1 * dm.store_f32) pre_sf = gsf[lane];
     if (lane == 0) pre_ts = B.timestep[e0];
   }
+  // key of a reset's draws: how the previous episode ended (its rows as the last step left them)
+  auto reset_key = [&](uint32_t env) {
+    return (uint32_t)B.timestep[env] ^ MJB_F2U(B.qpos[(size_t)env * dm.qpos_stride]) ^ (MJB_F2U(B.qvel[(size_t)env * dm.qvel_stride]) << 13);
+  };
   MJB_IMG_WAIT(c);
   MJB_G2S_WAIT();
   if (MJB_UNLIKELY(mode == MODE_RESET && dm.reset_noise > 0.f)) {
@@ -300,8 +332,7 @@ MJB_DEV void run_env(const Ctx& c_in, const mjb_buffers& B, int venv, int num_en
       const int k = K == 1 ? 0 : j / dm.njnt1;
       if (!fresh(k) || !has(k) || CI(jnt_type)[j] == MJB_JNT_FREE) continue;
       const uint32_t env = (uint32_t)(e0 + k);
-      const uint32_t ep = (uint32_t)B.timestep[env] ^ MJB_F2U(B.qpos[(size_t)env * dm.qpos_stride]) ^
-                          (MJB_F2U(B.qvel[(size_t)env * dm.qvel_stride]) << 13);
+      const uint32_t ep = reset_key(env);
       const float u = (float)(draw_u32(dm.seed ^ 0x5eedc0deULL, env, 0x4000u + (uint32_t)(j - k * dm.njnt1), ep) >> 8) * (1.f / 16777216.f);
       qpos[CI(jnt_qposadr)[j]] += dm.reset_noise * (2.f * u - 1.f);
     }
@@ -311,8 +342,7 @@ MJB_DEV void run_env(const Ctx& c_in, const mjb_buffers& B, int venv, int num_en
       split_copy(i, dm.nv1, K, k, j);
       if (!fresh(k) || !has(k)) continue;
       const uint32_t env = (uint32_t)(e0 + k);
-      const uint32_t ep = (uint32_t)B.timestep[env] ^ MJB_F2U(B.qpos[(size_t)env * dm.qpos_stride]) ^
-                          (MJB_F2U(B.qvel[(size_t)env * dm.qvel_stride]) << 13);
+      const uint32_t ep = reset_key(env);
       const float u = (float)(draw_u32(dm.seed ^ 0x5eedc0deULL, env, 0x8000u + (uint32_t)j, ep) >> 8) * (1.f / 16777216.f);
       qvel[i] = dm.reset_noise * (2.f * u - 1.f);
     }
@@ -424,8 +454,11 @@ MJB_DEV void run_env(const Ctx& c_in, const mjb_buffers& B, int venv, int num_en
       if (B.niter) B.niter[e0 + k] = niter;
     }
   }
+  // auto-reset pass, lane k < K: the key of copy k's reset draws, read before the stores below overwrite its rows
+  const uint32_t ep_k = (auto_pass && lane < K && ((upd >> lane) & 1u)) ? reset_key((uint32_t)(e0 + lane)) : 0u;
   MJB_SYNC();
   auto writes = [&](int k) { return ((upd >> k) & 1u) != 0; };
+  uint32_t ended = 0;   // copies whose episode this step ended (auto-reset)
   MJB_NOUNROLL
   for (int i = lane; i < dm.nq; i += 32) {
     int k, j;
@@ -510,23 +543,52 @@ MJB_DEV void run_env(const Ctx& c_in, const mjb_buffers& B, int venv, int num_en
     }
     MJB_SYNC();
     MJB_PH(c, PH_EPI_STAGE);
+    const uint32_t ep = auto_pass ? MJB_SHFL(ep_k, k) : 0u;
+    bool last_step = false;   // lane 0: this step ended the copy's episode
     if (lane == 0) {
+      // auto-reset: the dynamics see a random action (mjb_reset_action) in the one slot each of them reads
+      if (auto_pass) {
+        MJB_NOUNROLL
+        for (int a = 0; a < A1; a++) {
+          MJB_NOUNROLL
+          for (int p = 0; p < dm.n_dynamics; p++) {
+            const DevPlugin& dyn = dm.dynamics[p];
+            if (dyn.act_hi > dyn.act_lo)
+              s_act[a * dm.act_stride + dyn.act_lo] = reset_action(dm.seed, (uint32_t)env, (uint32_t)a, (uint32_t)dyn.act_lo, ep,
+                                                                   dm.dyn_act_low[p], dm.dyn_act_high[p]);
+          }
+        }
+      }
       // up to two agents (every level of the reference): the per-agent accumulators of the programme live in registers
       if (MJB_LIKELY(A1 <= 2))
-        run_plugins<2>(dm, SF(ctrl) + k * dm.nu1, B.obs + (size_t)env * A1 * dm.obs_stride, B.reward + (size_t)env * A1, B.term + (size_t)env * (A1 + 1),
-                       B.trunc + (size_t)env * (A1 + 1), env, k, mode == MODE_RESET, probe, s_si, s_sf, s_act, s_ts, s_dtab);
+        last_step = run_plugins<2>(dm, SF(ctrl) + k * dm.nu1, B.obs + (size_t)env * A1 * dm.obs_stride, B.reward + (size_t)env * A1, B.term + (size_t)env * (A1 + 1),
+                                   B.trunc + (size_t)env * (A1 + 1), env, k, mode == MODE_RESET, probe, s_si, s_sf, s_act, s_ts, s_dtab, auto_pass);
       else
-        run_plugins<MJB_MAX_AGENTS>(dm, SF(ctrl) + k * dm.nu1, B.obs + (size_t)env * A1 * dm.obs_stride, B.reward + (size_t)env * A1,
-                                    B.term + (size_t)env * (A1 + 1), B.trunc + (size_t)env * (A1 + 1), env, k, mode == MODE_RESET, probe, s_si, s_sf,
-                                    s_act, s_ts, s_dtab);
+        last_step = run_plugins<MJB_MAX_AGENTS>(dm, SF(ctrl) + k * dm.nu1, B.obs + (size_t)env * A1 * dm.obs_stride, B.reward + (size_t)env * A1,
+                                                B.term + (size_t)env * (A1 + 1), B.trunc + (size_t)env * (A1 + 1), env, k, mode == MODE_RESET, probe, s_si,
+                                                s_sf, s_act, s_ts, s_dtab, auto_pass);
     }
     MJB_SYNC();
     MJB_PH(c, PH_EPI_PLUG);
     for (int i = lane; i < A1 * dm.store_i32; i += 32) gsi[i] = s_si[i];
     if (lane < A1 * dm.store_f32) gsf[lane] = s_sf[lane];
     if (lane == 0) B.timestep[env] = *s_ts;
+    // (the physics-free step never auto-resets: batch creation refuses skipFrames = 0 with the flag)
+    if (AUTO && PHYS && mode == MODE_STEP && dm.autoreset && MJB_SHFL((int)last_step, 0)) {
+      // the episode's last observation, complete with lane 0's plugin columns (ordered by the MJB_SYNC above)
+      ended |= 1u << k;
+      const size_t o = (size_t)env * A1 * dm.obs_stride;
+      MJB_NOUNROLL
+      for (int i = lane; i < A1 * dm.obs_stride; i += 32) dm.final_obs[o + i] = B.obs[o + i];
+    }
   }
   MJB_PH(c, PH_EPILOGUE);
+  if (MJB_UNLIKELY(ended)) {
+    // the reset pass re-reads the rows the step pass stored: the warp barrier orders the lanes' global stores before it
+    MJB_SYNC();
+    fin = ended;
+    goto pass;
+  }
 }
 
 }  // namespace mjb

@@ -2,6 +2,7 @@
 // batch handle.  sm_100a only; there is no CPU fallback (creation fails without a device).
 #include <cuda_runtime.h>
 
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <string>
@@ -24,8 +25,9 @@ namespace mjb {
 // One CTA per SM, `warps` environments in flight per CTA; each warp walks the env index space with a grid-wide
 // stride (envs are independent: the warps only meet at the staging of the model image and at the alignment points).
 // `active` envs are walked starting at `env_base` (range launches of the host-buffer step) or through `env_ids`
-// (the env ids of one level: mjb_set_env_subset).
-template <bool PHYS, bool PACKED>
+// (the env ids of one level: mjb_set_env_subset).  AUTO: the step resets the envs it finishes (MJB_SPEC_AUTORESET), a
+// separate instantiation so that batches without the flag run exactly the code they ran before.
+template <bool PHYS, bool PACKED, bool AUTO = false>
 __global__ void __launch_bounds__(PHYS ? MJB_MAX_THREADS : 512, PHYS ? 1 : 4) k_env(const __grid_constant__ DevModel dm, const uint32_t* __restrict__ image, const mjb_buffers B,
                       int num_envs, int mode, int skip_frames, const uint8_t* __restrict__ mask,
                       const int* __restrict__ env_ids, int active, int env_base) {
@@ -67,7 +69,7 @@ __global__ void __launch_bounds__(PHYS ? MJB_MAX_THREADS : 512, PHYS ? 1 : 4) k_
       c.cta_threads = (mask == nullptr ? 32 : 0) * (busy > warps ? warps : (busy < 0 ? 0 : busy));
     }
     c.img_bar = r == 0 ? bar : nullptr;
-    if (env < nvirt) run_env<PHYS, PACKED>(c, B, env_ids ? env_ids[env] : env + env_base, num_envs, mode, skip_frames, mask);
+    if (env < nvirt) run_env<PHYS, PACKED, AUTO>(c, B, env_ids ? env_ids[env] : env + env_base, num_envs, mode, skip_frames, mask);
     if (r == 0) mbar_wait(bar, 0);   // warps that had nothing to do in the first round (or returned early) have not waited yet
     if (!PHYS) __syncthreads();
     MJB_PH(c, PH_BARRIER);
@@ -161,7 +163,8 @@ int launch(mjb_batch* b, int mode, int skip_frames, const uint8_t* mask, cudaStr
     mjb::k_env<false, false><<<b->lite_grid, b->lite_warps * 32, b->lite_smem, stream>>>(b->lite.dm, b->d_image, B, b->num_envs, mode,
                                                                                    skip_frames, mask, b->subset, active, base);
   } else {
-    auto kern = b->img.dm.pack > 1 ? mjb::k_env<true, true> : mjb::k_env<true, false>;
+    auto kern = b->img.dm.autoreset ? (b->img.dm.pack > 1 ? mjb::k_env<true, true, true> : mjb::k_env<true, false, true>)
+                                    : (b->img.dm.pack > 1 ? mjb::k_env<true, true> : mjb::k_env<true, false>);
     const int pack = b->img.dm.pack;
     const int need = ((active + pack - 1) / pack + b->warps - 1) / b->warps;
     kern<<<std::min(b->grid, std::max(1, need)), b->warps * 32, b->smem_bytes, stream>>>(
@@ -183,6 +186,10 @@ uint32_t mjb_draw_u32(uint64_t seed, uint32_t env, uint32_t agent, uint32_t coun
   return mjb::draw_u32(seed, env, agent, counter);
 }
 
+float mjb_reset_action(uint64_t seed, uint32_t env, uint32_t agent, uint32_t dim, uint32_t ep, float low, float high) {
+  return mjb::reset_action(seed, env, agent, dim, ep, low, high);
+}
+
 int mjb_batch_layout(const mjb_model* m, const mjb_env_spec* spec, int32_t num_envs, mjb_layout* out) {
   if (!m || !spec || !out || num_envs < 1) { mjb::set_error("mjb_batch_layout: bad argument"); return MJB_ERR_ARG; }
   try {
@@ -201,6 +208,18 @@ int mjb_batch_create(const mjb_model* m, const mjb_env_spec* spec, int32_t num_e
                      const mjb_buffers* buffers, mjb_batch** out) {
   if (!m || !spec || !buffers || !out || num_envs < 1) { mjb::set_error("mjb_batch_create: bad argument"); return MJB_ERR_ARG; }
   *out = nullptr;
+  if (spec->flags & MJB_SPEC_AUTORESET) {
+    if (spec->skip_frames == 0) {
+      mjb::set_error("mjb_batch_create: MJB_SPEC_AUTORESET needs skip_frames >= 1 (the physics-free step has no forward pass to reset with)");
+      return MJB_ERR_ARG;
+    }
+    if (!spec->final_obs) { mjb::set_error("mjb_batch_create: MJB_SPEC_AUTORESET needs spec.final_obs"); return MJB_ERR_ARG; }
+    for (int d = 0; d < spec->act_dim && d < 64; d++)
+      if (!(spec->act_low[d] <= spec->act_high[d]) || !std::isfinite(spec->act_low[d]) || !std::isfinite(spec->act_high[d])) {
+        mjb::set_error("mjb_batch_create: MJB_SPEC_AUTORESET needs finite act_low <= act_high");
+        return MJB_ERR_ARG;
+      }
+  }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) {
     mjb::set_error("mjb_batch_create: no CUDA device (the step path has no CPU fallback)");
@@ -250,7 +269,9 @@ int mjb_batch_create(const mjb_model* m, const mjb_env_spec* spec, int32_t num_e
   if (b->grid > sms) b->grid = sms;
   b->smem_bytes = fixed + per_env * warps;
   if (cudaFuncSetAttribute(mjb::k_env<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess ||
-      cudaFuncSetAttribute(mjb::k_env<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess) {
+      cudaFuncSetAttribute(mjb::k_env<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess ||
+      cudaFuncSetAttribute(mjb::k_env<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess ||
+      cudaFuncSetAttribute(mjb::k_env<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess) {
     mjb::set_error(std::string("cudaFuncSetAttribute(max dynamic smem) failed: ") + cudaGetErrorString(cudaGetLastError()));
     return fail(MJB_ERR_CUDA);
   }
@@ -366,6 +387,7 @@ int mjb_sync(mjb_batch* b) {
 
 int mjb_step_host(mjb_batch* b, const float* actions, float* obs, float* reward, uint8_t* term, uint8_t* trunc) {
   if (!b || !actions || !obs || !reward || !term || !trunc) { mjb::set_error("mjb_step_host: null argument"); return MJB_ERR_ARG; }
+  if (b->img.dm.autoreset) { mjb::set_error("mjb_step_host: not available on a batch created with MJB_SPEC_AUTORESET"); return MJB_ERR_ARG; }
   const mjb::DevModel& dm = b->img.dm;
   const size_t N = b->num_envs, A = dm.a1;   // agents of ONE real env (the image may pack several envs per warp)
   const size_t nb_act = sizeof(float) * N * A * dm.act_stride, nb_obs = sizeof(float) * N * A * dm.obs_stride;
@@ -504,6 +526,10 @@ int mjb_render(mjb_batch* b, const int32_t* cam_ids, int32_t ncams, int32_t widt
 
 int mjb_set_env_subset(mjb_batch* b, const int32_t* env_ids_dev, int32_t count) {
   if (!b) { mjb::set_error("mjb_set_env_subset: null batch"); return MJB_ERR_ARG; }
+  if (b->img.dm.autoreset) {
+    mjb::set_error("mjb_set_env_subset: level variants cannot auto-reset (a reset draws the env's level on the host)");
+    return MJB_ERR_ARG;
+  }
   if (!env_ids_dev) { b->subset = nullptr; b->subset_count = -1; return MJB_OK; }
   if (count < 0 || count > b->num_envs) { mjb::set_error("mjb_set_env_subset: count out of range"); return MJB_ERR_ARG; }
   if (b->img.dm.pack != 1) {

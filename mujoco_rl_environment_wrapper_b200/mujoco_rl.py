@@ -7,7 +7,8 @@ Mirrors the reference's public surface (MuJoCo_Gym/mujoco_rl.py:18-430, mujoco_p
 `timestep`, `max_steps`, `skip_frames`, `action_routing`, `agents_action_index`,
 `agents_observation_index`.
 
-New optional config keys: `num_envs` (default 1), `device`, `seed`.  Positions of the agents' bodies and of
+New optional config keys: `num_envs` (default 1), `device`, `seed`, `autoReset` (default False: `step()` resets every
+env whose episode it ends, in the same kernel launch; see `step`).  Positions of the agents' bodies and of
 the `filter_by_tag("target")` objects are exported every step (`distance`, `get_data`).  With `num_envs == 1` results are squeezed to the
 reference's shapes (numpy arrays, Python scalars); otherwise every per-agent value is a CUDA tensor
 with a leading `num_envs` dimension.  There is no CPU path: construction raises without a GPU.
@@ -74,6 +75,7 @@ class MuJoCoRL:
         self.num_envs = int(config_dict.get("num_envs", 1))
         self.seed = int(config_dict.get("seed", 1234))
         self.reset_noise = float(config_dict.get("resetNoise", 0.0))   # new, off: the reference restarts at qpos0
+        self.auto_reset = bool(config_dict.get("autoReset", False))     # new, off: the reference's loop resets by hand
         # new: names of further bodies / geoms whose positions (and orientations) are exported every step, or "all";
         # agents, "target"-tagged objects and static objects are always available to distance / get_data / data.body(n)
         self.export_positions = config_dict.get("exportPositions", [])
@@ -217,11 +219,26 @@ class MuJoCoRL:
     def __build_batch(self):
         """one spec + batch handle per level over ONE set of tensors; single-level envs keep env packing"""
         multi = len(self._levels) > 1
+        if self.auto_reset and multi:
+            raise Exception("autoReset: an xmlPath list with several levels is not supported (a reset draws the env's level "
+                            "on the host)")
+        if self.auto_reset and int(self.skip_frames) == 0:
+            raise Exception("autoReset needs skipFrames >= 1 (the physics-free step has no forward pass to reset with)")
         for lid, lv in enumerate(self._levels):
             self._use_level(lid)
             spec, keep = self.__build_spec()
             if multi:
                 spec.flags |= L.SPEC_NO_PACK
+            if self.auto_reset:
+                host = [getattr(p, "__name__", p.__class__.__name__) for p in
+                        [d for d, _, _ in self._host_dyn] + self._host_rew + self._host_done]
+                if host:
+                    raise Exception(f"autoReset: plugins that run as host code after the kernel are not supported ({host}): "
+                                    f"they would read the new episode's state of an env the step reset")
+                spec.flags |= L.SPEC_AUTORESET
+                asp = self._action_space[self.agents[0]]   # homogeneous across agents, as sample_actions assumes
+                for d in range(self._act_dim):
+                    spec.act_low[d], spec.act_high[d] = float(asp.low[d]), float(asp.high[d])
             lv["spec"], lv["target_names"], lv["probe_names"] = spec, self._target_names, self._probe_names
             with torch.cuda.device(self.device):
                 lv["batch"] = Batch(self.model, spec, self.num_envs, device=self.device, keepalive=keep,
@@ -441,7 +458,14 @@ class MuJoCoRL:
         return out
 
     def step(self, action):
-        """mujoco_rl.py:243-289 for all envs at once (one fused kernel launch)."""
+        """mujoco_rl.py:243-289 for all envs at once (one fused kernel launch).
+
+        With `autoReset`, every env whose step ends with `term["__all__"] | trunc["__all__"]` is reset in the same launch,
+        as `reset(mask=...)` would reset it, except that the dynamics see an action drawn in the kernel
+        (include/mjb.h, mjb_reset_action) and reward / term / trunc stay those of the finishing step.  The returned
+        observation of such an env is the new episode's first one; `infos[agent]["final_observation"]` holds the
+        episode's last one (valid where `infos[agent]["_final_observation"]` is set).  Per-env step counters are
+        `batch.timestep`; `self.timestep` counts calls."""
         b = self._batch
         self._load_actions(action)
         for lv in self._levels:
@@ -476,6 +500,11 @@ class MuJoCoRL:
                 terms["__all__"] = flag(b.term[:, A])   # the kernel's own OR over the agents
         self.timestep += 1
         obs = self._collect_obs(extra)
+        if self.auto_reset:
+            ended = (b.term[:, A] | b.trunc[:, A]).view(torch.bool)
+            for a, agent in enumerate(self.agents):
+                infos[agent]["final_observation"] = self._out(b.final_obs[:, a, :self._spec.obs_dim[a]])
+                infos[agent]["_final_observation"] = ended if N > 1 else bool(ended[0].item())
         if N == 1:
             rewards = {k: (v[0].item() if torch.is_tensor(v) else v) for k, v in rewards.items()}
             if not self.environment_dynamics and not self.reward_functions:

@@ -19,6 +19,8 @@ class GymnasiumWrapper:
         self.action_space = environment.action_space(agent)
 
     def step(self, action):
+        """With the environment's `autoReset`, `info` carries `final_observation` (the last observation of an episode the
+        step ended, the returned one being the next episode's first) and its mask `_final_observation`."""
         observations, rewards, terminations, truncations, infos = self.environment.step({self.agent: action})
         return observations[self.agent], rewards[self.agent], terminations[self.agent], truncations["__all__"], infos[self.agent]
 
