@@ -128,6 +128,15 @@ typedef struct mjb_env_spec {
    * [N, n_agents, obs_stride] that receives the last observation of every episode mjb_step ends; rows of other envs
    * are not written.  (A field of the spec, not of mjb_buffers, so that mjb_buffers keeps its layout.) */
   float* final_obs;
+  /* start-state pool (device memory, caller-owned, must stay valid while the batch lives): rows [n_start, nq] of qpos
+   * and [n_start, nv] of qvel of one real env.  n_start = 0: no pool, every reset starts from qpos0 / zero velocity.
+   * With a pool, every reset that would start from qpos0 (mjb_reset, full or masked, and the auto-reset of mjb_step)
+   * starts instead from pool row mjb_start_index(seed, env, ep, n_start), ep being the key reset_noise uses; the pool
+   * replaces qpos0 / zero velocity and nothing else (see mjb_reset_rows).  Level variants: give every level's handle
+   * the same pool.  mjb_batch_create refuses (MJB_ERR_ARG) n_start < 0 and n_start > 0 with a NULL pointer. */
+  const float* start_qpos;
+  const float* start_qvel;
+  int32_t n_start;
 } mjb_env_spec;
 
 /* mjb_env_spec.flags */
@@ -193,6 +202,13 @@ void mjb_batch_destroy(mjb_batch* b);
  * data_store wipe, timestep = 0, observations (dynamics applied once with `actions`, results discarded
  * from the store as mujoco_rl.py:322-328 does), reward / term / trunc = 0.  Never auto-resets. */
 int mjb_reset(mjb_batch* b, const uint8_t* mask_dev);
+/* mjb_reset, except that every masked env starts from the qpos / qvel rows it currently holds in buffers.qpos /
+ * buffers.qvel (as the caller wrote them) instead of qpos0 / zero velocity (or a pool row).  Everything else is as in
+ * mjb_reset: ctrl and warm start zeroed, one forward pass, store wiped keeping its draw counters, dynamics applied once
+ * with `actions` and discarded, timestep = 0, observations, reward / term / trunc = 0.  reset_noise is added on top
+ * (hinge / slide qpos += noise, qvel += noise, the same draws as mjb_reset), keyed by the caller's rows.  Rows are
+ * used as given, except that a free joint's quaternion is stored normalised, as every forward pass stores it. */
+int mjb_reset_rows(mjb_batch* b, const uint8_t* mask_dev);
 /* one MuJoCoRL.step for every env; reads buffers.actions, writes obs / reward / term / trunc.
  * With MJB_SPEC_AUTORESET, every env whose step sets term[n_agents] | trunc[n_agents] (the "__all__" columns) then
  * has its obs rows copied to spec.final_obs and is reset in the same launch, as mjb_reset with its mask byte set
@@ -246,6 +262,11 @@ uint32_t mjb_draw_u32(uint64_t seed, uint32_t env, uint32_t agent, uint32_t coun
  * ep = timestep ^ bits(qpos[0]) ^ (bits(qvel[0]) << 13) of the env's rows as the finishing step left them (the key
  * reset_noise uses); low / high = act_low[dim] / act_high[dim] of the spec */
 float mjb_reset_action(uint64_t seed, uint32_t env, uint32_t agent, uint32_t dim, uint32_t ep, float low, float high);
+/* the pool row a reset of `env` starts from (spec.n_start > 0), in [0, n_start):
+ *   p = (mjb_draw_u32(seed ^ 0x5eedc0de, env, 0xD000, ep) * (uint64_t)n_start) >> 32
+ * ep = the reset_noise / mjb_reset_action key of the env's rows before the reset.  Each env of a packed warp draws its
+ * own row.  Returns 0 for n_start < 1. */
+uint32_t mjb_start_index(uint64_t seed, uint32_t env, uint32_t ep, int32_t n_start);
 
 #ifdef __cplusplus
 }

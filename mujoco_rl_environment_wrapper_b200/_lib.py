@@ -49,6 +49,7 @@ class EnvSpec(ctypes.Structure):
         ("solver_iterations", ctypes.c_int32), ("ls_iterations", ctypes.c_int32), ("flags", ctypes.c_int32), ("reset_noise", ctypes.c_float),
         ("n_extra_probes", ctypes.c_int32), ("extra_objtype", ctypes.c_int32 * MAX_EXTRA_PROBES), ("extra_objid", ctypes.c_int32 * MAX_EXTRA_PROBES),
         ("act_low", ctypes.c_float * 64), ("act_high", ctypes.c_float * 64), ("final_obs", ctypes.c_void_p),
+        ("start_qpos", ctypes.c_void_p), ("start_qvel", ctypes.c_void_p), ("n_start", ctypes.c_int32),
     ]
 
 
@@ -102,6 +103,7 @@ def load(build_if_missing=True):
     lib.mjb_batch_destroy.argtypes = [vp]
     lib.mjb_batch_destroy.restype = None
     lib.mjb_reset.argtypes = [vp, vp]
+    lib.mjb_reset_rows.argtypes = [vp, vp]
     lib.mjb_step.argtypes = [vp]
     lib.mjb_physics.argtypes = [vp, i32]
     lib.mjb_forward.argtypes = [vp]
@@ -120,6 +122,8 @@ def load(build_if_missing=True):
     lib.mjb_reset_action.restype = ctypes.c_float
     lib.mjb_reset_action.argtypes = [ctypes.c_uint64, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32,
                                      ctypes.c_float, ctypes.c_float]
+    lib.mjb_start_index.restype = ctypes.c_uint32
+    lib.mjb_start_index.argtypes = [ctypes.c_uint64, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int32]
     _LIB = lib
     return lib
 

@@ -13,9 +13,11 @@ from . import _lib as L
 
 
 class Batch:
-    def __init__(self, model: "L.Model", spec: "L.EnvSpec", num_envs: int, device=None, keepalive=(), share=None, probe_quat=False):
+    def __init__(self, model: "L.Model", spec: "L.EnvSpec", num_envs: int, device=None, keepalive=(), share=None, probe_quat=False,
+                 start_states=None):
         """`share`: another Batch whose tensors this handle steps as well (level variants, see set_subset);
-        the two models must produce the same buffer layout."""
+        the two models must produce the same buffer layout.  `start_states`: (qpos [P, nq], qvel [P, nv]) float32 CUDA
+        tensors, a pool every reset draws its start state from (include/mjb.h, mjb_env_spec.start_qpos)."""
         self._lib = L.load()
         if not torch.cuda.is_available():
             raise RuntimeError("mujoco_rl_environment_wrapper_b200: no CUDA device — the step path is CUDA-only "
@@ -52,6 +54,15 @@ class Batch:
             self.final_obs = z((N, max(1, A), lay.obs_stride), f32)
             spec = L.EnvSpec.from_buffer_copy(spec)   # the caller's spec stays as it was
             spec.final_obs = self.final_obs.data_ptr()
+        if start_states is not None:
+            qp, qv = (t.to(device=dev, dtype=f32).contiguous() for t in start_states)
+            if qp.dim() != 2 or qv.dim() != 2 or qp.shape[0] < 1 or qv.shape[0] != qp.shape[0] or \
+                    qp.shape[1] != model.dims.nq or qv.shape[1] != model.dims.nv:
+                raise Exception(f"start_states: expected qpos [P, {model.dims.nq}] and qvel [P, {model.dims.nv}] with P >= 1, "
+                                f"got {tuple(qp.shape)} and {tuple(qv.shape)}")
+            self.start_states = (qp, qv)   # kept alive: the library reads them at every reset
+            spec = L.EnvSpec.from_buffer_copy(spec)
+            spec.start_qpos, spec.start_qvel, spec.n_start = qp.data_ptr(), qv.data_ptr(), int(qp.shape[0])
         B = L.Buffers()
         for k, v in self.buf.items():
             setattr(B, k, v.data_ptr())
@@ -79,12 +90,18 @@ class Batch:
         raise AttributeError(k)
 
     # ---- device-side entry points (asynchronous on self.stream)
+    def _mask_ptr(self, mask):
+        if mask is None:
+            return None
+        self._mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
+        return ctypes.c_void_p(self._mask.data_ptr())
+
     def reset(self, mask=None):
-        p = None
-        if mask is not None:
-            self._mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
-            p = ctypes.c_void_p(self._mask.data_ptr())
-        L.check(self._lib.mjb_reset(self._h, p), "reset")
+        L.check(self._lib.mjb_reset(self._h, self._mask_ptr(mask)), "reset")
+
+    def reset_rows(self, mask=None):
+        """reset the masked envs (None = all) from the qpos / qvel rows they hold (include/mjb.h, mjb_reset_rows)"""
+        L.check(self._lib.mjb_reset_rows(self._h, self._mask_ptr(mask)), "reset_rows")
 
     def step(self):
         L.check(self._lib.mjb_step(self._h), "step")

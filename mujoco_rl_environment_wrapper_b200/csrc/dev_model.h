@@ -159,6 +159,12 @@ struct DevModel {
   float* final_obs;    // [N, A, obs_stride] (mjb_env_spec.final_obs)
   int autoreset;
   float dyn_act_low[4], dyn_act_high[4];
+  // start-state pool (mjb_env_spec.start_qpos / start_qvel / n_start): rows of one real env, nq1 / nv1 floats each.
+  // 32 bytes, padded for the same reason as the auto-reset fields above.
+  const float* start_qpos;
+  const float* start_qvel;
+  int n_start;
+  int start_pad[3];
 };
 
 // ---- camera rendering (render_kernel.cuh): a second, small constant table next to the image -------------

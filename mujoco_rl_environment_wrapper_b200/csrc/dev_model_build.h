@@ -437,6 +437,8 @@ inline void build_dev_model(const ModelView& m, const mjb_env_spec& spec, DevIma
       dm.dyn_act_low[i] = spec.act_low[d]; dm.dyn_act_high[i] = spec.act_high[d];
     }
   }
+  if (spec.n_start < 0) throw std::runtime_error("n_start < 0");
+  if (spec.n_start > 0) { dm.start_qpos = spec.start_qpos; dm.start_qvel = spec.start_qvel; dm.n_start = spec.n_start; }
   for (int i = 0; i < spec.n_rewards; i++) cp(dm.rewards[i], spec.rewards[i]);
   for (int i = 0; i < spec.n_dones; i++) cp(dm.dones[i], spec.dones[i]);
   std::vector<int> pk, pid;

@@ -14,7 +14,8 @@
 
 namespace mjb {
 
-enum { MODE_STEP = 0, MODE_PHYSICS = 1, MODE_FORWARD = 2, MODE_RESET = 3 };
+// MODE_RESET_ROWS: MODE_RESET with the masked envs starting from their own qpos / qvel rows (mjb_reset_rows)
+enum { MODE_STEP = 0, MODE_PHYSICS = 1, MODE_FORWARD = 2, MODE_RESET = 3, MODE_RESET_ROWS = 4 };
 
 // agent loops of run_plugins: unrolled when the bound is small (registers), rolled in the general form (code size)
 #if defined(MJB_HOST_EMU)
@@ -43,6 +44,11 @@ MJB_HD float reset_action(unsigned long long seed, uint32_t env, uint32_t agent,
   volatile float span = u * (high - low);
   return low + span;
 #endif
+}
+
+// the start-state pool row of a reset (include/mjb.h, mjb_start_index), keyed like reset_noise
+MJB_HD uint32_t start_index(unsigned long long seed, uint32_t env, uint32_t ep, int n_start) {
+  return n_start < 1 ? 0u : (uint32_t)(((unsigned long long)draw_u32(seed ^ 0x5eedc0deULL, env, 0xD000u, ep) * (uint32_t)n_start) >> 32);
 }
 
 // Distances, the reward arithmetic and the done comparison run in fp64 on the fp32 positions (the reference computes
@@ -224,15 +230,18 @@ MJB_DEV void split_copy(int i, int n1, int K, int& k, int& j) {
 // of a per-copy array of length n1 maps to copy i / n1, element i % n1 of that real env's HBM row.
 // Auto-reset (MJB_SPEC_AUTORESET): after a step, the copies whose episode it ended run this body once more, in
 // MODE_RESET with `upd` = those copies, exactly as a masked reset of them would (same call sites: one forward pass in
-// the code, see DESIGN §4).  AUTO = false compiles the auto-reset out (the device kernels of batches without the flag);
-// with AUTO = true it follows dm.autoreset.
-template <bool PHYS, bool PACKED, bool AUTO = true>
+// the code, see DESIGN §4).  Start states (DESIGN §5d): a reset's fresh copies load the start-state pool row they draw
+// (dm.n_start > 0) or, in MODE_RESET_ROWS, their own rows, instead of qpos0 / zero velocity.
+// EXT = false compiles auto-reset and start states out (the device kernels of batches and launches that use neither);
+// with EXT = true they follow dm.autoreset, dm.n_start and the mode.
+template <bool PHYS, bool PACKED, bool EXT = true>
 MJB_DEV void run_env(const Ctx& c_in, const mjb_buffers& B, int venv, int num_envs, int mode_in, int skip_frames,
                      const uint8_t* reset_mask) {
   uint32_t fin = 0;   // 0: the pass the launch asked for; else the auto-reset pass over these copies (the step pass finished them)
 pass:
   const bool auto_pass = fin != 0;
-  const int mode = auto_pass ? (int)MODE_RESET : mode_in;
+  const bool own_rows = EXT && mode_in == MODE_RESET_ROWS;
+  const int mode = (auto_pass || own_rows) ? (int)MODE_RESET : mode_in;
   Ctx c = c_in;
   float* probe = c.probe;
   const DevModel& dm = *c.dm;
@@ -253,13 +262,29 @@ pass:
   // the loads below read the image only for copies that start from qpos0 or hold no env
   if (mode == MODE_RESET || live != (K >= 32 ? 0xffffffffu : (1u << K) - 1u)) MJB_IMG_WAIT(c);
   float *qpos = SF(qpos), *qvel = SF(qvel), *qacc = SF(qacc), *ctrl = SF(ctrl), *sens = SF(sens);
-  auto fresh = [&](int k) { return mode == MODE_RESET && ((upd >> k) & 1u); };   // copy starts from qpos0
+  auto fresh = [&](int k) { return mode == MODE_RESET && ((upd >> k) & 1u); };   // copy starts from qpos0 (or a start state)
   auto has = [&](int k) { return ((live >> k) & 1u) != 0; };
+  // key of a reset's draws: how the previous episode ended (its rows as the last step left them)
+  auto reset_key = [&](uint32_t env) {
+    return (uint32_t)B.timestep[env] ^ MJB_F2U(B.qpos[(size_t)env * dm.qpos_stride]) ^ (MJB_F2U(B.qvel[(size_t)env * dm.qvel_stride]) << 13);
+  };
+  // start states: fresh copies load their own rows (own_rows) or the pool row pr[k] they draw, before any row is stored
+  const bool pool = EXT && mode == MODE_RESET && !own_rows && dm.n_start > 0, from_start = own_rows || pool;
+  uint32_t pr[MJB_MAX_PACK] = {0, 0, 0, 0};
+  if (pool) {
+#pragma unroll
+    for (int k = 0; k < MJB_MAX_PACK; k++)
+      if (k < K && fresh(k)) pr[k] = start_index(dm.seed, (uint32_t)(e0 + k), reset_key((uint32_t)(e0 + k)), dm.n_start);
+  }
+  auto pool_row = [&](const float* base, int n1, int k) {   // constant indices into pr: it stays in registers
+    return base + (size_t)(K == 1 || k == 0 ? pr[0] : k == 1 ? pr[1] : k == 2 ? pr[2] : pr[3]) * n1;
+  };
   MJB_NOUNROLL
   for (int i = lane; i < dm.nq; i += 32) {
     int k, j;
     split_copy(i, dm.nq1, K, k, j);
-    if (fresh(k) || !has(k)) qpos[i] = CF(qpos0)[i];
+    if (from_start && fresh(k)) MJB_G2S(&qpos[i], pool ? pool_row(dm.start_qpos, dm.nq1, k) + j : &B.qpos[(size_t)(e0 + k) * dm.qpos_stride + j]);
+    else if (fresh(k) || !has(k)) qpos[i] = CF(qpos0)[i];
     else MJB_G2S(&qpos[i], &B.qpos[(size_t)(e0 + k) * dm.qpos_stride + j]);
   }
   MJB_NOUNROLL
@@ -267,7 +292,10 @@ pass:
     int k, j;
     split_copy(i, dm.nv1, K, k, j);
     bool z = fresh(k) || !has(k);
-    if (z) { qvel[i] = 0.f; qacc[i] = 0.f; }
+    if (from_start && fresh(k)) {
+      MJB_G2S(&qvel[i], pool ? pool_row(dm.start_qvel, dm.nv1, k) + j : &B.qvel[(size_t)(e0 + k) * dm.qvel_stride + j]);
+      qacc[i] = 0.f;
+    } else if (z) { qvel[i] = 0.f; qacc[i] = 0.f; }
     else {
       MJB_G2S(&qvel[i], &B.qvel[(size_t)(e0 + k) * dm.qvel_stride + j]);
       MJB_G2S(&qacc[i], &B.warmstart[(size_t)(e0 + k) * dm.qvel_stride + j]);
@@ -317,10 +345,6 @@ pass:
     if (lane < dm.a1 * dm.store_f32) pre_sf = gsf[lane];
     if (lane == 0) pre_ts = B.timestep[e0];
   }
-  // key of a reset's draws: how the previous episode ended (its rows as the last step left them)
-  auto reset_key = [&](uint32_t env) {
-    return (uint32_t)B.timestep[env] ^ MJB_F2U(B.qpos[(size_t)env * dm.qpos_stride]) ^ (MJB_F2U(B.qvel[(size_t)env * dm.qvel_stride]) << 13);
-  };
   MJB_IMG_WAIT(c);
   MJB_G2S_WAIT();
   if (MJB_UNLIKELY(mode == MODE_RESET && dm.reset_noise > 0.f)) {
@@ -344,7 +368,8 @@ pass:
       const uint32_t env = (uint32_t)(e0 + k);
       const uint32_t ep = reset_key(env);
       const float u = (float)(draw_u32(dm.seed ^ 0x5eedc0deULL, env, 0x8000u + (uint32_t)j, ep) >> 8) * (1.f / 16777216.f);
-      qvel[i] = dm.reset_noise * (2.f * u - 1.f);
+      const float d = dm.reset_noise * (2.f * u - 1.f);
+      qvel[i] = EXT ? qvel[i] + d : d;   // start velocity + noise (0 + d == d: the same bits without a start state)
     }
   }
   MJB_SYNC();
@@ -574,7 +599,7 @@ pass:
     if (lane < A1 * dm.store_f32) gsf[lane] = s_sf[lane];
     if (lane == 0) B.timestep[env] = *s_ts;
     // (the physics-free step never auto-resets: batch creation refuses skipFrames = 0 with the flag)
-    if (AUTO && PHYS && mode == MODE_STEP && dm.autoreset && MJB_SHFL((int)last_step, 0)) {
+    if (EXT && PHYS && mode == MODE_STEP && dm.autoreset && MJB_SHFL((int)last_step, 0)) {
       // the episode's last observation, complete with lane 0's plugin columns (ordered by the MJB_SYNC above)
       ended |= 1u << k;
       const size_t o = (size_t)env * A1 * dm.obs_stride;

@@ -25,9 +25,10 @@ namespace mjb {
 // One CTA per SM, `warps` environments in flight per CTA; each warp walks the env index space with a grid-wide
 // stride (envs are independent: the warps only meet at the staging of the model image and at the alignment points).
 // `active` envs are walked starting at `env_base` (range launches of the host-buffer step) or through `env_ids`
-// (the env ids of one level: mjb_set_env_subset).  AUTO: the step resets the envs it finishes (MJB_SPEC_AUTORESET), a
-// separate instantiation so that batches without the flag run exactly the code they ran before.
-template <bool PHYS, bool PACKED, bool AUTO = false>
+// (the env ids of one level: mjb_set_env_subset).  EXT: the step resets the envs it finishes (MJB_SPEC_AUTORESET) and
+// resets start from start states (pool or the caller's rows), a separate instantiation so that batches and launches that
+// use neither run exactly the code they ran before.
+template <bool PHYS, bool PACKED, bool EXT = false>
 __global__ void __launch_bounds__(PHYS ? MJB_MAX_THREADS : 512, PHYS ? 1 : 4) k_env(const __grid_constant__ DevModel dm, const uint32_t* __restrict__ image, const mjb_buffers B,
                       int num_envs, int mode, int skip_frames, const uint8_t* __restrict__ mask,
                       const int* __restrict__ env_ids, int active, int env_base) {
@@ -69,7 +70,7 @@ __global__ void __launch_bounds__(PHYS ? MJB_MAX_THREADS : 512, PHYS ? 1 : 4) k_
       c.cta_threads = (mask == nullptr ? 32 : 0) * (busy > warps ? warps : (busy < 0 ? 0 : busy));
     }
     c.img_bar = r == 0 ? bar : nullptr;
-    if (env < nvirt) run_env<PHYS, PACKED, AUTO>(c, B, env_ids ? env_ids[env] : env + env_base, num_envs, mode, skip_frames, mask);
+    if (env < nvirt) run_env<PHYS, PACKED, EXT>(c, B, env_ids ? env_ids[env] : env + env_base, num_envs, mode, skip_frames, mask);
     if (r == 0) mbar_wait(bar, 0);   // warps that had nothing to do in the first round (or returned early) have not waited yet
     if (!PHYS) __syncthreads();
     MJB_PH(c, PH_BARRIER);
@@ -163,8 +164,9 @@ int launch(mjb_batch* b, int mode, int skip_frames, const uint8_t* mask, cudaStr
     mjb::k_env<false, false><<<b->lite_grid, b->lite_warps * 32, b->lite_smem, stream>>>(b->lite.dm, b->d_image, B, b->num_envs, mode,
                                                                                    skip_frames, mask, b->subset, active, base);
   } else {
-    auto kern = b->img.dm.autoreset ? (b->img.dm.pack > 1 ? mjb::k_env<true, true, true> : mjb::k_env<true, false, true>)
-                                    : (b->img.dm.pack > 1 ? mjb::k_env<true, true> : mjb::k_env<true, false>);
+    const bool ext = b->img.dm.autoreset || mode == mjb::MODE_RESET_ROWS || (mode == mjb::MODE_RESET && b->img.dm.n_start > 0);
+    auto kern = ext ? (b->img.dm.pack > 1 ? mjb::k_env<true, true, true> : mjb::k_env<true, false, true>)
+                    : (b->img.dm.pack > 1 ? mjb::k_env<true, true> : mjb::k_env<true, false>);
     const int pack = b->img.dm.pack;
     const int need = ((active + pack - 1) / pack + b->warps - 1) / b->warps;
     kern<<<std::min(b->grid, std::max(1, need)), b->warps * 32, b->smem_bytes, stream>>>(
@@ -188,6 +190,10 @@ uint32_t mjb_draw_u32(uint64_t seed, uint32_t env, uint32_t agent, uint32_t coun
 
 float mjb_reset_action(uint64_t seed, uint32_t env, uint32_t agent, uint32_t dim, uint32_t ep, float low, float high) {
   return mjb::reset_action(seed, env, agent, dim, ep, low, high);
+}
+
+uint32_t mjb_start_index(uint64_t seed, uint32_t env, uint32_t ep, int32_t n_start) {
+  return mjb::start_index(seed, env, ep, n_start);
 }
 
 int mjb_batch_layout(const mjb_model* m, const mjb_env_spec* spec, int32_t num_envs, mjb_layout* out) {
@@ -219,6 +225,11 @@ int mjb_batch_create(const mjb_model* m, const mjb_env_spec* spec, int32_t num_e
         mjb::set_error("mjb_batch_create: MJB_SPEC_AUTORESET needs finite act_low <= act_high");
         return MJB_ERR_ARG;
       }
+  }
+  if (spec->n_start < 0) { mjb::set_error("mjb_batch_create: spec.n_start < 0"); return MJB_ERR_ARG; }
+  if (spec->n_start > 0 && (!spec->start_qpos || !spec->start_qvel)) {
+    mjb::set_error("mjb_batch_create: spec.n_start > 0 needs spec.start_qpos and spec.start_qvel");
+    return MJB_ERR_ARG;
   }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) {
@@ -366,6 +377,10 @@ void mjb_batch_destroy(mjb_batch* b) {
 int mjb_reset(mjb_batch* b, const uint8_t* mask_dev) {
   if (!b) { mjb::set_error("mjb_reset: null batch"); return MJB_ERR_ARG; }
   return launch(b, mjb::MODE_RESET, 0, mask_dev);
+}
+int mjb_reset_rows(mjb_batch* b, const uint8_t* mask_dev) {
+  if (!b) { mjb::set_error("mjb_reset_rows: null batch"); return MJB_ERR_ARG; }
+  return launch(b, mjb::MODE_RESET_ROWS, 0, mask_dev);
 }
 int mjb_step(mjb_batch* b) {
   if (!b) { mjb::set_error("mjb_step: null batch"); return MJB_ERR_ARG; }

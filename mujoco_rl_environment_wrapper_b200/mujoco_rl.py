@@ -8,7 +8,8 @@ Mirrors the reference's public surface (MuJoCo_Gym/mujoco_rl.py:18-430, mujoco_p
 `agents_observation_index`.
 
 New optional config keys: `num_envs` (default 1), `device`, `seed`, `autoReset` (default False: `step()` resets every
-env whose episode it ends, in the same kernel launch; see `step`).  Positions of the agents' bodies and of
+env whose episode it ends, in the same kernel launch; see `step`), `startStates` ({"qpos": [P, nq], "qvel": [P, nv]}:
+every reset starts from a pool row drawn per env and reset instead of qpos0; see `reset`).  Positions of the agents' bodies and of
 the `filter_by_tag("target")` objects are exported every step (`distance`, `get_data`).  With `num_envs == 1` results are squeezed to the
 reference's shapes (numpy arrays, Python scalars); otherwise every per-agent value is a CUDA tensor
 with a leading `num_envs` dimension.  There is no CPU path: construction raises without a GPU.
@@ -52,6 +53,32 @@ class AgentStore(dict):
         if col is None:
             raise KeyError(key)
         return col if self._env.num_envs > 1 else col[0].item()
+
+
+def state_rows(what, v, rows, width, device):
+    """float32 tensor [rows, width] on `device` from a numpy array or tensor; rows = None: any count >= 1; with rows = 1
+    a single row [width] is accepted too"""
+    t = (v if torch.is_tensor(v) else torch.as_tensor(np.asarray(v, dtype=np.float32))).to(device, torch.float32)
+    if rows == 1 and t.dim() == 1:
+        t = t.reshape(1, -1)
+    if t.dim() != 2 or t.shape[1] != width or (rows is None and t.shape[0] < 1) or (rows is not None and t.shape[0] != rows):
+        want = f"[{'P >= 1' if rows is None else rows}, {width}]" + (f" (or [{width}])" if rows == 1 else "")
+        raise Exception(f"{what}: expected shape {want}, got {tuple(t.shape)}")
+    return t.contiguous()
+
+
+def parse_start_states(cfg, nq, nv, device):
+    """config "startStates" {"qpos": [P, nq], "qvel": [P, nv] (optional, zeros)} -> (qpos, qvel) tensors, or None"""
+    if cfg is None:
+        return None
+    if not isinstance(cfg, dict) or cfg.get("qpos") is None:
+        raise Exception('startStates: expected {"qpos": [P, nq], "qvel": [P, nv] (optional)}')
+    qpos = state_rows("startStates['qpos']", cfg["qpos"], None, nq, device)
+    qvel = state_rows("startStates['qvel']", cfg["qvel"], qpos.shape[0], nv, device) if cfg.get("qvel") is not None \
+        else torch.zeros((qpos.shape[0], nv), dtype=torch.float32, device=device)
+    if not bool(torch.isfinite(qpos).all() and torch.isfinite(qvel).all()):
+        raise Exception("startStates: qpos / qvel must be finite")
+    return qpos, qvel
 
 
 class MuJoCoRL:
@@ -118,6 +145,7 @@ class MuJoCoRL:
                                 f"(the reference builds its index tables once and reuses them for every level)")
         self._first_level = self._level_paths.index(random.choice(self._level_paths)) if self.num_envs == 1 else 0
         self._use_level(self._first_level)
+        self._start_states = parse_start_states(config_dict.get("startStates"), self.model.nq, self.model.nv, self.device)
         self.agents_action_index = self._tables.agents_action_index
         self.agents_observation_index = self._tables.agents_observation_index
 
@@ -242,7 +270,8 @@ class MuJoCoRL:
             lv["spec"], lv["target_names"], lv["probe_names"] = spec, self._target_names, self._probe_names
             with torch.cuda.device(self.device):
                 lv["batch"] = Batch(self.model, spec, self.num_envs, device=self.device, keepalive=keep,
-                                    share=self._levels[0]["batch"] if lid else None, probe_quat=self.export_orientation)
+                                    share=self._levels[0]["batch"] if lid else None, probe_quat=self.export_orientation,
+                                    start_states=self._start_states)
         self._use_level(0)
         self._spec, self._batch = self._levels[0]["spec"], self._levels[0]["batch"]
         self.level_id = torch.zeros(self.num_envs, dtype=torch.int32, device=self.device)
@@ -514,13 +543,34 @@ class MuJoCoRL:
         return obs, rewards, terms, truncs, infos
 
     def reset(self, *, seed=None, options=None, mask=None):
-        """mujoco_rl.py:291-331.  `mask` (bool[N]) resets a subset of envs (new; the reference has one env)."""
+        """mujoco_rl.py:291-331.  `mask` (bool[N]) resets a subset of envs (new; the reference has one env).
+
+        `options={"qpos": ..., "qvel": ...}` (new) starts the reset envs from these rows instead of qpos0 / zero velocity
+        (or a `startStates` row): [N, nq] / [N, nv] for N > 1, [nq] / [nv] for N = 1; `qvel` defaults to zeros.  Rows of
+        envs outside `mask` are ignored.  Everything else is an ordinary reset (include/mjb.h, mjb_reset_rows); rows are
+        used as given (a free joint's quaternion comes back normalised, as after any forward pass)."""
         b = self._batch
+        rows = options is not None and options.get("qpos") is not None
+        if options is not None and not rows and options.get("qvel") is not None:
+            raise Exception("reset(options=...): 'qvel' needs 'qpos'")
+        if rows:
+            N, nq, nv = self.num_envs, self.model.nq, self.model.nv
+            qpos = state_rows("reset(options['qpos'])", options["qpos"], N, nq, self.device)
+            qvel = state_rows("reset(options['qvel'])", options["qvel"], N, nv, self.device) if options.get("qvel") is not None \
+                else torch.zeros((N, nv), dtype=torch.float32, device=self.device)
+            if mask is None:
+                b.qpos[:, :nq], b.qvel[:, :nv] = qpos, qvel
+            else:
+                m = mask.to(device=self.device, dtype=torch.bool).reshape(-1)
+                b.qpos[m, :nq], b.qvel[m, :nv] = qpos[m], qvel[m]
         b.actions[:, :, :self._act_dim] = self.sample_actions()  # the reference applies dynamics once with a sampled action
         if len(self._levels) > 1:
             self._draw_levels(mask)
         for lv in self._levels:
-            lv["batch"].reset(mask)
+            if rows:
+                lv["batch"].reset_rows(mask)
+            else:
+                lv["batch"].reset(mask)
         for st in self.data_store.values():
             st.clear()
         infos = {agent: {dyn.__class__.__name__: {} for dyn in self._fused_dyn} for agent in self.agents}

@@ -25,7 +25,8 @@ class GymnasiumWrapper:
         return observations[self.agent], rewards[self.agent], terminations[self.agent], truncations["__all__"], infos[self.agent]
 
     def reset(self, *, seed=1, options=None):
-        observations, infos = self.environment.reset()
+        """`options`: passed to the environment's reset, e.g. {"qpos": ..., "qvel": ...} to start from a given state."""
+        observations, infos = self.environment.reset(options=options)
         return observations[self.agent], infos
 
     def render(self):
