@@ -62,6 +62,20 @@ int mjb_name2id(const mjb_model* m, int objtype, const char* name);
 const char* mjb_id2name(const mjb_model* m, int objtype, int id);
 const char* mjb_last_error(void);
 const char* mjb_version(void);
+/* row layout of a per-env parameter table (mjb_env_spec.params) for this model: offsets (in floats) of the five fields
+ * in a row, and the row length */
+typedef struct mjb_param_offsets {
+  int32_t body_mass, body_inertia, geom_friction, actuator_gear, dof_damping;
+  int32_t n_params;
+} mjb_param_offsets;
+int mjb_param_layout(const mjb_model* m, mjb_param_offsets* out);
+/* overwrite the fp64 field `name` (count values, the field's full length) of the model, as MuJoCo's
+ * `model.body_mass[:] = x` does: nothing mj_setConst derives from it is recomputed (body / dof invweight0, subtree
+ * masses ...).  `geom_friction` is the one exception: MuJoCo mixes a contact's friction from the geoms' values at
+ * collision time, and this model stores that mix per collision pair (pair_friction, the elementwise max of the two
+ * geoms'), so setting geom_friction mixes pair_friction again.  Batches created afterwards use the new values.
+ * MJB_ERR_ARG for an unknown name, an int field or a wrong count. */
+int mjb_model_set_field(mjb_model* m, const char* name, const double* values, int32_t count);
 
 /* ---- per-step plugin programme (the reference's plugin lists re-expressed as data) --------- */
 enum {
@@ -137,13 +151,34 @@ typedef struct mjb_env_spec {
   const float* start_qpos;
   const float* start_qvel;
   int32_t n_start;
+  /* per-env physical parameters (device memory, caller-owned, must stay valid while the batch lives): rows
+   * [N, n_params] of fp32, laid out as mjb_param_layout says, in MuJoCo id order: body_mass [nbody], body_inertia
+   * [nbody, 3] (principal), geom_friction [ngeom] (sliding), actuator_gear [nu] (gear[0]), dof_damping [nv].  NULL: no
+   * table, every env uses the model's values.  With a table, env n steps exactly as an env of a model whose five fields
+   * hold row n would; a contact's friction is max(geom_friction[g1], geom_friction[g2]).  What MuJoCo derives from these
+   * fields in mj_setConst keeps its nominal value (body / dof invweight0 and with them the contact and limit
+   * regularisers, subtree masses), as after editing model.body_mass in MuJoCo without calling mj_setConst.  Entries of
+   * static bodies (and of the world body) are ignored.  Rows persist: the caller may write them between launches and the
+   * next launch uses them.
+   * MJB_SPEC_RANDOMIZE: every reset (mjb_reset, full or masked, mjb_reset_rows and the auto-reset of mjb_step)
+   * overwrites the row of every env it resets with nominal * s before the env's forward pass, s = mjb_param_scale(seed,
+   * env, family, index, ep, param_lo[family], param_hi[family]) drawn per element (index: the MuJoCo body / geom /
+   * actuator / dof id; a body's three inertia entries take its mass's s); families 0 body_mass + body_inertia,
+   * 1 geom_friction, 2 actuator_gear, 3 dof_damping.  Entries of static bodies are not written.  Level variants: give
+   * every level's handle the same table; rows hold values, not scales, so when the caller moves an env to another
+   * level it writes that env's row (MuJoCoRL writes the new level's nominal values unless it randomises).  mjb_batch_create refuses (MJB_ERR_ARG) MJB_SPEC_RANDOMIZE without a table,
+   * non-finite ranges, lo > hi, lo < 0 (lo <= 0 for family 0), and a table with skip_frames = 0. */
+  float* params;
+  float param_lo[4], param_hi[4];
 } mjb_env_spec;
 
 /* mjb_env_spec.flags */
 enum {
   MJB_SPEC_NO_PACK = 1,   /* one env per warp even for small models (needed by mjb_set_env_subset) */
-  MJB_SPEC_AUTORESET = 2  /* mjb_step resets every env whose step ends its episode, in the same launch (see mjb_step) */
+  MJB_SPEC_AUTORESET = 2, /* mjb_step resets every env whose step ends its episode, in the same launch (see mjb_step) */
+  MJB_SPEC_RANDOMIZE = 4  /* every reset draws the env's row of spec.params (see mjb_env_spec.params) */
 };
+
 
 /* Caller-owned device buffers (torch CUDA tensors on the Python side).  Row-major, env-major;
  * strides are in elements and come from mjb_batch_layout. Optional pointers may be NULL. */
@@ -267,6 +302,11 @@ float mjb_reset_action(uint64_t seed, uint32_t env, uint32_t agent, uint32_t dim
  * ep = the reset_noise / mjb_reset_action key of the env's rows before the reset.  Each env of a packed warp draws its
  * own row.  Returns 0 for n_start < 1. */
 uint32_t mjb_start_index(uint64_t seed, uint32_t env, uint32_t ep, int32_t n_start);
+/* the scale a randomising reset (MJB_SPEC_RANDOMIZE) applies to element `index` of parameter family `family` (0..3):
+ *   u = (mjb_draw_u32(seed ^ 0x5eedc0de, env, 0x10000 + 0x1000 * family + index, ep) >> 8) * 2^-24
+ *   s = lo + u * (hi - lo)     (fp32, each operation rounded to nearest, no fused multiply-add)
+ * the new value is nominal * s (fp32).  ep = the reset_noise / mjb_reset_action key of the env's rows before the reset. */
+float mjb_param_scale(uint64_t seed, uint32_t env, int32_t family, uint32_t index, uint32_t ep, float lo, float hi);
 
 #ifdef __cplusplus
 }

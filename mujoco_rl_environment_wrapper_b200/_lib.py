@@ -11,7 +11,10 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MJB_LIB") or os.path.join(_HERE, "libmjb.so")
 
 MAX_AGENTS, MAX_PLUGINS, MAX_TARGETS, MAX_EXTRA_PROBES = 8, 4, 16, 48
-SPEC_NO_PACK, SPEC_AUTORESET = 1, 2   # mjb_env_spec.flags
+SPEC_NO_PACK, SPEC_AUTORESET, SPEC_RANDOMIZE = 1, 2, 4   # mjb_env_spec.flags
+# per-env parameter table (include/mjb.h, mjb_env_spec.params): the fields of a row, and the randomisation family of each
+PARAM_FIELDS = ("body_mass", "body_inertia", "geom_friction", "actuator_gear", "dof_damping")
+PARAM_FAMILIES = ("body_mass", "geom_friction", "actuator_gear", "dof_damping")
 OBJ_BODY, OBJ_JOINT, OBJ_GEOM, OBJ_SITE, OBJ_CAMERA, OBJ_ACTUATOR, OBJ_SENSOR = 1, 3, 5, 6, 7, 19, 20
 DYN_LANGUAGE, DYN_PICKUP = 1, 2
 REW_TAG_DISTANCE, REW_ANT = 1, 2
@@ -50,7 +53,12 @@ class EnvSpec(ctypes.Structure):
         ("n_extra_probes", ctypes.c_int32), ("extra_objtype", ctypes.c_int32 * MAX_EXTRA_PROBES), ("extra_objid", ctypes.c_int32 * MAX_EXTRA_PROBES),
         ("act_low", ctypes.c_float * 64), ("act_high", ctypes.c_float * 64), ("final_obs", ctypes.c_void_p),
         ("start_qpos", ctypes.c_void_p), ("start_qvel", ctypes.c_void_p), ("n_start", ctypes.c_int32),
+        ("params", ctypes.c_void_p), ("param_lo", ctypes.c_float * 4), ("param_hi", ctypes.c_float * 4),
     ]
+
+
+class ParamOffsets(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int32) for n in PARAM_FIELDS + ("n_params",)]
 
 
 class Layout(ctypes.Structure):
@@ -124,6 +132,11 @@ def load(build_if_missing=True):
                                      ctypes.c_float, ctypes.c_float]
     lib.mjb_start_index.restype = ctypes.c_uint32
     lib.mjb_start_index.argtypes = [ctypes.c_uint64, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int32]
+    lib.mjb_param_layout.argtypes = [vp, ctypes.POINTER(ParamOffsets)]
+    lib.mjb_model_set_field.argtypes = [vp, ctypes.c_char_p, ctypes.POINTER(ctypes.c_double), i32]
+    lib.mjb_param_scale.restype = ctypes.c_float
+    lib.mjb_param_scale.argtypes = [ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int32, ctypes.c_uint32, ctypes.c_uint32,
+                                    ctypes.c_float, ctypes.c_float]
     _LIB = lib
     return lib
 
@@ -158,13 +171,41 @@ class Model:
         d = Dims()
         check(self._lib.mjb_model_dims(h, ctypes.byref(d)))
         self.dims = d
-        n = ctypes.c_int64()
-        p = self._lib.mjb_model_blob(h, ctypes.byref(n))
-        self.blob = bytes((ctypes.c_char * n.value).from_address(p))
-        self.fields = parse_blob(self.blob)
+        self._read_blob()
         for k in ("nq", "nv", "nu", "nbody", "njnt", "ngeom", "nsite", "nsensor", "nsensordata", "npair", "ncam"):
             setattr(self, k, getattr(d, k))
         self.timestep = d.timestep
+
+    def _read_blob(self):
+        n = ctypes.c_int64()
+        p = self._lib.mjb_model_blob(self._h, ctypes.byref(n))
+        self.blob = bytes((ctypes.c_char * n.value).from_address(p))
+        self.fields = parse_blob(self.blob)
+
+    def set_field(self, name, values):
+        """Overwrite the fp64 field `name` (its full length) like MuJoCo's `model.<name>[:] = values`: nothing derived from
+        it is recomputed (include/mjb.h, mjb_model_set_field).  Batches created afterwards use the new values."""
+        v = np.ascontiguousarray(np.asarray(values, dtype=np.float64).reshape(-1))
+        check(self._lib.mjb_model_set_field(self._h, name.encode(), v.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), v.size),
+              "set_field")
+        self._read_blob()
+
+    def param_layout(self):
+        """ParamOffsets: where the five fields sit in a row of a per-env parameter table, and the row length"""
+        out = ParamOffsets()
+        check(self._lib.mjb_param_layout(self._h, ctypes.byref(out)), "param layout")
+        return out
+
+    def nominal_params(self):
+        """the model's own parameter row (float32 [n_params]) in the table layout of param_layout()"""
+        lay, f = self.param_layout(), self.fields
+        row = np.zeros(lay.n_params, np.float32)
+        vals = {"body_mass": f["body_mass"], "body_inertia": f["body_inertia"], "geom_friction": f["geom_friction"][0::3],
+                "actuator_gear": f["actuator_gear"], "dof_damping": f["dof_damping"]}
+        for k, v in vals.items():
+            o = getattr(lay, k)
+            row[o:o + v.size] = v
+        return row
 
     @classmethod
     def from_xml_path(cls, path):

@@ -14,10 +14,13 @@ from . import _lib as L
 
 class Batch:
     def __init__(self, model: "L.Model", spec: "L.EnvSpec", num_envs: int, device=None, keepalive=(), share=None, probe_quat=False,
-                 start_states=None):
+                 start_states=None, params=False, param_ranges=None):
         """`share`: another Batch whose tensors this handle steps as well (level variants, see set_subset);
         the two models must produce the same buffer layout.  `start_states`: (qpos [P, nq], qvel [P, nv]) float32 CUDA
-        tensors, a pool every reset draws its start state from (include/mjb.h, mjb_env_spec.start_qpos)."""
+        tensors, a pool every reset draws its start state from (include/mjb.h, mjb_env_spec.start_qpos).
+        `params`: give every env its own physical parameters, the table `self.params` [N, n_params] (include/mjb.h,
+        mjb_env_spec.params), filled with the model's values (or `share`'s table).  `param_ranges`: four (lo, hi) scale
+        ranges, one per family of L.PARAM_FAMILIES: every reset then draws the env's row (MJB_SPEC_RANDOMIZE)."""
         self._lib = L.load()
         if not torch.cuda.is_available():
             raise RuntimeError("mujoco_rl_environment_wrapper_b200: no CUDA device — the step path is CUDA-only "
@@ -63,6 +66,22 @@ class Batch:
             self.start_states = (qp, qv)   # kept alive: the library reads them at every reset
             spec = L.EnvSpec.from_buffer_copy(spec)
             spec.start_qpos, spec.start_qvel, spec.n_start = qp.data_ptr(), qv.data_ptr(), int(qp.shape[0])
+        if params or param_ranges is not None:
+            off = model.param_layout()
+            self.param_offsets = {f: getattr(off, f) for f in L.PARAM_FIELDS + ("n_params",)}
+            if share is not None and getattr(share, "params", None) is not None:
+                if share.param_offsets != self.param_offsets:
+                    raise Exception("level variants sharing a parameter table need the same parameter layout "
+                                    f"({self.param_offsets} != {share.param_offsets})")
+                self.params = share.params
+            else:
+                self.params = torch.from_numpy(model.nominal_params()).to(dev).repeat(N, 1).contiguous()
+            spec = L.EnvSpec.from_buffer_copy(spec)
+            spec.params = self.params.data_ptr()
+            if param_ranges is not None:
+                spec.flags |= L.SPEC_RANDOMIZE
+                for f, (lo, hi) in enumerate(param_ranges):
+                    spec.param_lo[f], spec.param_hi[f] = float(lo), float(hi)
         B = L.Buffers()
         for k, v in self.buf.items():
             setattr(B, k, v.data_ptr())

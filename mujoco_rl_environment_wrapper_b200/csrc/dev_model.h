@@ -165,7 +165,21 @@ struct DevModel {
   const float* start_qvel;
   int n_start;
   int start_pad[3];
+  // per-env parameter table (mjb_env_spec.params, DESIGN §5e): 64 bytes, padded like the fields above.  Only batches with
+  // a table set them; their kernels (PRM) keep the env's values in a scratch block of prm_n words at soff prm_soff:
+  // body mass [nmb] and inertia [nmb*3] in kernel order, then dof damping [nv], actuator gear [nu], geom friction
+  // [ngeom] in (virtual) MuJoCo order.  Image word offsets: prm_map (u32 [prm_n]: row offset | index << 16 | family << 28
+  // | copy << 30) and prm_nominal (f32 [prm_n]).
+  float* params;       // [N, n_params]
+  int n_params, prm_n;
+  int randomize, prm_soff, off_prm_map, off_prm_nominal;
+  float prm_lo[4], prm_hi[4];
 };
+// offsets of the parameter families inside the PRM scratch block
+MJB_HD int prm_inertia(const DevModel& dm) { return dm.nmb; }
+MJB_HD int prm_damping(const DevModel& dm) { return 4 * dm.nmb; }
+MJB_HD int prm_gear(const DevModel& dm) { return 4 * dm.nmb + dm.nv; }
+MJB_HD int prm_friction(const DevModel& dm) { return 4 * dm.nmb + dm.nv + dm.nu; }
 
 // ---- camera rendering (render_kernel.cuh): a second, small constant table next to the image -------------
 // cam record: kernel body (-1 = static: pose already in the world frame), mode (0 fixed), pos[3], quat[4],

@@ -50,6 +50,20 @@ inline int env_int(const char* name, int dflt) {
   return (s && *s) ? atoi(s) : dflt;
 }
 
+// why a spec's parameter-table fields cannot be used (nullptr: they can), see mjb_env_spec.params
+inline const char* param_spec_error(const mjb_env_spec& spec) {
+  if ((spec.flags & MJB_SPEC_RANDOMIZE) && !spec.params) return "MJB_SPEC_RANDOMIZE needs spec.params";
+  if (spec.params && spec.skip_frames == 0) return "spec.params needs skip_frames >= 1 (the physics-free step reads no parameter)";
+  if (spec.flags & MJB_SPEC_RANDOMIZE)
+    for (int f = 0; f < 4; f++) {
+      const float lo = spec.param_lo[f], hi = spec.param_hi[f];
+      if (!std::isfinite(lo) || !std::isfinite(hi)) return "param_lo / param_hi must be finite";
+      if (lo > hi) return "param_lo must be <= param_hi";
+      if (lo < 0.f || (f == 0 && lo <= 0.f)) return "param_lo must be >= 0 (> 0 for body mass)";
+    }
+  return nullptr;
+}
+
 inline void build_dev_model(const ModelView& m, const mjb_env_spec& spec, DevImage& out, bool lite = false, int pack = 1) {
   DevModel& dm = out.dm;
   memset(&dm, 0, sizeof(dm));
@@ -487,6 +501,43 @@ inline void build_dev_model(const ModelView& m, const mjb_env_spec& spec, DevIma
   w.begin(IF_tri_lut);
   for (int r = 0; r < 16; r++) for (int cc = 0; cc <= r; cc++) w.u((uint32_t)r | ((uint32_t)cc << 8));
   w.begin(IF_qpos0); for (int i = 0; i < m.nq; i++) w.f(m.qpos0[i]);
+  if (spec.params && !lite) {
+    // per-env parameter table: where every word of the PRM scratch block comes from in the env's row, its draw key and
+    // its nominal value.  Rows are per REAL env: copy c of a packed env reads row e0 + c, with the real model's ids.
+    if (const char* e = param_spec_error(spec)) throw std::runtime_error(e);
+    const int nb1 = (nbody - 1) / pack + 1, ng1 = m.ngeom / pack, nu1 = m.nu / pack, nv1 = m.nv / pack;
+    const int o_inertia = nb1, o_friction = 4 * nb1, o_gear = 4 * nb1 + ng1, o_damping = 4 * nb1 + ng1 + nu1;
+    dm.n_params = 4 * nb1 + ng1 + nu1 + nv1;
+    if (dm.n_params >= 65536) throw std::runtime_error("kernel limit: parameter row of more than 65535 floats");
+    if (nb1 >= 4096) throw std::runtime_error("kernel limit: a parameter table needs fewer than 4096 bodies");
+    std::vector<uint32_t> map;
+    std::vector<double> nominal;
+    auto add = [&](int off, int index, int family, int copy, double v) {
+      map.push_back((uint32_t)off | ((uint32_t)index << 16) | ((uint32_t)family << 28) | ((uint32_t)copy << 30));
+      nominal.push_back(v);
+    };
+    for (int k = 0; k < nmb; k++) {
+      const int vb = korder[k], c = (vb - 1) / (nb1 - 1), b = 1 + (vb - 1) % (nb1 - 1);
+      add(b, b, 0, c, m.body_mass[vb]);
+    }
+    for (int k = 0; k < nmb; k++) {
+      const int vb = korder[k], c = (vb - 1) / (nb1 - 1), b = 1 + (vb - 1) % (nb1 - 1);
+      for (int i = 0; i < 3; i++) add(o_inertia + 3 * b + i, b, 0, c, m.body_inertia[3 * vb + i]);
+    }
+    for (int d = 0; d < m.nv; d++) add(o_damping + d % nv1, d % nv1, 3, d / nv1, m.dof_damping[d]);
+    for (int u = 0; u < m.nu; u++) add(o_gear + u % nu1, u % nu1, 2, u / nu1, m.actuator_gear[u]);
+    for (int g = 0; g < m.ngeom; g++) add(o_friction + g % ng1, g % ng1, 1, g / ng1, m.geom_friction[3 * g]);
+    dm.params = spec.params;
+    dm.prm_n = (int)map.size();
+    dm.randomize = (spec.flags & MJB_SPEC_RANDOMIZE) ? 1 : 0;
+    for (int f = 0; f < 4; f++) { dm.prm_lo[f] = spec.param_lo[f]; dm.prm_hi[f] = spec.param_hi[f]; }
+    while (W.size() % 4) W.push_back(0);
+    dm.off_prm_map = (int)W.size();
+    for (uint32_t v : map) w.u(v);
+    while (W.size() % 4) W.push_back(0);
+    dm.off_prm_nominal = (int)W.size();
+    for (double v : nominal) w.f(v);
+  }
   while (W.size() % 4) W.push_back(0);
   dm.image_words = (int)W.size();
 
@@ -576,6 +627,7 @@ inline void build_dev_model(const ModelView& m, const mjb_env_spec& spec, DevIma
     for (int f : solver_fields)
       if (aliased[f]) { dm.soff[f] = o; o += r4(sizes[f]); }
   }
+  if (dm.prm_n > 0) { dm.prm_soff = off; off += r4(dm.prm_n); }   // the env's parameters: live through the whole pass
   dm.env_words = off;
 
   // ---- HBM row strides (16-byte aligned rows)

@@ -51,6 +51,18 @@ MJB_HD uint32_t start_index(unsigned long long seed, uint32_t env, uint32_t ep, 
   return n_start < 1 ? 0u : (uint32_t)(((unsigned long long)draw_u32(seed ^ 0x5eedc0deULL, env, 0xD000u, ep) * (uint32_t)n_start) >> 32);
 }
 
+// the scale of a randomising reset (include/mjb.h, mjb_param_scale) for element `index` of parameter family `family`,
+// keyed like reset_noise; rounded like reset_action
+MJB_HD float param_scale(unsigned long long seed, uint32_t env, uint32_t family, uint32_t index, uint32_t ep, float lo, float hi) {
+  const float u = (float)(draw_u32(seed ^ 0x5eedc0deULL, env, 0x10000u + 0x1000u * family + index, ep) >> 8) * (1.f / 16777216.f);
+#if defined(__CUDA_ARCH__)
+  return __fadd_rn(lo, __fmul_rn(u, hi - lo));
+#else
+  volatile float span = u * (hi - lo);
+  return lo + span;
+#endif
+}
+
 // Distances, the reward arithmetic and the done comparison run in fp64 on the fp32 positions (the reference computes
 // math.dist on float64 numpy views, mujoco_parent.py:428-449): given identical xipos the reward, cast to fp32, and the
 // done flag are those of the reference's own arithmetic.  The stored distance keeps its fp64 value in two store_f
@@ -234,7 +246,9 @@ MJB_DEV void split_copy(int i, int n1, int K, int& k, int& j) {
 // (dm.n_start > 0) or, in MODE_RESET_ROWS, their own rows, instead of qpos0 / zero velocity.
 // EXT = false compiles auto-reset and start states out (the device kernels of batches and launches that use neither);
 // with EXT = true they follow dm.autoreset, dm.n_start and the mode.
-template <bool PHYS, bool PACKED, bool EXT = true>
+// PRM (batches with a parameter table, DESIGN §5e): every copy loads its row of dm.params into the scratch block the
+// physics reads; the fresh copies of a reset with dm.randomize draw the row instead and store it back.
+template <bool PHYS, bool PACKED, bool EXT = true, bool PRM = false>
 MJB_DEV void run_env(const Ctx& c_in, const mjb_buffers& B, int venv, int num_envs, int mode_in, int skip_frames,
                      const uint8_t* reset_mask) {
   uint32_t fin = 0;   // 0: the pass the launch asked for; else the auto-reset pass over these copies (the step pass finished them)
@@ -346,6 +360,25 @@ pass:
     if (lane == 0) pre_ts = B.timestep[e0];
   }
   MJB_IMG_WAIT(c);
+  if (PRM) {
+    // the env's parameters (the map and the nominal values are image words)
+    float* prm = c.s + dm.prm_soff;
+    const uint32_t* map = c.img + dm.off_prm_map;
+    const float* nominal = (const float*)(c.img + dm.off_prm_nominal);
+    MJB_NOUNROLL
+    for (int i = lane; i < dm.prm_n; i += 32) {
+      const uint32_t e = map[i];
+      const int k = (int)(e >> 30), off = (int)(e & 0xffffu);
+      float* row = dm.params + (size_t)(e0 + k) * dm.n_params;
+      if (!has(k)) prm[i] = nominal[i];
+      else if (dm.randomize && fresh(k)) {
+        const uint32_t f = (e >> 28) & 3u;
+        const float s = param_scale(dm.seed, (uint32_t)(e0 + k), f, (e >> 16) & 0xfffu, reset_key((uint32_t)(e0 + k)), dm.prm_lo[f], dm.prm_hi[f]);
+        prm[i] = nominal[i] * s;
+        row[off] = prm[i];
+      } else MJB_G2S(&prm[i], &row[off]);
+    }
+  }
   MJB_G2S_WAIT();
   if (MJB_UNLIKELY(mode == MODE_RESET && dm.reset_noise > 0.f)) {
     // optional decorrelated starts (off by default: the reference always restarts at qpos0).  The draw is keyed by
@@ -407,7 +440,7 @@ pass:
   if (PHYS) {
     int dropped[MJB_MAX_PACK] = {0, 0, 0, 0};
     MJB_NOUNROLL
-    for (int f = 0; f < passes; f++) ncon = substep(c, f == passes - 1, integrate, &niter, dropped);
+    for (int f = 0; f < passes; f++) ncon = substep<PRM>(c, f == passes - 1, integrate, &niter, dropped);
     if (B.ncon_dropped && lane == 0) {   // cumulative per real env: stays 0 while no contact was ever dropped
 #pragma unroll
       for (int k = 0; k < MJB_MAX_PACK; k++)

@@ -5,6 +5,8 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <map>
+#include <mutex>
 #include <string>
 #include <vector>
 
@@ -27,8 +29,9 @@ namespace mjb {
 // `active` envs are walked starting at `env_base` (range launches of the host-buffer step) or through `env_ids`
 // (the env ids of one level: mjb_set_env_subset).  EXT: the step resets the envs it finishes (MJB_SPEC_AUTORESET) and
 // resets start from start states (pool or the caller's rows), a separate instantiation so that batches and launches that
-// use neither run exactly the code they ran before.
-template <bool PHYS, bool PACKED, bool EXT = false>
+// use neither run exactly the code they ran before.  PRM: the batch has a per-env parameter table (DESIGN §5e); only
+// instantiated with EXT, which covers every launch of such a batch.
+template <bool PHYS, bool PACKED, bool EXT = false, bool PRM = false>
 __global__ void __launch_bounds__(PHYS ? MJB_MAX_THREADS : 512, PHYS ? 1 : 4) k_env(const __grid_constant__ DevModel dm, const uint32_t* __restrict__ image, const mjb_buffers B,
                       int num_envs, int mode, int skip_frames, const uint8_t* __restrict__ mask,
                       const int* __restrict__ env_ids, int active, int env_base) {
@@ -70,7 +73,7 @@ __global__ void __launch_bounds__(PHYS ? MJB_MAX_THREADS : 512, PHYS ? 1 : 4) k_
       c.cta_threads = (mask == nullptr ? 32 : 0) * (busy > warps ? warps : (busy < 0 ? 0 : busy));
     }
     c.img_bar = r == 0 ? bar : nullptr;
-    if (env < nvirt) run_env<PHYS, PACKED, EXT>(c, B, env_ids ? env_ids[env] : env + env_base, num_envs, mode, skip_frames, mask);
+    if (env < nvirt) run_env<PHYS, PACKED, EXT, PRM>(c, B, env_ids ? env_ids[env] : env + env_base, num_envs, mode, skip_frames, mask);
     if (r == 0) mbar_wait(bar, 0);   // warps that had nothing to do in the first round (or returned early) have not waited yet
     if (!PHYS) __syncthreads();
     MJB_PH(c, PH_BARRIER);
@@ -165,7 +168,8 @@ int launch(mjb_batch* b, int mode, int skip_frames, const uint8_t* mask, cudaStr
                                                                                    skip_frames, mask, b->subset, active, base);
   } else {
     const bool ext = b->img.dm.autoreset || mode == mjb::MODE_RESET_ROWS || (mode == mjb::MODE_RESET && b->img.dm.n_start > 0);
-    auto kern = ext ? (b->img.dm.pack > 1 ? mjb::k_env<true, true, true> : mjb::k_env<true, false, true>)
+    auto kern = b->img.dm.prm_n > 0 ? (b->img.dm.pack > 1 ? mjb::k_env<true, true, true, true> : mjb::k_env<true, false, true, true>)
+              : ext ? (b->img.dm.pack > 1 ? mjb::k_env<true, true, true> : mjb::k_env<true, false, true>)
                     : (b->img.dm.pack > 1 ? mjb::k_env<true, true> : mjb::k_env<true, false>);
     const int pack = b->img.dm.pack;
     const int need = ((active + pack - 1) / pack + b->warps - 1) / b->warps;
@@ -196,8 +200,13 @@ uint32_t mjb_start_index(uint64_t seed, uint32_t env, uint32_t ep, int32_t n_sta
   return mjb::start_index(seed, env, ep, n_start);
 }
 
+float mjb_param_scale(uint64_t seed, uint32_t env, int32_t family, uint32_t index, uint32_t ep, float lo, float hi) {
+  return mjb::param_scale(seed, env, (uint32_t)family, index, ep, lo, hi);
+}
+
 int mjb_batch_layout(const mjb_model* m, const mjb_env_spec* spec, int32_t num_envs, mjb_layout* out) {
   if (!m || !spec || !out || num_envs < 1) { mjb::set_error("mjb_batch_layout: bad argument"); return MJB_ERR_ARG; }
+  if (const char* e = mjb::param_spec_error(*spec)) { mjb::set_error(std::string("mjb_batch_layout: ") + e); return MJB_ERR_ARG; }
   try {
     mjb::ModelView mv(m->host.blob.data());
     mjb::DevImage img;
@@ -231,6 +240,7 @@ int mjb_batch_create(const mjb_model* m, const mjb_env_spec* spec, int32_t num_e
     mjb::set_error("mjb_batch_create: spec.n_start > 0 needs spec.start_qpos and spec.start_qvel");
     return MJB_ERR_ARG;
   }
+  if (const char* e = mjb::param_spec_error(*spec)) { mjb::set_error(std::string("mjb_batch_create: ") + e); return MJB_ERR_ARG; }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) {
     mjb::set_error("mjb_batch_create: no CUDA device (the step path has no CPU fallback)");
@@ -279,13 +289,22 @@ int mjb_batch_create(const mjb_model* m, const mjb_env_spec* spec, int32_t num_e
   b->grid = (nvirt + warps - 1) / warps;
   if (b->grid > sms) b->grid = sms;
   b->smem_bytes = fixed + per_env * warps;
-  if (cudaFuncSetAttribute(mjb::k_env<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess ||
+  // The limit is an attribute of the kernel on the device, shared by every batch: it is only ever raised, so that a batch
+  // created later with less shared memory per CTA (one without a parameter table, a smaller model) leaves the launches
+  // of the earlier ones valid.
+  static std::mutex smem_attr_mu;
+  static std::map<int, size_t> smem_attr;
+  std::lock_guard<std::mutex> smem_attr_lock(smem_attr_mu);
+  if (b->smem_bytes > smem_attr[device] && (cudaFuncSetAttribute(mjb::k_env<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess ||
       cudaFuncSetAttribute(mjb::k_env<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess ||
       cudaFuncSetAttribute(mjb::k_env<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess ||
-      cudaFuncSetAttribute(mjb::k_env<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess) {
+      cudaFuncSetAttribute(mjb::k_env<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess ||
+      cudaFuncSetAttribute(mjb::k_env<true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess ||
+      cudaFuncSetAttribute(mjb::k_env<true, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_bytes) != cudaSuccess)) {
     mjb::set_error(std::string("cudaFuncSetAttribute(max dynamic smem) failed: ") + cudaGetErrorString(cudaGetLastError()));
     return fail(MJB_ERR_CUDA);
   }
+  smem_attr[device] = std::max(smem_attr[device], b->smem_bytes);
   if (spec->skip_frames == 0) {
     try {
       mjb::ModelView mv(m->host.blob.data());

@@ -1,5 +1,6 @@
 // mjb_model.cpp — host-only half of the C-ABI (include/mjb.h): MJCF -> model handle,
 // dims, blob access and name lookups.  No CUDA in this translation unit.
+#include <algorithm>
 #include <cstring>
 #include <string>
 
@@ -69,6 +70,44 @@ int mjb_name2id(const mjb_model* m, int objtype, const char* name) {
   for (size_t i = 0; i < it->second.size(); i++)
     if (it->second[i] == name) return (int)i;
   return -1;
+}
+
+int mjb_param_layout(const mjb_model* m, mjb_param_offsets* out) {
+  if (!m || !out) { mjb::set_error("mjb_param_layout: null argument"); return MJB_ERR_ARG; }
+  const mjb::HostModel& h = m->host;
+  const int nbody = h.get_int("nbody"), ngeom = h.get_int("ngeom"), nu = h.get_int("nu"), nv = h.get_int("nv");
+  out->body_mass = 0;
+  out->body_inertia = nbody;
+  out->geom_friction = 4 * nbody;
+  out->actuator_gear = 4 * nbody + ngeom;
+  out->dof_damping = 4 * nbody + ngeom + nu;
+  out->n_params = 4 * nbody + ngeom + nu + nv;
+  return MJB_OK;
+}
+
+int mjb_model_set_field(mjb_model* m, const char* name, const double* values, int32_t count) {
+  if (!m || !name || (!values && count > 0)) { mjb::set_error("mjb_model_set_field: null argument"); return MJB_ERR_ARG; }
+  auto it = m->host.f64.find(name);
+  if (it == m->host.f64.end()) {
+    mjb::set_error(std::string("mjb_model_set_field: no fp64 field named '") + name + "'");
+    return MJB_ERR_ARG;
+  }
+  if (count != (int32_t)it->second.size()) {
+    mjb::set_error(std::string("mjb_model_set_field: '") + name + "' has " + std::to_string(it->second.size()) + " values, got " +
+                   std::to_string(count));
+    return MJB_ERR_ARG;
+  }
+  it->second.assign(values, values + count);
+  if (std::string(name) == "geom_friction") {
+    // MuJoCo mixes friction per contact from the geoms' values; here the compiler stores the mix per collision pair
+    // (mjcf_compile.cpp): mix it again so that the edit reaches the contacts as it does in MuJoCo
+    const std::vector<int32_t>&g1 = m->host.Iv("pair_geom1"), &g2 = m->host.Iv("pair_geom2");
+    std::vector<double>& pf = m->host.f64["pair_friction"];
+    for (size_t k = 0; k < g1.size(); k++)
+      for (int i = 0; i < 3; i++) pf[3 * k + i] = std::max(it->second[3 * g1[k] + i], it->second[3 * g2[k] + i]);
+  }
+  m->host.pack();
+  return MJB_OK;
 }
 
 const char* mjb_id2name(const mjb_model* m, int objtype, int id) {

@@ -113,6 +113,8 @@ __device__ __forceinline__ void mjb_phase(long long* t_last, int lane, int id) {
 #define CF(f) ((const float*)(c.img + c.dm->off[IF_##f]))
 #define SF(f) (c.s + c.dm->soff[SF_##f])
 #define SI(f) ((int*)(c.s + c.dm->soff[SF_##f]))
+// a parameter of the per-env table (DESIGN §5e): the env's value in its scratch block under PRM, else the image's
+#define PF(f, blk) (PRM ? c.s + c.dm->prm_soff + (blk) : CF(f))
 
 // packed lower triangle: element (i, j), j <= i.  Lane i reading (i, k) is bank-conflict free for
 // i < 32 (triangular numbers are distinct mod 32).
@@ -369,6 +371,7 @@ MJB_DEV void rne_pass(const Ctx& c, bool with_acc) {
 // I a + v x* I v.  Composite inertias later accumulate IN PLACE in SF_cinert; SF_crb holds the body forces.
 // dyn_backward = the inward halves of crb_mass and rne_pass in one walk (16 words per body), then one loop over the dofs
 // for the rows of M and qfrc_smooth.  (fk / crb_mass / rne_pass stay for the renderer and the accelerometer pass.)
+template <bool PRM = false>
 MJB_DEV void kin_forward(const Ctx& c) {
   const DevModel& dm = *c.dm;
   const int* level_adr = CI(level_adr);
@@ -477,8 +480,8 @@ MJB_DEV void kin_forward(const Ctx& c) {
     {
       float Ri[9];
       q2m(qmul(ldq(xquat + 4 * b), ldq(CF(mb_iquat) + 4 * b)), Ri);
-      const f3 In = ld3(CF(mb_inertia) + 3 * b);
-      const float m = CF(mb_mass)[b];
+      const f3 In = ld3(PF(mb_inertia, prm_inertia(dm)) + 3 * b);
+      const float m = PF(mb_mass, 0)[b];
       const f3 cc = ipos - o;
       I[0] = m; I[1] = m * cc.x; I[2] = m * cc.y; I[3] = m * cc.z;
       I[4] = Ri[0] * Ri[0] * In.x + Ri[1] * Ri[1] * In.y + Ri[2] * Ri[2] * In.z + m * (cc.y * cc.y + cc.z * cc.z);
@@ -528,6 +531,7 @@ MJB_DEV void kin_forward(const Ctx& c) {
   MJB_SYNC();
 }
 
+template <bool PRM = false>
 MJB_DEV void dyn_backward(const Ctx& c) {
   const DevModel& dm = *c.dm;
   const int* level_adr = CI(level_adr);
@@ -573,14 +577,14 @@ MJB_DEV void dyn_backward(const Ctx& c) {
       M[tri(i, j)] = v;  // j is an ancestor dof: j <= i
     }
     const float bias = dot(sw, ld3(cfrc + 10 * b)) + dot(sv, ld3(cfrc + 10 * b + 3));
-    float fq = -CF(dof_damping)[i] * qvel[i] - bias;
+    float fq = -PF(dof_damping, prm_damping(dm))[i] * qvel[i] - bias;
     MJB_NOUNROLL
     for (int k = CI(dof_actadr)[i]; k < CI(dof_actadr)[i] + CI(dof_actnum)[i]; k++) {
       int u = CI(act_list)[k];
       const float* ap = CF(act_param) + 4 * u;
       float cv = ctrl[u];
       if (ap[1] != 0.f) cv = fminf(ap[3], fmaxf(ap[2], cv));
-      fq += ap[0] * cv;
+      fq += (PRM ? c.s[dm.prm_soff + prm_gear(dm) + u] : ap[0]) * cv;
     }
     qfrc[i] = fq;
   }
@@ -860,6 +864,7 @@ MJB_DEV void store_contact(const Ctx& c, int idx, const ConOut& o, int pair, flo
 
 // returns the number of contacts stored (warp-uniform); fills SF_con.  `tot[copy]` is ADVANCED by the number of
 // contacts found for that copy of a packed env (pack == 1: tot[0]) before the per-copy quota of maxcon1 slots
+template <bool PRM = false>
 MJB_DEV int collide(const Ctx& c, int* tot) {
   const DevModel& dm = *c.dm;
   const uint32_t* pairs = CU(pair_pack);
@@ -953,7 +958,7 @@ MJB_DEV int collide(const Ctx& c, int* tot) {
       int g1 = pk & 0xfff, g2 = (pk >> 12) & 0xfff;
       const float* pc = CF(pclass) + PC_STRIDE * (pk >> 24);
       float margin = pc[PC_MARGIN];
-      mu = pc[PC_MU];
+      mu = PRM ? fmaxf(c.s[dm.prm_soff + prm_friction(dm) + g1], c.s[dm.prm_soff + prm_friction(dm) + g2]) : pc[PC_MU];
       GeomW a = geom_world(c, g1), b = geom_world(c, g2);
       if (a.type == MJB_GEOM_PLANE) {
         f3 nrm = colv(a.mat, 2);
@@ -1020,7 +1025,7 @@ MJB_DEV int collide(const Ctx& c, int* tot) {
     int g1 = pk & 0xfff, g2 = (pk >> 12) & 0xfff;
     int t1 = CI(geom_type)[g1];
     const float* pc = CF(pclass) + PC_STRIDE * (pk >> 24);
-    float margin = pc[PC_MARGIN], mu = pc[PC_MU];
+    float margin = pc[PC_MARGIN], mu = PRM ? fmaxf(c.s[dm.prm_soff + prm_friction(dm) + g1], c.s[dm.prm_soff + prm_friction(dm) + g2]) : pc[PC_MU];
     GeomW a = geom_world(c, g1), b = geom_world(c, g2);
     bool hit = false;
     ConOut o;
@@ -1081,6 +1086,7 @@ MJB_DEV float impedance(const float* solimp, float pos, float margin) {
 }
 
 // rows: [0, 2 nlim) limit slots (lower, upper per limited joint; inactive -> D = 0), then 4 per contact
+template <bool PRM = false>
 MJB_DEV void make_constraints(const Ctx& c, int ncon) {
   const DevModel& dm = *c.dm;
   float *efcD = SF(efcD), *efcAref = SF(efcAref), *qpos = SF(qpos), *qvel = SF(qvel);
@@ -1158,7 +1164,7 @@ MJB_DEV void make_constraints(const Ctx& c, int ncon) {
     const float* pc = CF(pclass) + PC_STRIDE * (pk >> 24);
     int b1 = CI(geom_mb)[pk & 0xfff], b2 = CI(geom_mb)[(pk >> 12) & 0xfff];
     float tran = (b1 >= 0 ? CF(mb_invweight)[b1] : 0.f) + (b2 >= 0 ? CF(mb_invweight)[b2] : 0.f);
-    float mu = pc[PC_MU], dist = r[CON_DIST], inc = pc[PC_INCMARGIN];
+    float mu = PRM ? r[CON_MU] : pc[PC_MU], dist = r[CON_DIST], inc = pc[PC_INCMARGIN];
     float imp = impedance(pc + PC_SOLIMP, dist, inc);
     float vn = 0.f, v1 = 0.f, v2 = 0.f;
     {
@@ -1809,9 +1815,10 @@ MJB_DEV void sensors_acc(const Ctx& c, int ncon) {
 
 // =================================================================================================
 // one forward-dynamics evaluation: SF_qpos / qvel / ctrl -> SF_qacc.  Returns the contact count.
+template <bool PRM = false>
 MJB_DEV int forward(const Ctx& c, bool sensors, bool probes, int* iters_out, int* found) {
   MJB_PH(c, PH_INTEGRATE);
-  kin_forward(c);
+  kin_forward<PRM>(c);
   if (probes) {
     // exported positions belong to the LAST forward pass of the step (what `data.xipos` holds after
     // mj_step): for Euler that is the state before the integration (SURVEY 3.3), for RK4 the fourth stage.
@@ -1838,10 +1845,10 @@ MJB_DEV int forward(const Ctx& c, bool sensors, bool probes, int* iters_out, int
     MJB_SYNC();
   }
   MJB_PH(c, PH_FK);
-  dyn_backward(c);
+  dyn_backward<PRM>(c);
   MJB_PH(c, PH_RNE);
   int tot[MJB_MAX_PACK] = {0, 0, 0, 0};
-  int ncon = collide(c, tot);
+  int ncon = collide<PRM>(c, tot);
   MJB_PH(c, PH_COLLIDE);
   if (found) {   // contacts found beyond a copy's quota were dropped: keep the count visible (mjb_buffers.ncon_dropped)
 #pragma unroll
@@ -1849,7 +1856,7 @@ MJB_DEV int forward(const Ctx& c, bool sensors, bool probes, int* iters_out, int
   }
   if (sensors) sensors_pos(c);
   MJB_PH(c, PH_SENS);
-  make_constraints(c, ncon);
+  make_constraints<PRM>(c, ncon);
   MJB_PH(c, PH_CONSTR);
   int it = newton(c, ncon);
   // The Newton solve is where the envs of a round drift apart (1 .. 5 iterations).  Waiting for the slowest one HERE
@@ -1889,6 +1896,9 @@ MJB_DEV void integrate_pos(const Ctx& c, float* qpos, const float* v, float h) {
 // is a single stage, RK4 four stages of the same loop (stages 2..4 without sensors).  SF_qacc keeps the
 // solver's qacc (not the damping-corrected one): it is the warm start of the next solve, as MuJoCo's
 // qacc_warmstart.
+// PRM: the env's physical parameters come from its scratch block (DESIGN §5e); the implicit-damping solve then always
+// runs, since a row may hold damping where the model has none.
+template <bool PRM = false>
 MJB_DEV int substep(const Ctx& c, bool sensors, bool integrate, int* iters_out, int* dropped) {
   const DevModel& dm = *c.dm;
   const int nv = dm.nv, lane = c.lane;
@@ -1914,7 +1924,7 @@ MJB_DEV int substep(const Ctx& c, bool sensors, bool integrate, int* iters_out, 
       if (lane < nv) qvel[lane] = v0[lane] + h * A * aprev;
       MJB_SYNC();
     }
-    ncon = forward(c, sensors && st == 0, sensors && st == nstage - 1, st == 0 ? iters_out : nullptr, dropped);
+    ncon = forward<PRM>(c, sensors && st == 0, sensors && st == nstage - 1, st == 0 ? iters_out : nullptr, dropped);
     if (rk4) {
       const float Bw = (st == 0 || st == 3) ? (1.f / 6) : (1.f / 3);
       if (st == 0) {
@@ -1937,13 +1947,13 @@ MJB_DEV int substep(const Ctx& c, bool sensors, bool integrate, int* iters_out, 
     return ncon;
   }
   float acc = lane < nv ? qacc[lane] : 0.f;
-  if (dm.has_damping) {
+  if (PRM || dm.has_damping) {
     // (M + h D) a' = qfrc_smooth + qfrc_constraint
     float *M = SF(M), *H = SF(H);
     const int t0 = CI(dof_t0)[lane], t1 = CI(dof_t1)[lane];
     float rhs = lane < nv ? SF(vecA)[lane] : 0.f;   // qfrc_smooth + J' f at the solver's exit point
     MJB_SYNC();
-    acc = factor_solve(M, H, lane, t0, t1, dm.maxtree, lane < nv ? h * CF(dof_damping)[lane] : 0.f, rhs, nv);
+    acc = factor_solve(M, H, lane, t0, t1, dm.maxtree, lane < nv ? h * PF(dof_damping, prm_damping(dm))[lane] : 0.f, rhs, nv);
   }
   if (lane < nv) qvel[lane] += h * acc;
   MJB_SYNC();

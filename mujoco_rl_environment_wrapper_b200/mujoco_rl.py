@@ -9,7 +9,10 @@ Mirrors the reference's public surface (MuJoCo_Gym/mujoco_rl.py:18-430, mujoco_p
 
 New optional config keys: `num_envs` (default 1), `device`, `seed`, `autoReset` (default False: `step()` resets every
 env whose episode it ends, in the same kernel launch; see `step`), `startStates` ({"qpos": [P, nq], "qvel": [P, nv]}:
-every reset starts from a pool row drawn per env and reset instead of qpos0; see `reset`).  Positions of the agents' bodies and of
+every reset starts from a pool row drawn per env and reset instead of qpos0; see `reset`), `perEnvParams` (True: every
+env has its own body masses / inertias, geom frictions, actuator gears and dof dampings, `env.params`) and
+`randomizeParams` ({"body_mass": [lo, hi], "geom_friction": ..., "actuator_gear": ..., "dof_damping": ...}: every reset
+scales the env's parameters by factors drawn in [lo, hi]; implies `perEnvParams`).  Positions of the agents' bodies and of
 the `filter_by_tag("target")` objects are exported every step (`distance`, `get_data`).  With `num_envs == 1` results are squeezed to the
 reference's shapes (numpy arrays, Python scalars); otherwise every per-agent value is a CUDA tensor
 with a leading `num_envs` dimension.  There is no CPU path: construction raises without a GPU.
@@ -65,6 +68,25 @@ def state_rows(what, v, rows, width, device):
         want = f"[{'P >= 1' if rows is None else rows}, {width}]" + (f" (or [{width}])" if rows == 1 else "")
         raise Exception(f"{what}: expected shape {want}, got {tuple(t.shape)}")
     return t.contiguous()
+
+
+def parse_param_ranges(cfg):
+    """config "randomizeParams" {family: [lo, hi]} -> four (lo, hi) in L.PARAM_FAMILIES order (missing: (1, 1)), or None"""
+    if cfg is None:
+        return None
+    if not isinstance(cfg, dict) or any(k not in L.PARAM_FAMILIES for k in cfg):
+        raise Exception(f"randomizeParams: expected a dict with keys among {list(L.PARAM_FAMILIES)}, got {cfg!r}")
+    out = []
+    for f in L.PARAM_FAMILIES:
+        r = cfg.get(f, (1.0, 1.0))
+        try:
+            lo, hi = (float(x) for x in r)
+        except (TypeError, ValueError):
+            raise Exception(f"randomizeParams['{f}']: expected [lo, hi], got {r!r}")
+        if not (np.isfinite(lo) and np.isfinite(hi)) or lo > hi or lo < 0 or (f == "body_mass" and lo <= 0):
+            raise Exception(f"randomizeParams['{f}']: need finite 0 {'<' if f == 'body_mass' else '<='} lo <= hi, got [{lo}, {hi}]")
+        out.append((lo, hi))
+    return out
 
 
 def parse_start_states(cfg, nq, nv, device):
@@ -146,6 +168,10 @@ class MuJoCoRL:
         self._first_level = self._level_paths.index(random.choice(self._level_paths)) if self.num_envs == 1 else 0
         self._use_level(self._first_level)
         self._start_states = parse_start_states(config_dict.get("startStates"), self.model.nq, self.model.nv, self.device)
+        self._param_ranges = parse_param_ranges(config_dict.get("randomizeParams"))
+        self._per_env_params = bool(config_dict.get("perEnvParams", False)) or self._param_ranges is not None
+        if self._per_env_params and int(self.skip_frames) == 0:
+            raise Exception("perEnvParams / randomizeParams need skipFrames >= 1 (the physics-free step reads no parameter)")
         self.agents_action_index = self._tables.agents_action_index
         self.agents_observation_index = self._tables.agents_observation_index
 
@@ -271,9 +297,10 @@ class MuJoCoRL:
             with torch.cuda.device(self.device):
                 lv["batch"] = Batch(self.model, spec, self.num_envs, device=self.device, keepalive=keep,
                                     share=self._levels[0]["batch"] if lid else None, probe_quat=self.export_orientation,
-                                    start_states=self._start_states)
+                                    start_states=self._start_states, params=self._per_env_params, param_ranges=self._param_ranges)
         self._use_level(0)
         self._spec, self._batch = self._levels[0]["spec"], self._levels[0]["batch"]
+        self.params = self.__param_views() if self._per_env_params else None
         self.level_id = torch.zeros(self.num_envs, dtype=torch.int32, device=self.device)
         self._level_host = np.zeros(self.num_envs, dtype=np.int64)
         if multi:
@@ -283,6 +310,22 @@ class MuJoCoRL:
         self._act_low = torch.tensor(np.asarray(self._action_space[self.agents[0]].low), device=self.device)
         self._act_high = torch.tensor(np.asarray(self._action_space[self.agents[0]].high), device=self.device)
 
+    def __param_views(self):
+        """`env.params`: writable views of the per-env parameter table (include/mjb.h, mjb_env_spec.params), MuJoCo id
+        order: body_mass [N, nbody], body_inertia [N, nbody, 3], geom_friction [N, ngeom], actuator_gear [N, nu],
+        dof_damping [N, nv]; the leading dimension is dropped for num_envs == 1.  Writes take effect at the next launch;
+        with randomizeParams every reset overwrites the rows of the envs it resets.  With an `xmlPath` list the levels share
+        the table; an env that moves to another level gets that level's values.  `env.model` keeps the nominal values."""
+        t, off, m = self._batch.params, self._batch.param_offsets, self.model
+        n = {"body_mass": m.nbody, "body_inertia": 3 * m.nbody, "geom_friction": m.ngeom, "actuator_gear": m.nu, "dof_damping": m.nv}
+        views = {}
+        for f in L.PARAM_FIELDS:
+            v = t[:, off[f]:off[f] + n[f]]
+            if f == "body_inertia":
+                v = v.unflatten(1, (m.nbody, 3))
+            views[f] = v if self.num_envs > 1 else v[0]
+        return views
+
     def _draw_levels(self, mask, first=False):
         """a fresh level for every env being reset (the reference's random.choice at reset, mujoco_parent.py:351-352),
         then each level's handle is pointed at the envs it owns.  Host-side: resets are rare next to steps."""
@@ -291,12 +334,23 @@ class MuJoCoRL:
             draw = np.array([self._first_level if first else self._level_paths.index(random.choice(self._level_paths))])
         else:
             draw = self._level_rng.integers(0, n_lv, size=self.num_envs)
+        old = self._level_host
         if mask is None:
             self._level_host = draw
         else:
             m = mask.detach().to("cpu").numpy().astype(bool).reshape(-1)
             self._level_host = np.where(m, draw, self._level_host)
         self.level_id.copy_(torch.from_numpy(self._level_host.astype(np.int32)))
+        if self._per_env_params and self._param_ranges is None:
+            # the levels share one table: an env that moves to another level starts from that level's own values
+            # (a randomising reset draws them from the level's image anyway)
+            moved = np.ones(self.num_envs, bool) if first else self._level_host != old
+            table = self._levels[0]["batch"].params
+            for lid, lv in enumerate(self._levels):
+                ids = np.nonzero(moved & (self._level_host == lid))[0]
+                if len(ids):
+                    row = torch.from_numpy(lv["model"].nominal_params()).to(table.device)
+                    table[torch.from_numpy(ids).to(table.device)] = row
         for lid, lv in enumerate(self._levels):
             lv["batch"].set_subset(torch.from_numpy(np.nonzero(self._level_host == lid)[0].astype(np.int32)))
         self._use_level(int(self._level_host[0]))
