@@ -41,9 +41,14 @@ typedef struct mjb_blob_field {
  * that `model.geom(n).type` style queries keep their meaning). */
 enum { MJB_GEOM_PLANE = 0, MJB_GEOM_SPHERE = 2, MJB_GEOM_CAPSULE = 3, MJB_GEOM_BOX = 6 };
 enum { MJB_JNT_FREE = 0, MJB_JNT_SLIDE = 2, MJB_JNT_HINGE = 3 };
-enum { MJB_SENS_TOUCH = 0, MJB_SENS_ACCELEROMETER = 1, MJB_SENS_RANGEFINDER = 7,
-       MJB_SENS_FRAMEXAXIS = 28, MJB_SENS_FRAMEYAXIS = 29, MJB_SENS_FRAMEZAXIS = 30 };
-enum { MJB_OBJ_BODY = 1, MJB_OBJ_JOINT = 3, MJB_OBJ_GEOM = 5, MJB_OBJ_SITE = 6, MJB_OBJ_CAMERA = 7,
+enum { MJB_SENS_TOUCH = 0, MJB_SENS_ACCELEROMETER = 1, MJB_SENS_VELOCIMETER = 2, MJB_SENS_GYRO = 3,
+       MJB_SENS_RANGEFINDER = 7, MJB_SENS_JOINTPOS = 9, MJB_SENS_JOINTVEL = 10, MJB_SENS_FRAMEPOS = 26,
+       MJB_SENS_FRAMEQUAT = 27, MJB_SENS_FRAMEXAXIS = 28, MJB_SENS_FRAMEYAXIS = 29, MJB_SENS_FRAMEZAXIS = 30,
+       MJB_SENS_FRAMELINVEL = 31, MJB_SENS_FRAMEANGVEL = 32 };
+/* sensor_datatype: MuJoCo's mjtDataType */
+enum { MJB_DATA_REAL = 0, MJB_DATA_POSITIVE = 1, MJB_DATA_AXIS = 2, MJB_DATA_QUATERNION = 3 };
+/* object types: MuJoCo's mjtObj (XBODY = the body frame, BODY = its inertial frame for frame sensors) */
+enum { MJB_OBJ_BODY = 1, MJB_OBJ_XBODY = 2, MJB_OBJ_JOINT = 3, MJB_OBJ_GEOM = 5, MJB_OBJ_SITE = 6, MJB_OBJ_CAMERA = 7,
        MJB_OBJ_ACTUATOR = 19, MJB_OBJ_SENSOR = 20 };
 enum { MJB_INT_EULER = 0, MJB_INT_RK4 = 1 };
 

@@ -15,7 +15,12 @@ SPEC_NO_PACK, SPEC_AUTORESET, SPEC_RANDOMIZE = 1, 2, 4   # mjb_env_spec.flags
 # per-env parameter table (include/mjb.h, mjb_env_spec.params): the fields of a row, and the randomisation family of each
 PARAM_FIELDS = ("body_mass", "body_inertia", "geom_friction", "actuator_gear", "dof_damping")
 PARAM_FAMILIES = ("body_mass", "geom_friction", "actuator_gear", "dof_damping")
-OBJ_BODY, OBJ_JOINT, OBJ_GEOM, OBJ_SITE, OBJ_CAMERA, OBJ_ACTUATOR, OBJ_SENSOR = 1, 3, 5, 6, 7, 19, 20
+OBJ_BODY, OBJ_XBODY, OBJ_JOINT, OBJ_GEOM, OBJ_SITE, OBJ_CAMERA, OBJ_ACTUATOR, OBJ_SENSOR = 1, 2, 3, 5, 6, 7, 19, 20
+# sensor types (include/mjb_blob.h: MuJoCo's mjtSensor numbering) and datatypes (mjtDataType)
+SENSOR_TYPE = {"touch": 0, "accelerometer": 1, "velocimeter": 2, "gyro": 3, "rangefinder": 7, "jointpos": 9, "jointvel": 10,
+               "framepos": 26, "framequat": 27, "framexaxis": 28, "frameyaxis": 29, "framezaxis": 30, "framelinvel": 31,
+               "frameangvel": 32}
+DATA_REAL, DATA_POSITIVE, DATA_AXIS, DATA_QUATERNION = 0, 1, 2, 3
 DYN_LANGUAGE, DYN_PICKUP = 1, 2
 REW_TAG_DISTANCE, REW_ANT = 1, 2
 DONE_DISTANCE_LE = 1

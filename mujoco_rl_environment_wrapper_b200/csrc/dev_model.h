@@ -74,10 +74,10 @@ namespace mjb {
   X(site_quat)      /* f32 [nsite*4]                                                             */ \
   X(site_size)      /* f32 [nsite*3]                                                             */ \
   X(sensor_type)    /* int [nsensor]                                                             */ \
-  X(sensor_site)    /* int [nsensor]                                                             */ \
+  X(sensor_site)    /* int [nsensor]   site; jointpos / jointvel: qpos / dof address             */ \
   X(sensor_adr)     /* int [nsensor]                                                             */ \
   X(sensor_dim)     /* int [nsensor]                                                             */ \
-  X(sensor_dtype)   /* int [nsensor]   0 real, 1 positive, 2 axis                                */ \
+  X(sensor_dtype)   /* int [nsensor]   0 real, 1 positive, 2 axis, 3 quaternion                  */ \
   X(sensor_cutoff)  /* f32 [nsensor]                                                             */ \
   X(act_dof)        /* int [nu]                                                                  */ \
   X(act_param)      /* f32 [nu*4]      gear, ctrllimited, lo, hi                                 */ \
@@ -174,7 +174,16 @@ struct DevModel {
   int n_params, prm_n;
   int randomize, prm_soff, off_prm_map, off_prm_nominal;
   float prm_lo[4], prm_hi[4];
+  // frame, velocity and joint sensors (DESIGN §5f): 16 bytes, padded like the fields above.  off_sens_obj: image word
+  // offset of one SO_STRIDE record per sensor, present only when ext_sensors is set.
+  int ext_sensors, off_sens_obj, ext_pad[2];
 };
+// Object record of a frame / velocity sensor: the kernel body the object rides on (-1: static) and the object's pose in
+// that body's frame (in the world frame when static).  jointpos / jointvel keep their qpos / dof address in sensor_site.
+enum { SO_MB = 0, SO_POS = 1, SO_QUAT = 4, SO_STRIDE = 8 };
+// Image sensor_type of framex/y/zaxis on a body, xbody or geom: the evaluation pass of the other frame sensors takes them,
+// the site-only path in sensors_pos does not.
+enum { KSENS_OBJ_AXIS = 64 };
 // offsets of the parameter families inside the PRM scratch block
 MJB_HD int prm_inertia(const DevModel& dm) { return dm.nmb; }
 MJB_HD int prm_damping(const DevModel& dm) { return 4 * dm.nmb; }

@@ -403,8 +403,28 @@ inline void build_dev_model(const ModelView& m, const mjb_env_spec& spec, DevIma
     w.f(q.w); w.f(q.x); w.f(q.y); w.f(q.z);
   }
   w.begin(IF_site_size); for (int t = 0; t < 3 * m.nsite; t++) w.f(m.site_size[t]);
-  w.begin(IF_sensor_type); for (int i = 0; i < m.nsensor; i++) w.i(m.sensor_type[i]); if (!m.nsensor) w.i(0);
-  w.begin(IF_sensor_site); for (int i = 0; i < m.nsensor; i++) w.i(m.sensor_objid[i]); if (!m.nsensor) w.i(0);
+  // frame / velocity / joint sensors (DESIGN §5f): evaluated by their own pass from an object record each (SO_*)
+  auto frame_axis = [](int t) { return t >= MJB_SENS_FRAMEXAXIS && t <= MJB_SENS_FRAMEZAXIS; };
+  auto ext_sensor = [&](int i) {
+    const int t = m.sensor_type[i];
+    return t == MJB_SENS_VELOCIMETER || t == MJB_SENS_GYRO || t == MJB_SENS_JOINTPOS || t == MJB_SENS_JOINTVEL ||
+           t == MJB_SENS_FRAMEPOS || t == MJB_SENS_FRAMEQUAT || t == MJB_SENS_FRAMELINVEL || t == MJB_SENS_FRAMEANGVEL ||
+           (frame_axis(t) && m.sensor_objtype[i] != MJB_OBJ_SITE);
+  };
+  for (int i = 0; i < m.nsensor; i++) if (ext_sensor(i)) dm.ext_sensors = 1;
+  w.begin(IF_sensor_type);
+  for (int i = 0; i < m.nsensor; i++) {
+    const int t = m.sensor_type[i];
+    w.i(frame_axis(t) && ext_sensor(i) ? KSENS_OBJ_AXIS + (t - MJB_SENS_FRAMEXAXIS) : t);
+  }
+  if (!m.nsensor) w.i(0);
+  w.begin(IF_sensor_site);
+  for (int i = 0; i < m.nsensor; i++) {
+    const int t = m.sensor_type[i], id = m.sensor_objid[i];
+    if (m.sensor_objtype[i] == MJB_OBJ_JOINT) w.i(t == MJB_SENS_JOINTPOS ? m.jnt_qposadr[id] : m.jnt_dofadr[id]);
+    else w.i(m.sensor_objtype[i] == MJB_OBJ_SITE ? id : 0);
+  }
+  if (!m.nsensor) w.i(0);
   w.begin(IF_sensor_adr); for (int i = 0; i < m.nsensor; i++) w.i(m.sensor_adr[i]); if (!m.nsensor) w.i(0);
   w.begin(IF_sensor_dim); for (int i = 0; i < m.nsensor; i++) w.i(m.sensor_dim[i]); if (!m.nsensor) w.i(0);
   w.begin(IF_sensor_dtype); for (int i = 0; i < m.nsensor; i++) w.i(m.sensor_datatype[i]); if (!m.nsensor) w.i(0);
@@ -537,6 +557,33 @@ inline void build_dev_model(const ModelView& m, const mjb_env_spec& spec, DevIma
     while (W.size() % 4) W.push_back(0);
     dm.off_prm_nominal = (int)W.size();
     for (double v : nominal) w.f(v);
+  }
+  if (dm.ext_sensors && !lite) {
+    while (W.size() % 4) W.push_back(0);
+    dm.off_sens_obj = (int)W.size();
+    for (int i = 0; i < m.nsensor; i++) {
+      // body the object rides on and its pose there: site / geom frame, inertial frame (body), body frame (xbody)
+      const int ot = m.sensor_objtype[i], id = m.sensor_objid[i];
+      int b = 0;
+      V3 lp;
+      Quat lq;
+      if (ot == MJB_OBJ_SITE) {
+        b = m.site_bodyid[id]; lp = V3(m.site_pos[3 * id], m.site_pos[3 * id + 1], m.site_pos[3 * id + 2]);
+        lq = Quat{m.site_quat[4 * id], m.site_quat[4 * id + 1], m.site_quat[4 * id + 2], m.site_quat[4 * id + 3]};
+      } else if (ot == MJB_OBJ_GEOM) {
+        b = m.geom_bodyid[id]; lp = V3(m.geom_pos[3 * id], m.geom_pos[3 * id + 1], m.geom_pos[3 * id + 2]);
+        lq = Quat{m.geom_quat[4 * id], m.geom_quat[4 * id + 1], m.geom_quat[4 * id + 2], m.geom_quat[4 * id + 3]};
+      } else if (ot == MJB_OBJ_BODY) {
+        b = id; lp = V3(m.body_ipos[3 * id], m.body_ipos[3 * id + 1], m.body_ipos[3 * id + 2]);
+        lq = Quat{m.body_iquat[4 * id], m.body_iquat[4 * id + 1], m.body_iquat[4 * id + 2], m.body_iquat[4 * id + 3]};
+      } else if (ot == MJB_OBJ_XBODY) {
+        b = id;
+      }
+      if (!moving[b]) { lp = kin.xpos[b] + mulv(kin.xmat[b], lp); lq = qnormalized(qmul(kin.xquat[b], lq)); }
+      w.i(moving[b] ? b2k[b] : -1);
+      for (int k = 0; k < 3; k++) w.f(lp[k]);
+      w.f(lq.w); w.f(lq.x); w.f(lq.y); w.f(lq.z);
+    }
   }
   while (W.size() % 4) W.push_back(0);
   dm.image_words = (int)W.size();

@@ -5,7 +5,8 @@
 //   <compiler angle eulerseq>, <option timestep integrator gravity iterations tolerance impratio>,
 //   one unnamed <default> (joint / geom / site / motor), <worldbody> with nested <body>,
 //   <geom plane|sphere|capsule|box>, <joint free|hinge|slide>, <site>, <sensor touch|
-//   accelerometer|rangefinder|framexaxis|frameyaxis|framezaxis>, <actuator><motor>.
+//   accelerometer|rangefinder|framexaxis|frameyaxis|framezaxis|gyro|velocimeter|jointpos|jointvel|
+//   framepos|framequat|framelinvel|frameangvel>, <actuator><motor>.
 // The derived constants follow MuJoCo's documented compiler behaviour (inertia from
 // geoms, fromto -> pos/quat/size, degrees -> radians, qpos0, bounding radii, static
 // collision filters, body/dof invweight0).  MuJoCo's source is not part of the
@@ -578,28 +579,54 @@ void compile_mjcf(const std::string& xml_text, HostModel& M) {
   int nsensordata = 0;
   if (const XmlNode* sn = root->child("sensor")) {
     for (auto& s : sn->children) {
-      int type, dim, datatype = 0;  // 0 real, 1 positive, 2 axis
-      std::string objname;
-      if (s->tag == "touch") { type = MJB_SENS_TOUCH; dim = 1; datatype = 1; }
+      const std::string what = "MJCF: sensor <" + s->tag + (s->attr("name") ? " name='" + *s->attr("name") + "'" : std::string()) + ">";
+      auto fail = [&](const std::string& why) { throw std::runtime_error(what + ": " + why); };
+      int type, dim, datatype = MJB_DATA_REAL;
+      // attribute naming the object: "site", "joint" or "objname" (with "objtype")
+      enum { BY_SITE, BY_JOINT, BY_FRAME } by = BY_SITE;
+      if (s->tag == "touch") { type = MJB_SENS_TOUCH; dim = 1; datatype = MJB_DATA_POSITIVE; }
       else if (s->tag == "accelerometer") { type = MJB_SENS_ACCELEROMETER; dim = 3; }
-      else if (s->tag == "rangefinder") { type = MJB_SENS_RANGEFINDER; dim = 1; datatype = 1; }
-      else if (s->tag == "framexaxis") { type = MJB_SENS_FRAMEXAXIS; dim = 3; datatype = 2; }
-      else if (s->tag == "frameyaxis") { type = MJB_SENS_FRAMEYAXIS; dim = 3; datatype = 2; }
-      else if (s->tag == "framezaxis") { type = MJB_SENS_FRAMEZAXIS; dim = 3; datatype = 2; }
+      else if (s->tag == "velocimeter") { type = MJB_SENS_VELOCIMETER; dim = 3; }
+      else if (s->tag == "gyro") { type = MJB_SENS_GYRO; dim = 3; }
+      else if (s->tag == "rangefinder") { type = MJB_SENS_RANGEFINDER; dim = 1; datatype = MJB_DATA_POSITIVE; }
+      else if (s->tag == "jointpos") { type = MJB_SENS_JOINTPOS; dim = 1; by = BY_JOINT; }
+      else if (s->tag == "jointvel") { type = MJB_SENS_JOINTVEL; dim = 1; by = BY_JOINT; }
+      else if (s->tag == "framepos") { type = MJB_SENS_FRAMEPOS; dim = 3; by = BY_FRAME; }
+      else if (s->tag == "framequat") { type = MJB_SENS_FRAMEQUAT; dim = 4; datatype = MJB_DATA_QUATERNION; by = BY_FRAME; }
+      else if (s->tag == "framexaxis") { type = MJB_SENS_FRAMEXAXIS; dim = 3; datatype = MJB_DATA_AXIS; by = BY_FRAME; }
+      else if (s->tag == "frameyaxis") { type = MJB_SENS_FRAMEYAXIS; dim = 3; datatype = MJB_DATA_AXIS; by = BY_FRAME; }
+      else if (s->tag == "framezaxis") { type = MJB_SENS_FRAMEZAXIS; dim = 3; datatype = MJB_DATA_AXIS; by = BY_FRAME; }
+      else if (s->tag == "framelinvel") { type = MJB_SENS_FRAMELINVEL; dim = 3; by = BY_FRAME; }
+      else if (s->tag == "frameangvel") { type = MJB_SENS_FRAMEANGVEL; dim = 3; by = BY_FRAME; }
       else throw std::runtime_error("MJCF: unsupported sensor <" + s->tag + ">");
-      if (datatype == 2) {
+      if (s->attr("reftype") || s->attr("refname")) fail("reftype / refname are not supported");
+      int objtype = MJB_OBJ_SITE, objid = -1;
+      std::string objname;
+      if (by == BY_FRAME) {
         const std::string* ot = s->attr("objtype");
-        if (!ot || *ot != "site") throw std::runtime_error("MJCF: frame sensors are supported for objtype=site only");
-        if (!s->attr("objname")) throw std::runtime_error("MJCF: frame sensor needs objname");
+        if (!ot) fail("needs objtype");
+        if (!s->attr("objname")) fail("needs objname");
         objname = *s->attr("objname");
+        if (*ot == "site") { objtype = MJB_OBJ_SITE; objid = find_name(B.site_name, objname); }
+        else if (*ot == "body" || *ot == "xbody") {
+          objtype = *ot == "body" ? MJB_OBJ_BODY : MJB_OBJ_XBODY;
+          objid = find_name(B.body_name, objname);
+        } else if (*ot == "geom") { objtype = MJB_OBJ_GEOM; objid = find_name(B.geom_name, objname); }
+        else fail("objtype '" + *ot + "' is not supported (supported: site, body, xbody, geom)");
+      } else if (by == BY_JOINT) {
+        if (!s->attr("joint")) fail("needs a joint");
+        objname = *s->attr("joint");
+        objtype = MJB_OBJ_JOINT;
+        objid = find_name(B.jnt_name, objname);
+        if (objid >= 0 && B.jnt_type[objid] == MJB_JNT_FREE) fail("joint '" + objname + "' is a free joint (supported: hinge, slide)");
       } else {
-        if (!s->attr("site")) throw std::runtime_error("MJCF: sensor <" + s->tag + "> needs a site");
+        if (!s->attr("site")) fail("needs a site");
         objname = *s->attr("site");
+        objid = find_name(B.site_name, objname);
       }
-      int sid = find_name(B.site_name, objname);
-      if (sid < 0) throw std::runtime_error("MJCF: sensor refers to unknown site '" + objname + "'");
+      if (objid < 0) fail("refers to unknown object '" + objname + "'");
       Attrs a{s.get(), nullptr};
-      sensor_type.push_back(type); sensor_objtype.push_back(MJB_OBJ_SITE); sensor_objid.push_back(sid);
+      sensor_type.push_back(type); sensor_objtype.push_back(objtype); sensor_objid.push_back(objid);
       sensor_adr.push_back(nsensordata); sensor_dim.push_back(dim); sensor_datatype.push_back(datatype);
       sensor_cutoff.push_back(a.num("cutoff", 0));
       B.sensor_name.push_back(s->attr("name") ? *s->attr("name") : "");

@@ -20,7 +20,8 @@ inline void replicate_model(const HostModel& src, int K, HostModel& dst) {
             njnt = src.get_int("njnt"), ngeom = src.get_int("ngeom"), nsite = src.get_int("nsite"),
             nsensor = src.get_int("nsensor"), nsensordata = src.get_int("nsensordata"), npair = src.get_int("npair"),
             ntree = src.get_int("ntree");
-  (void)nu; (void)nsensor; (void)npair;
+  (void)nu; (void)npair;
+  const std::vector<int32_t>& sensor_objtype = src.Iv("sensor_objtype");
   auto bmap = [&](int b, int c) { return b <= 0 ? b : 1 + c * (nbody - 1) + (b - 1); };
   auto off = [](int v, int add) { return v < 0 ? v : v + add; };
   dst = HostModel();
@@ -55,7 +56,11 @@ inline void replicate_model(const HostModel& src, int K, HostModel& dst) {
           else if (name == "body_geomadr" || name == "pair_geom1" || name == "pair_geom2") x = off(x, c * ngeom);
           else if (name == "body_treeid") x = off(x, c * ntree);
           else if (name == "jnt_qposadr") x = off(x, c * nq);
-          else if (name == "sensor_objid") x = off(x, c * nsite);
+          else if (name == "sensor_objid") {   // numbered in its object type's id space
+            const int ot = sensor_objtype[(i - i0) % nsensor];
+            x = ot == MJB_OBJ_BODY || ot == MJB_OBJ_XBODY ? bmap(x, c)
+                : off(x, c * (ot == MJB_OBJ_GEOM ? ngeom : ot == MJB_OBJ_JOINT ? njnt : nsite));
+          }
           else if (name == "sensor_adr") x = off(x, c * nsensordata);
           o.push_back(x);
         }

@@ -1813,6 +1813,54 @@ MJB_DEV void sensors_acc(const Ctx& c, int ncon) {
   MJB_SYNC();
 }
 
+// frame, velocity and joint sensors (DESIGN §5f), lane = sensor.  Runs between the bias pass and the collision pass:
+// the only window where cvel and the body frames are both live (the broad phase's candidates overwrite cvel, the
+// constraint rows overwrite xquat / xmat).  Velocities as the accelerometer's: cvel is about the tree root's origin.
+MJB_DEV void sensors_frame(const Ctx& c) {
+  const DevModel& dm = *c.dm;
+  float* sens = SF(sens);
+  const float *xpos = SF(xpos), *xquat = SF(xquat), *xmat = SF(xmat), *cvel = SF(cvel);
+  MJB_NOUNROLL
+  for (int i = c.lane; i < dm.nsensor; i += 32) {
+    const int type = CI(sensor_type)[i], adr = CI(sensor_adr)[i];
+    if (type == MJB_SENS_JOINTPOS || type == MJB_SENS_JOINTVEL) {
+      const int a = CI(sensor_site)[i];
+      sens[adr] = cutoff(c, i, type == MJB_SENS_JOINTPOS ? SF(qpos)[a] : SF(qvel)[a]);
+      continue;
+    }
+    const bool axis = type >= KSENS_OBJ_AXIS;
+    if (!axis && type != MJB_SENS_VELOCIMETER && type != MJB_SENS_GYRO && type != MJB_SENS_FRAMEPOS && type != MJB_SENS_FRAMEQUAT &&
+        type != MJB_SENS_FRAMELINVEL && type != MJB_SENS_FRAMEANGVEL)
+      continue;
+    const float* rec = (const float*)(c.img + dm.off_sens_obj + SO_STRIDE * i);
+    const int b = ((const int*)rec)[SO_MB];
+    f3 p = ld3(rec + SO_POS), w = mk3(0, 0, 0), v = mk3(0, 0, 0);
+    q4 q = ldq(rec + SO_QUAT);
+    if (b >= 0) {
+      p = ld3(xpos + 3 * b) + mulv(xmat + 9 * b, p);
+      q = qmul(ldq(xquat + 4 * b), q);
+      w = ld3(cvel + 6 * b);
+      v = ld3(cvel + 6 * b + 3) + cross(w, p - ld3(xpos + 3 * CI(mb_root)[b]));
+    }
+    if (type == MJB_SENS_FRAMEQUAT) {   // never clamped
+      q = qnorm(q);
+      sens[adr] = q.w; sens[adr + 1] = q.x; sens[adr + 2] = q.y; sens[adr + 3] = q.z;
+      continue;
+    }
+    f3 r = type == MJB_SENS_FRAMEPOS ? p : (type == MJB_SENS_FRAMEANGVEL ? w : v);
+    if (axis) {   // column of the object's rotation
+      const int a = type - KSENS_OBJ_AXIS;
+      r = qrot(q, mk3(a == 0, a == 1, a == 2));
+    } else if (type == MJB_SENS_GYRO || type == MJB_SENS_VELOCIMETER) {   // in the object's frame: R' x
+      q4 qc = q;
+      qc.x = -q.x; qc.y = -q.y; qc.z = -q.z;
+      r = qrot(qc, type == MJB_SENS_GYRO ? w : v);
+    }
+    sens[adr] = cutoff(c, i, r.x); sens[adr + 1] = cutoff(c, i, r.y); sens[adr + 2] = cutoff(c, i, r.z);
+  }
+  MJB_SYNC();
+}
+
 // =================================================================================================
 // one forward-dynamics evaluation: SF_qpos / qvel / ctrl -> SF_qacc.  Returns the contact count.
 template <bool PRM = false>
@@ -1847,6 +1895,7 @@ MJB_DEV int forward(const Ctx& c, bool sensors, bool probes, int* iters_out, int
   MJB_PH(c, PH_FK);
   dyn_backward<PRM>(c);
   MJB_PH(c, PH_RNE);
+  if (sensors && c.dm->ext_sensors) sensors_frame(c);
   int tot[MJB_MAX_PACK] = {0, 0, 0, 0};
   int ncon = collide<PRM>(c, tot);
   MJB_PH(c, PH_COLLIDE);

@@ -113,6 +113,14 @@ class ModelView:
     def camera(self, name):
         return _Named(id=self._id(L.OBJ_CAMERA, name, "camera"), name=name)
 
+    def sensor(self, name):
+        i = self._id(L.OBJ_SENSOR, name, "sensor")
+        f = self._m.fields
+        return _Named(id=i, name=self._m.id2name(L.OBJ_SENSOR, i), type=np.array([f["sensor_type"][i]]),
+                      adr=np.array([f["sensor_adr"][i]]), dim=np.array([f["sensor_dim"][i]]),
+                      objtype=np.array([f["sensor_objtype"][i]]), objid=np.array([f["sensor_objid"][i]]),
+                      cutoff=np.array([f["sensor_cutoff"][i]]))
+
 
 class _Contact:
     def __init__(self, g1, g2, dist):
@@ -193,6 +201,14 @@ class DataView:
         i = env.model._id(L.OBJ_GEOM, name, "geom")
         nm = env.model.id2name(L.OBJ_GEOM, i)
         return _LazyObject(env, nm, L.OBJ_GEOM, i)
+
+    def sensor(self, name):
+        """`data.sensor(n)`: id, name and `.data`, the sensor's slice of sensordata (numpy for one env, a [N, dim] view)"""
+        env = self._env
+        i = env.model._id(L.OBJ_SENSOR, name, "sensor")
+        f = env.model.fields
+        adr, dim = int(f["sensor_adr"][i]), int(f["sensor_dim"][i])
+        return _Named(id=i, name=env.model.id2name(L.OBJ_SENSOR, i), data=self._out(env._batch.sensordata[:, adr:adr + dim]))
 
 
 class _LazyObject:

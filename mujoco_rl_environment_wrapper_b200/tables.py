@@ -11,7 +11,12 @@ import xml.etree.ElementTree as ET
 
 from . import _lib as L
 
-SENSOR_DIM = {"touch": 1, "accelerometer": 3, "rangefinder": 1, "framexaxis": 3, "frameyaxis": 3, "framezaxis": 3}
+SENSOR_DIM = {"touch": 1, "accelerometer": 3, "rangefinder": 1, "framexaxis": 3, "frameyaxis": 3, "framezaxis": 3,
+              "velocimeter": 3, "gyro": 3, "jointpos": 1, "jointvel": 1, "framepos": 3, "framequat": 4, "framelinvel": 3,
+              "frameangvel": 3}
+# the attribute naming a sensor's object ("objname" with "objtype" for the frame sensors)
+_SITE_SENSORS = ("touch", "accelerometer", "rangefinder", "velocimeter", "gyro")
+_JOINT_SENSORS = ("jointpos", "jointvel")
 
 
 def _iter_bodies(elem):
@@ -39,12 +44,18 @@ def sensor_space(kind, cutoff):
     """(low, high) lists for one sensor, sensor.py:64-116."""
     if kind == "touch":
         return [0], [float(cutoff)]
-    if kind == "accelerometer":
+    if kind == "accelerometer" and cutoff is not None:
         return [-float(cutoff)] * 3, [float(cutoff)] * 3
     if kind == "rangefinder":
         return [-1], [float(cutoff)]
     if kind in ("framexaxis", "frameyaxis", "framezaxis"):
         return [-1] * 3, [1] * 3
+    if kind == "framequat":
+        return [-1] * 4, [1] * 4
+    if kind in SENSOR_DIM:   # real-valued: clamped to +-cutoff when cutoff > 0
+        c = float(cutoff) if cutoff is not None else 0.0
+        b = c if c > 0 else float("inf")
+        return [-b] * SENSOR_DIM[kind], [b] * SENSOR_DIM[kind]
     raise Exception(f"unsupported sensor type {kind}")
 
 
@@ -87,8 +98,13 @@ class Tables:
                 kind = s.tag
                 if kind not in SENSOR_DIM:
                     raise Exception(f"unsupported sensor <{kind}>")
-                site = s.get("site") if kind in ("touch", "accelerometer", "rangefinder") else s.get("objname")
-                self.sensors.append({"name": s.get("name"), "type": kind, "site": site, "cutoff": s.get("cutoff"),
+                if kind in _SITE_SENSORS:
+                    objtype, obj = "site", s.get("site")
+                elif kind in _JOINT_SENSORS:
+                    objtype, obj = "joint", s.get("joint")
+                else:
+                    objtype, obj = s.get("objtype"), s.get("objname")
+                self.sensors.append({"name": s.get("name"), "type": kind, "objtype": objtype, "obj": obj, "cutoff": s.get("cutoff"),
                                      "indices": list(range(adr, adr + SENSOR_DIM[kind]))})
                 adr += SENSOR_DIM[kind]
         self.agents_observation_index, self.agents_action_index = {}, {}
@@ -102,8 +118,10 @@ class Tables:
             body = find_body(self.root, agent)
             self.agent_body[agent] = model.name2id(L.OBJ_BODY, agent)
             self.rgb_sensors[agent] = [c.get("name") for c in _subtree_elems(body, "camera")]
-            sites = {s.get("name") for s in _subtree_elems(body, "site")}
-            mine = [s for s in self.sensors if s["site"] in sites]
+            # a sensor belongs to the agent whose subtree holds its object
+            owned = {t: {e.get("name") for e in _subtree_elems(body, t)} for t in ("site", "joint", "geom")}
+            owned["body"] = owned["xbody"] = {body.get("name")} | {e.get("name") for e in _subtree_elems(body, "body")}
+            mine = [s for s in self.sensors if s["obj"] in owned.get(s["objtype"], ())]
             s_idx = [i for s in mine for i in s["indices"]]
             low, high = [], []
             for s in mine:
