@@ -78,11 +78,14 @@ def make_spec(model, tables, agents, free_joint, skip_frames=1, max_steps=1024, 
     return spec, (ai, oi_)
 
 
-def oracle_states(model, tables, agents, free_joint, n_states, stride=4, seed=0, settle=0):
+def oracle_states(model, tables, agents, free_joint, n_states, stride=4, seed=0, settle=0, start=None):
     """Pre-step states (qpos, qvel, warmstart, physical action per agent) along an oracle rollout with
-    random actions; the rollout itself defines the expected post-step state."""
+    random actions; the rollout itself defines the expected post-step state.  `start(qpos)` may edit the
+    initial qpos in place (e.g. to begin next to a wall)."""
     from oracle import OracleSim
     sim = OracleSim(model.blob)
+    if start is not None:
+        start(sim.qpos)
     rng = np.random.default_rng(seed)
     n_phys = len(tables.act_space[agents[0]]["low"])
     out = []
