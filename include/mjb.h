@@ -27,7 +27,9 @@
 #ifndef MJB_H_
 #define MJB_H_
 
+#if !defined(__CUDACC_RTC__)
 #include <stdint.h>
+#endif
 
 #include "mjb_blob.h"
 
@@ -176,7 +178,8 @@ typedef struct mjb_env_spec {
 enum {
   MJB_SPEC_NO_PACK = 1,   /* one env per warp even for small models (needed by mjb_set_env_subset) */
   MJB_SPEC_AUTORESET = 2, /* mjb_step resets every env whose step ends its episode, in the same launch (see mjb_step) */
-  MJB_SPEC_RANDOMIZE = 4  /* every reset draws the env's row of spec.params (see mjb_env_spec.params) */
+  MJB_SPEC_RANDOMIZE = 4, /* every reset draws the env's row of spec.params (see mjb_env_spec.params) */
+  MJB_SPEC_GENERIC = 8    /* mjb_step runs the generic step kernel, not the one compiled for the model's shape */
 };
 
 
@@ -285,6 +288,14 @@ int mjb_set_env_subset(mjb_batch* b, const int32_t* env_ids_dev, int32_t count);
 int mjb_render(mjb_batch* b, const int32_t* cam_ids, int32_t ncams, int32_t width, int32_t height, uint8_t* rgb_dev);
 /* launch geometry chosen at creation: CTAs, env-warps per CTA, dynamic shared memory per CTA */
 int mjb_batch_geometry(const mjb_batch* b, int32_t* grid, int32_t* warps_per_cta, int64_t* smem_bytes);
+/* The physics step of mjb_step runs a kernel compiled at mjb_batch_create for the model's shape (sizes, strides and
+ * offsets as constants; NVRTC, once per shape and process), with the same results as the generic kernel.  Without NVRTC
+ * of the release that built the library, with MJB_SPEC_GENERIC, or when the compile fails, the batch runs the generic
+ * kernel.  `specialised`: which one runs; `compile_ms`: NVRTC time of the shape; `reason`: why not specialised ("" if it is). */
+int mjb_batch_spec_info(const mjb_batch* b, int32_t* specialised, double* compile_ms, char* reason, int32_t reason_len);
+/* compile the specialised step kernel a batch of (m, spec, num_envs) would run, without a device: its cubin goes to
+ * `cubin` when *cubin_bytes is large enough; *cubin_bytes returns its size */
+int mjb_spec_compile(const mjb_model* m, const mjb_env_spec* spec, int32_t num_envs, double* compile_ms, void* cubin, int64_t* cubin_bytes);
 /* debug builds (-DMJB_PHASE_PROF) only: reads and clears the per-phase clock-cycle counters of the step kernel
  * (step_kernel.cuh PH_*); returns the number of phases, 0 in the product build */
 int mjb_phase_cycles(uint64_t* out, int32_t n);

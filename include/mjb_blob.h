@@ -11,8 +11,14 @@
 #ifndef MJB_BLOB_H_
 #define MJB_BLOB_H_
 
+#if defined(__CUDACC_RTC__)
+/* NVRTC (the step kernel specialised at batch creation) compiles without host headers */
+typedef signed char int8_t; typedef unsigned char uint8_t; typedef short int16_t; typedef unsigned short uint16_t;
+typedef int int32_t; typedef unsigned int uint32_t; typedef long long int64_t; typedef unsigned long long uint64_t;
+#else
 #include <stdint.h>
 #include <string.h>
+#endif
 
 #ifdef __cplusplus
 extern "C" {
@@ -52,6 +58,7 @@ enum { MJB_OBJ_BODY = 1, MJB_OBJ_XBODY = 2, MJB_OBJ_JOINT = 3, MJB_OBJ_GEOM = 5,
        MJB_OBJ_ACTUATOR = 19, MJB_OBJ_SENSOR = 20 };
 enum { MJB_INT_EULER = 0, MJB_INT_RK4 = 1 };
 
+#if !defined(__CUDACC_RTC__)
 static inline const mjb_blob_field* mjb_blob_find(const void* blob, const char* name) {
   const mjb_blob_header* h = (const mjb_blob_header*)blob;
   const mjb_blob_field* f = (const mjb_blob_field*)((const char*)blob + sizeof(mjb_blob_header));
@@ -71,6 +78,7 @@ static inline const double* mjb_blob_f64(const void* blob, const char* name, int
   if (count) *count = f->count;
   return (const double*)((const char*)blob + f->offset);
 }
+#endif
 
 #ifdef __cplusplus
 }

@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MJB_LIB") or os.path.join(_HERE, "libmjb.so")
 
 MAX_AGENTS, MAX_PLUGINS, MAX_TARGETS, MAX_EXTRA_PROBES = 8, 4, 16, 48
-SPEC_NO_PACK, SPEC_AUTORESET, SPEC_RANDOMIZE = 1, 2, 4   # mjb_env_spec.flags
+SPEC_NO_PACK, SPEC_AUTORESET, SPEC_RANDOMIZE, SPEC_GENERIC = 1, 2, 4, 8   # mjb_env_spec.flags
 # per-env parameter table (include/mjb.h, mjb_env_spec.params): the fields of a row, and the randomisation family of each
 PARAM_FIELDS = ("body_mass", "body_inertia", "geom_friction", "actuator_gear", "dof_damping")
 PARAM_FAMILIES = ("body_mass", "geom_friction", "actuator_gear", "dof_damping")
@@ -81,6 +81,25 @@ class Buffers(ctypes.Structure):
 _LIB = None
 
 
+def _preload_nvrtc():
+    """Without a CUDA toolkit, make the NVRTC a CUDA wheel of torch ships visible to libmjb's dlopen("libnvrtc.so.12"),
+    which compiles the step kernel specialised to each batch's model (csrc/spec_jit.h).  Without either, batches run the
+    generic kernel."""
+    if os.path.exists(os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "lib64", "libnvrtc.so.12")) or \
+            os.path.exists("/usr/local/cuda/lib64/libnvrtc.so.12"):
+        return
+    import importlib.util
+    spec = importlib.util.find_spec("nvidia.cuda_nvrtc")
+    for root in (spec.submodule_search_locations or []) if spec else []:
+        path = os.path.join(root, "lib", "libnvrtc.so.12")
+        if os.path.exists(path):
+            try:
+                ctypes.CDLL(path, mode=ctypes.RTLD_GLOBAL)
+            except OSError:
+                pass
+            return
+
+
 def load(build_if_missing=True):
     """Load libmjb.so; builds it in-tree with nvcc when missing or stale (CPU container only)."""
     global _LIB
@@ -97,6 +116,7 @@ def load(build_if_missing=True):
     if not os.path.exists(LIB_PATH):
         raise RuntimeError(f"{LIB_PATH} is missing: run `python -m mujoco_rl_environment_wrapper_b200.build` "
                            "(there is no CPU fallback for the step path)")
+    _preload_nvrtc()
     lib = ctypes.CDLL(LIB_PATH)
     vp, i32, i64 = ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64
     lib.mjb_last_error.restype = ctypes.c_char_p
@@ -129,6 +149,8 @@ def load(build_if_missing=True):
     lib.mjb_set_env_subset.argtypes = [vp, vp, ctypes.c_int32]
     lib.mjb_render.argtypes = [vp, ctypes.POINTER(ctypes.c_int32), ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, vp]
     lib.mjb_batch_geometry.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(i32), ctypes.POINTER(i64)]
+    lib.mjb_batch_spec_info.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(ctypes.c_double), ctypes.c_char_p, i32]
+    lib.mjb_spec_compile.argtypes = [vp, ctypes.POINTER(EnvSpec), i32, ctypes.POINTER(ctypes.c_double), vp, ctypes.POINTER(i64)]
     lib.mjb_phase_cycles.argtypes = [ctypes.POINTER(ctypes.c_uint64), i32]
     lib.mjb_draw_u32.restype = ctypes.c_uint32
     lib.mjb_draw_u32.argtypes = [ctypes.c_uint64, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32]
@@ -144,6 +166,17 @@ def load(build_if_missing=True):
                                     ctypes.c_float, ctypes.c_float]
     _LIB = lib
     return lib
+
+
+def spec_compile(model, spec, num_envs):
+    """NVRTC-compile the specialised step kernel a batch of (model, spec, num_envs) would run (no device needed):
+    (cubin bytes, compile ms)"""
+    lib = load()
+    ms, n = ctypes.c_double(), ctypes.c_int64(0)
+    check(lib.mjb_spec_compile(model._h, ctypes.byref(spec), int(num_envs), ctypes.byref(ms), None, ctypes.byref(n)), "spec compile")
+    buf = ctypes.create_string_buffer(n.value)
+    check(lib.mjb_spec_compile(model._h, ctypes.byref(spec), int(num_envs), ctypes.byref(ms), buf, ctypes.byref(n)), "spec compile")
+    return buf.raw[:n.value], ms.value
 
 
 def check(rc, what=""):

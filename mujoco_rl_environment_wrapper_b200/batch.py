@@ -193,4 +193,7 @@ class Batch:
     def geometry(self):
         g, w, s = ctypes.c_int32(), ctypes.c_int32(), ctypes.c_int64()
         self._lib.mjb_batch_geometry(self._h, ctypes.byref(g), ctypes.byref(w), ctypes.byref(s))
-        return {"grid": g.value, "warps_per_cta": w.value, "smem_bytes": s.value}
+        spec, ms, why = ctypes.c_int32(), ctypes.c_double(), ctypes.create_string_buffer(4096)
+        self._lib.mjb_batch_spec_info(self._h, ctypes.byref(spec), ctypes.byref(ms), why, len(why))
+        return {"grid": g.value, "warps_per_cta": w.value, "smem_bytes": s.value, "specialised": bool(spec.value),
+                "spec_reason": why.value.decode(errors="replace"), "spec_compile_ms": ms.value}

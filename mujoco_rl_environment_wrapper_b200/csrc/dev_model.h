@@ -5,7 +5,9 @@
 // (cp.async.bulk, SASS UBLKCP), plus a small POD header (DevModel) passed as a kernel parameter.
 // Device side: typed accessors over the image.
 #pragma once
+#if !defined(__CUDACC_RTC__)
 #include <stdint.h>
+#endif
 
 #ifndef MJB_HD
 #if defined(__CUDACC__)
@@ -185,10 +187,35 @@ enum { SO_MB = 0, SO_POS = 1, SO_QUAT = 4, SO_STRIDE = 8 };
 // the site-only path in sensors_pos does not.
 enum { KSENS_OBJ_AXIS = 64 };
 // offsets of the parameter families inside the PRM scratch block
-MJB_HD int prm_inertia(const DevModel& dm) { return dm.nmb; }
-MJB_HD int prm_damping(const DevModel& dm) { return 4 * dm.nmb; }
-MJB_HD int prm_gear(const DevModel& dm) { return 4 * dm.nmb + dm.nv; }
-MJB_HD int prm_friction(const DevModel& dm) { return 4 * dm.nmb + dm.nv + dm.nu; }
+template <class M> MJB_HD int prm_inertia(const M& dm) { return dm.nmb; }
+template <class M> MJB_HD int prm_damping(const M& dm) { return 4 * dm.nmb; }
+template <class M> MJB_HD int prm_gear(const M& dm) { return 4 * dm.nmb + dm.nv; }
+template <class M> MJB_HD int prm_friction(const M& dm) { return 4 * dm.nmb + dm.nv + dm.nu; }
+
+// The model's warp-uniform integer shape: sizes, strides, word offsets, plugin counts and flags.  Two models with the same
+// shape differ only in values (floats, pointers, seed, the per-lane image tables) and can share one specialised kernel.
+#define MJB_SHAPE_FIELDS(X)                                                                                                  \
+  X(nq) X(nv) X(nu) X(nmb) X(njnt) X(nlim) X(ngeom) X(ngdyn) X(nsite) X(nsensor) X(nsensordata) X(npair) X(nclass)         \
+  X(nlevel) X(nprobe) X(maxcon) X(maxcand) X(maxefc) X(ldj) X(maxtree) X(nblock)                                           \
+  X(pack) X(a1) X(t1) X(nq1) X(nv1) X(nu1) X(ns1) X(np1) X(ngeom1) X(maxcon1) X(njnt1)                                     \
+  X(integrator) X(has_damping) X(need_acc_sensors) X(solver_iterations) X(ls_iterations)                                   \
+  X(n_agents) X(free_joint) X(n_phys_act) X(act_dim) X(n_dynamics) X(n_rewards) X(n_dones) X(n_targets)                   \
+  X(image_words) X(env_words) X(qpos_stride) X(qvel_stride) X(ctrl_stride) X(sensor_stride) X(act_stride) X(obs_stride)    \
+  X(store_i32) X(store_f32) X(autoreset) X(n_params) X(prm_n) X(prm_soff) X(off_prm_map) X(off_prm_nominal)                \
+  X(ext_sensors) X(off_sens_obj)
+
+// The step kernel reads the model through `DM`.  In the generic build DM is DevModel: every field is a load of the kernel
+// parameter.  The specialised build (MJB_SPEC: one NVRTC compile per batch shape, mjb_batch.cu) includes a generated
+// header that derives SpecModel from DevModel and hides each MJB_SHAPE_FIELDS member with a constant of the same name, and
+// defines the image / scratch word offsets (spec_off, spec_soff): the same source then folds the shape into the code.
+#if defined(MJB_SPEC)
+}  // namespace mjb
+#include "mjb_spec_shape.h"
+namespace mjb {
+typedef SpecModel DM;
+#else
+typedef DevModel DM;
+#endif
 
 // ---- camera rendering (render_kernel.cuh): a second, small constant table next to the image -------------
 // cam record: kernel body (-1 = static: pose already in the world frame), mode (0 fixed), pos[3], quat[4],

@@ -100,7 +100,7 @@ MJB_DEV void st_dist(float* sfa, double d) {
 // A reset zeroes rew / term / trunc unless `keep_flags` (auto-reset: they stay those of the step that ended the episode).
 // Returns whether the step ended the episode (term[A] | trunc[A]); false for a reset.
 template <int AMAX>
-MJB_DEV bool run_plugins(const DevModel& dm, const float* ctrl, float* obs, float* rew, uint8_t* term, uint8_t* trunc, int env, int copy,
+MJB_DEV bool run_plugins(const DM& dm, const float* ctrl, float* obs, float* rew, uint8_t* term, uint8_t* trunc, int env, int copy,
                          bool is_reset, const float* probe, int* si, float* sf, const float* act, int* ts_io, const double* dtab = nullptr,
                          bool keep_flags = false) {
   // `env` is the REAL environment, `copy` its slot inside the (possibly packed) virtual env of this warp
@@ -258,7 +258,7 @@ pass:
   const int mode = (auto_pass || own_rows) ? (int)MODE_RESET : mode_in;
   Ctx c = c_in;
   float* probe = c.probe;
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const int lane = c.lane, K = PACKED ? dm.pack : 1, e0 = venv * K;   // K == 1 folds all copy arithmetic away
   c.probe_quat = (!PACKED && B.probe_quat) ? B.probe_quat + (size_t)e0 * dm.np1 * 4 : nullptr;
   // which copies hold a real env, and which of them this launch updates
@@ -648,5 +648,68 @@ pass:
     goto pass;
   }
 }
+
+#if !defined(MJB_HOST_EMU)
+#ifndef MJB_MAX_THREADS
+#define MJB_MAX_THREADS 512
+#endif
+
+// One CTA per SM, `warps` environments in flight per CTA; each warp walks the env index space with a grid-wide
+// stride (envs are independent: the warps only meet at the staging of the model image and at the alignment points).
+// `active` envs are walked starting at `env_base` (range launches of the host-buffer step) or through `env_ids`
+// (the env ids of one level: mjb_set_env_subset).  EXT: the step resets the envs it finishes (MJB_SPEC_AUTORESET) and
+// resets start from start states (pool or the caller's rows), a separate instantiation so that batches and launches that
+// use neither run exactly the code they ran before.  PRM: the batch has a per-env parameter table (DESIGN §5e); only
+// instantiated with EXT, which covers every launch of such a batch.
+template <bool PHYS, bool PACKED, bool EXT = false, bool PRM = false>
+__global__ void __launch_bounds__(PHYS ? MJB_MAX_THREADS : 512, PHYS ? 1 : 4) k_env(const __grid_constant__ DM dm, const uint32_t* __restrict__ image, const mjb_buffers B,
+                      int num_envs, int mode, int skip_frames, const uint8_t* __restrict__ mask,
+                      const int* __restrict__ env_ids, int active, int env_base) {
+  extern __shared__ __align__(128) uint32_t smem[];
+  uint64_t* bar = reinterpret_cast<uint64_t*>(smem);
+  uint32_t* img = smem + 4;  // 16 B after the barrier
+  const int warps = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x == 0) {
+    mbar_init(bar, 1);
+    mbar_fence_init();
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    uint32_t bytes = (uint32_t)dm.image_words * 4u;
+    mbar_expect_tx(bar, bytes);
+    bulk_g2s(img, image, bytes, bar);
+  }
+  float* scratch = reinterpret_cast<float*>(img + dm.image_words) + (size_t)warp * (dm.env_words + 4 * ((dm.nprobe + 3) & ~3));
+  float* probe = scratch + dm.env_words;
+  Ctx c{&dm, img, scratch, lane, probe, 0};
+#if defined(MJB_PHASE_PROF)
+  long long t_last = clock64();
+  c.t_last = &t_last;
+#endif
+  // Lock-step rounds: every env-warp of the CTA takes one env per round, so the warps walk through the (large) step
+  // code together and share instruction-cache lines (measured 2x at 65536 envs against a grid-wide work counter).
+  // The physics step re-aligns the busy env-warps right after the Newton solve (step_kernel.cuh, forward): they leave
+  // it together and stay together through the tail of the step and the head of the next env, so there is no barrier
+  // at the round boundary.  The physics-free step has no alignment point inside and re-aligns at the end of each round.
+  const int stride = gridDim.x * warps;
+  const int pack = PACKED ? dm.pack : 1;
+  const int nvirt = (active + pack - 1) / pack;   // virtual envs: `pack` real envs share a warp (active = envs this launch walks)
+  const int rounds = (nvirt - blockIdx.x * warps + stride - 1) / stride;
+  int env = blockIdx.x * warps + warp;
+  for (int r = 0; r < rounds; r++) {
+    if (PHYS) {
+      int busy = nvirt - (blockIdx.x * warps + r * stride);  // env-warps of this CTA with work in this round
+      // (a masked reset lets warps skip their env, so intra-step alignment is off for it)
+      c.cta_threads = (mask == nullptr ? 32 : 0) * (busy > warps ? warps : (busy < 0 ? 0 : busy));
+    }
+    c.img_bar = r == 0 ? bar : nullptr;
+    if (env < nvirt) run_env<PHYS, PACKED, EXT, PRM>(c, B, env_ids ? env_ids[env] : env + env_base, num_envs, mode, skip_frames, mask);
+    if (r == 0) mbar_wait(bar, 0);   // warps that had nothing to do in the first round (or returned early) have not waited yet
+    if (!PHYS) __syncthreads();
+    MJB_PH(c, PH_BARRIER);
+    env += stride;
+  }
+}
+#endif
 
 }  // namespace mjb

@@ -17,71 +17,7 @@
 #include "tma_prims.cuh"
 #include "lite_kernel.cuh"
 #include "mjb_internal.h"
-
-#ifndef MJB_MAX_THREADS
-#define MJB_MAX_THREADS 512
-#endif
-
-namespace mjb {
-
-// One CTA per SM, `warps` environments in flight per CTA; each warp walks the env index space with a grid-wide
-// stride (envs are independent: the warps only meet at the staging of the model image and at the alignment points).
-// `active` envs are walked starting at `env_base` (range launches of the host-buffer step) or through `env_ids`
-// (the env ids of one level: mjb_set_env_subset).  EXT: the step resets the envs it finishes (MJB_SPEC_AUTORESET) and
-// resets start from start states (pool or the caller's rows), a separate instantiation so that batches and launches that
-// use neither run exactly the code they ran before.  PRM: the batch has a per-env parameter table (DESIGN §5e); only
-// instantiated with EXT, which covers every launch of such a batch.
-template <bool PHYS, bool PACKED, bool EXT = false, bool PRM = false>
-__global__ void __launch_bounds__(PHYS ? MJB_MAX_THREADS : 512, PHYS ? 1 : 4) k_env(const __grid_constant__ DevModel dm, const uint32_t* __restrict__ image, const mjb_buffers B,
-                      int num_envs, int mode, int skip_frames, const uint8_t* __restrict__ mask,
-                      const int* __restrict__ env_ids, int active, int env_base) {
-  extern __shared__ __align__(128) uint32_t smem[];
-  uint64_t* bar = reinterpret_cast<uint64_t*>(smem);
-  uint32_t* img = smem + 4;  // 16 B after the barrier
-  const int warps = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    mbar_init(bar, 1);
-    mbar_fence_init();
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    uint32_t bytes = (uint32_t)dm.image_words * 4u;
-    mbar_expect_tx(bar, bytes);
-    bulk_g2s(img, image, bytes, bar);
-  }
-  float* scratch = reinterpret_cast<float*>(img + dm.image_words) + (size_t)warp * (dm.env_words + 4 * ((dm.nprobe + 3) & ~3));
-  float* probe = scratch + dm.env_words;
-  Ctx c{&dm, img, scratch, lane, probe, 0};
-#if defined(MJB_PHASE_PROF)
-  long long t_last = clock64();
-  c.t_last = &t_last;
-#endif
-  // Lock-step rounds: every env-warp of the CTA takes one env per round, so the warps walk through the (large) step
-  // code together and share instruction-cache lines (measured 2x at 65536 envs against a grid-wide work counter).
-  // The physics step re-aligns the busy env-warps right after the Newton solve (step_kernel.cuh, forward): they leave
-  // it together and stay together through the tail of the step and the head of the next env, so there is no barrier
-  // at the round boundary.  The physics-free step has no alignment point inside and re-aligns at the end of each round.
-  const int stride = gridDim.x * warps;
-  const int pack = PACKED ? dm.pack : 1;
-  const int nvirt = (active + pack - 1) / pack;   // virtual envs: `pack` real envs share a warp (active = envs this launch walks)
-  const int rounds = (nvirt - blockIdx.x * warps + stride - 1) / stride;
-  int env = blockIdx.x * warps + warp;
-  for (int r = 0; r < rounds; r++) {
-    if (PHYS) {
-      int busy = nvirt - (blockIdx.x * warps + r * stride);  // env-warps of this CTA with work in this round
-      // (a masked reset lets warps skip their env, so intra-step alignment is off for it)
-      c.cta_threads = (mask == nullptr ? 32 : 0) * (busy > warps ? warps : (busy < 0 ? 0 : busy));
-    }
-    c.img_bar = r == 0 ? bar : nullptr;
-    if (env < nvirt) run_env<PHYS, PACKED, EXT, PRM>(c, B, env_ids ? env_ids[env] : env + env_base, num_envs, mode, skip_frames, mask);
-    if (r == 0) mbar_wait(bar, 0);   // warps that had nothing to do in the first round (or returned early) have not waited yet
-    if (!PHYS) __syncthreads();
-    MJB_PH(c, PH_BARRIER);
-    env += stride;
-  }
-}
-
-}  // namespace mjb
+#include "spec_jit.h"
 
 struct mjb_batch {
   mjb::PackedModel packed;   // K real envs per warp (K = 1: plain)
@@ -96,6 +32,10 @@ struct mjb_batch {
   int* d_lite_tab = nullptr;   // the tile kernel's index tables (lite_tables())
   mjb::DevModel* d_lite_dm = nullptr;   // ... and its DevModel header, padded to 16 bytes
   mjb_buffers B;
+  // MODE_STEP of the physics step: the kernel compiled for this batch's shape (spec_jit.h), null: the generic k_env
+  cudaKernel_t spec_kern = nullptr;
+  std::string spec_why;      // why there is none
+  double spec_ms = 0;        // NVRTC compile time of this shape (once per process: later batches find it in the cache)
   int num_envs = 0, device = 0, warps = 0, grid = 0;
   size_t smem_bytes = 0;
   cudaStream_t stream = nullptr;
@@ -173,8 +113,17 @@ int launch(mjb_batch* b, int mode, int skip_frames, const uint8_t* mask, cudaStr
                     : (b->img.dm.pack > 1 ? mjb::k_env<true, true> : mjb::k_env<true, false>);
     const int pack = b->img.dm.pack;
     const int need = ((active + pack - 1) / pack + b->warps - 1) / b->warps;
-    kern<<<std::min(b->grid, std::max(1, need)), b->warps * 32, b->smem_bytes, stream>>>(
-        b->img.dm, b->d_image, B, b->num_envs, mode, skip_frames, mask, b->subset, active, base / pack);
+    const int grid = std::min(b->grid, std::max(1, need)), env_base = base / pack;
+    if (mode == mjb::MODE_STEP && b->spec_kern) {
+      // the same instantiation as `kern`, compiled for this shape (the generic kernels give the same bits: spec_jit.h)
+      const int* env_ids = b->subset;
+      void* args[] = {(void*)&b->img.dm, (void*)&b->d_image, (void*)&B, (void*)&b->num_envs, (void*)&mode, (void*)&skip_frames,
+                      (void*)&mask, (void*)&env_ids, (void*)&active, (void*)&env_base};
+      CUDA_TRY(cudaLaunchKernel((const void*)b->spec_kern, dim3(grid), dim3(b->warps * 32), args, b->smem_bytes, stream));
+    } else {
+      kern<<<grid, b->warps * 32, b->smem_bytes, stream>>>(b->img.dm, b->d_image, B, b->num_envs, mode, skip_frames, mask, b->subset,
+                                                           active, env_base);
+    }
   }
   CUDA_TRY(cudaGetLastError());
   if (b->timing) {
@@ -305,6 +254,13 @@ int mjb_batch_create(const mjb_model* m, const mjb_env_spec* spec, int32_t num_e
     return fail(MJB_ERR_CUDA);
   }
   smem_attr[device] = std::max(smem_attr[device], b->smem_bytes);
+  if (spec->flags & MJB_SPEC_GENERIC) b->spec_why = "MJB_SPEC_GENERIC";
+  else if (spec->skip_frames == 0) b->spec_why = "skip_frames = 0 (the physics-free step)";
+  else {
+    mjb::SpecKernel* sk = mjb::spec_compile(dm);
+    b->spec_kern = mjb::spec_kernel(sk, device, b->smem_bytes, b->spec_why);
+    b->spec_ms = sk->compile_ms;
+  }
   if (spec->skip_frames == 0) {
     try {
       mjb::ModelView mv(m->host.blob.data());
@@ -588,6 +544,35 @@ int mjb_phase_cycles(uint64_t* out, int32_t n) {
   (void)out; (void)n;
   return 0;
 #endif
+}
+
+int mjb_batch_spec_info(const mjb_batch* b, int32_t* specialised, double* compile_ms, char* reason, int32_t reason_len) {
+  if (!b) return MJB_ERR_ARG;
+  if (specialised) *specialised = b->spec_kern ? 1 : 0;
+  if (compile_ms) *compile_ms = b->spec_ms;
+  if (reason && reason_len > 0) snprintf(reason, (size_t)reason_len, "%s", b->spec_why.c_str());
+  return MJB_OK;
+}
+
+int mjb_spec_compile(const mjb_model* m, const mjb_env_spec* spec, int32_t num_envs, double* compile_ms, void* cubin, int64_t* cubin_bytes) {
+  if (!m || !spec || num_envs < 1 || !cubin_bytes) { mjb::set_error("mjb_spec_compile: bad argument"); return MJB_ERR_ARG; }
+  mjb::DevImage img;
+  try {
+    mjb::PackedModel packed;
+    const int K = mjb::choose_pack(m->host, *spec, num_envs);
+    mjb::make_packed(m->host, *spec, K, packed);
+    mjb::ModelView mv(K > 1 ? packed.rep.blob.data() : m->host.blob.data());
+    mjb::build_dev_model(mv, packed.vspec, img, false, K);
+  } catch (const std::exception& e) {
+    mjb::set_error(e.what());
+    return MJB_ERR_LIMIT;
+  }
+  const mjb::SpecKernel* sk = mjb::spec_compile(img.dm);
+  if (!sk->why.empty()) { mjb::set_error("mjb_spec_compile: " + sk->why); return MJB_ERR_CUDA; }
+  if (compile_ms) *compile_ms = sk->compile_ms;
+  if (cubin && *cubin_bytes >= (int64_t)sk->cubin.size()) memcpy(cubin, sk->cubin.data(), sk->cubin.size());
+  *cubin_bytes = (int64_t)sk->cubin.size();
+  return MJB_OK;
 }
 
 /* query of the launch geometry, for bench / docs */

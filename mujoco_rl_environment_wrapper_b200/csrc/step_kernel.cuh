@@ -80,7 +80,7 @@ MJB_DEV q4 axisangle(f3 ax, float ang) {
 
 // ---- kernel context ----------------------------------------------------------------------------
 struct Ctx {
-  const DevModel* dm;
+  const DM* dm;
   const uint32_t* img;  // constant image (shared memory)
   float* s;             // this env's scratch (shared memory)
   int lane;
@@ -108,11 +108,18 @@ __device__ __forceinline__ void mjb_phase(long long* t_last, int lane, int id) {
 #define MJB_PH(c, id) ((void)0)
 #define MJB_COUNT(c, slot, n) ((void)0)
 #endif
-#define CI(f) ((const int*)(c.img + c.dm->off[IF_##f]))
-#define CU(f) ((const uint32_t*)(c.img + c.dm->off[IF_##f]))
-#define CF(f) ((const float*)(c.img + c.dm->off[IF_##f]))
-#define SF(f) (c.s + c.dm->soff[SF_##f])
-#define SI(f) ((int*)(c.s + c.dm->soff[SF_##f]))
+#if defined(MJB_SPEC)
+#define MJB_OFF(f) spec_off[IF_##f]
+#define MJB_SOFF(f) spec_soff[SF_##f]
+#else
+#define MJB_OFF(f) c.dm->off[IF_##f]
+#define MJB_SOFF(f) c.dm->soff[SF_##f]
+#endif
+#define CI(f) ((const int*)(c.img + MJB_OFF(f)))
+#define CU(f) ((const uint32_t*)(c.img + MJB_OFF(f)))
+#define CF(f) ((const float*)(c.img + MJB_OFF(f)))
+#define SF(f) (c.s + MJB_SOFF(f))
+#define SI(f) ((int*)(c.s + MJB_SOFF(f)))
 // a parameter of the per-env table (DESIGN §5e): the env's value in its scratch block under PRM, else the image's
 #define PF(f, blk) (PRM ? c.s + c.dm->prm_soff + (blk) : CF(f))
 
@@ -131,7 +138,7 @@ MJB_DEV void inertia_mul(const float* I, f3 w, f3 v, f3& n, f3& f) {
 // =================================================================================================
 // kinematics: body frames, motion subspaces (about the tree root's origin), inertias, geom frames
 MJB_DEV void fk(const Ctx& c) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const int* level_adr = CI(level_adr);
   float* qpos = SF(qpos);
   float *xpos = SF(xpos), *xquat = SF(xquat), *xmat = SF(xmat), *xipos = SF(xipos), *cdof = SF(cdof);
@@ -242,7 +249,7 @@ MJB_DEV void fk(const Ctx& c) {
 
 // composite rigid body inertias and the joint-space inertia matrix (packed lower triangle)
 MJB_DEV void crb_mass(const Ctx& c) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const int* level_adr = CI(level_adr);
   float *cinert = SF(cinert), *crb = SF(crb), *M = SF(M), *cdof = SF(cdof);
   MJB_NOUNROLL
@@ -289,7 +296,7 @@ MJB_DEV void crb_mass(const Ctx& c) {
 // qfrc_smooth = passive - bias + actuation.  With `with_acc` the pass includes qacc (post-constraint
 // body accelerations for the accelerometer) and only fills cvel / cacc.
 MJB_DEV void rne_pass(const Ctx& c, bool with_acc) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const int* level_adr = CI(level_adr);
   float *cdof = SF(cdof), *cvel = SF(cvel), *cacc = SF(cacc), *qvel = SF(qvel), *qacc = SF(qacc);
   float *cinert = SF(cinert), *cfrc = SF(crb);  // crb is dead after crb_mass: reuse as body force
@@ -373,7 +380,7 @@ MJB_DEV void rne_pass(const Ctx& c, bool with_acc) {
 // for the rows of M and qfrc_smooth.  (fk / crb_mass / rne_pass stay for the renderer and the accelerometer pass.)
 template <bool PRM = false>
 MJB_DEV void kin_forward(const Ctx& c) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const int* level_adr = CI(level_adr);
   float *qpos = SF(qpos), *qvel = SF(qvel);
   float *xpos = SF(xpos), *xquat = SF(xquat), *xmat = SF(xmat), *xipos = SF(xipos), *cdof = SF(cdof);
@@ -533,7 +540,7 @@ MJB_DEV void kin_forward(const Ctx& c) {
 
 template <bool PRM = false>
 MJB_DEV void dyn_backward(const Ctx& c) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const int* level_adr = CI(level_adr);
   float *crb = SF(cinert), *cfrc = SF(crb), *M = SF(M), *cdof = SF(cdof), *qvel = SF(qvel);
   MJB_NOUNROLL
@@ -866,7 +873,7 @@ MJB_DEV void store_contact(const Ctx& c, int idx, const ConOut& o, int pair, flo
 // contacts found for that copy of a packed env (pack == 1: tot[0]) before the per-copy quota of maxcon1 slots
 template <bool PRM = false>
 MJB_DEV int collide(const Ctx& c, int* tot) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const uint32_t* pairs = CU(pair_pack);
   int* cand = SI(cand);
   int ncand = 0;
@@ -1088,7 +1095,7 @@ MJB_DEV float impedance(const float* solimp, float pos, float margin) {
 // rows: [0, 2 nlim) limit slots (lower, upper per limited joint; inactive -> D = 0), then 4 per contact
 template <bool PRM = false>
 MJB_DEV void make_constraints(const Ctx& c, int ncon) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   float *efcD = SF(efcD), *efcAref = SF(efcAref), *qpos = SF(qpos), *qvel = SF(qvel);
   MJB_NOUNROLL
   for (int k = c.lane; k < dm.nlim; k += 32) {
@@ -1414,7 +1421,7 @@ MJB_DEV float factor_solve(const float* A, float* L, int lane, int t0, int t1, i
 
 // jar-like product for every row: out[row] = J_row . x   (limit rows: +-x[dof]; contact rows: pyramid edges)
 MJB_DEV void rows_mul(const Ctx& c, int ncon, const float* x, float* out, const float* sub) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   MJB_NOUNROLL
   for (int k = c.lane; k < dm.nlim; k += 32) {
     float v = x[CI(lim_dof)[k]];
@@ -1454,7 +1461,7 @@ MJB_DEV void rows_mul(const Ctx& c, int ncon, const float* x, float* out, const 
 
 // J' w for a per-row weight vector w (limit rows +-e_dof, contact rows = pyramid edges): the lane's dof component
 MJB_DEV float jt_mul(const Ctx& c, int ncon, int base, int mylim, const float* w) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const float* J = SF(J);
   const float* con = SF(con);
   float out = mylim >= 0 ? w[2 * mylim] - w[2 * mylim + 1] : 0.f;
@@ -1472,7 +1479,7 @@ MJB_DEV float jt_mul(const Ctx& c, int ncon, int base, int mylim, const float* w
 }
 // the same for two weight vectors at once (one pass over the Jacobian)
 MJB_DEV void jt_mul2(const Ctx& c, int ncon, int base, int mylim, const float* w, const float* v, float& ow, float& ov) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const float* J = SF(J);
   const float* con = SF(con);
   ow = mylim >= 0 ? w[2 * mylim] - w[2 * mylim + 1] : 0.f;
@@ -1501,7 +1508,7 @@ MJB_DEV void jt_mul2(const Ctx& c, int ncon, int base, int mylim, const float* w
 // On exit SF_qacc = solution, SF_vecA = qfrc_smooth + J' f (= M a - g: the total force the implicit-damping solve
 // needs), SF_vecB = g, SF_efcJar = J a - aref.  Returns iterations used.
 MJB_DEV int newton(const Ctx& c, int ncon) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const int nv = dm.nv, lane = c.lane;
   const int t0 = CI(dof_t0)[lane], t1 = CI(dof_t1)[lane];
   float *M = SF(M), *H = SF(H), *a = SF(qacc), *sv = SF(vecC);
@@ -1730,7 +1737,7 @@ MJB_DEV float cutoff(const Ctx& c, int i, float x) {
 
 // position-stage sensors (rangefinder, frame axes)
 MJB_DEV void sensors_pos(const Ctx& c) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   float* sens = SF(sens);
   MJB_NOUNROLL
   for (int i = 0; i < dm.nsensor; i++) {
@@ -1764,7 +1771,7 @@ MJB_DEV void sensors_pos(const Ctx& c) {
 
 // acceleration-stage sensors (touch, accelerometer); needs the solved qacc and efcJar
 MJB_DEV void sensors_acc(const Ctx& c, int ncon) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   if (!dm.need_acc_sensors) return;
   float* sens = SF(sens);
   bool did_rne = false;
@@ -1817,7 +1824,7 @@ MJB_DEV void sensors_acc(const Ctx& c, int ncon) {
 // the only window where cvel and the body frames are both live (the broad phase's candidates overwrite cvel, the
 // constraint rows overwrite xquat / xmat).  Velocities as the accelerometer's: cvel is about the tree root's origin.
 MJB_DEV void sensors_frame(const Ctx& c) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   float* sens = SF(sens);
   const float *xpos = SF(xpos), *xquat = SF(xquat), *xmat = SF(xmat), *cvel = SF(cvel);
   MJB_NOUNROLL
@@ -1871,7 +1878,7 @@ MJB_DEV int forward(const Ctx& c, bool sensors, bool probes, int* iters_out, int
     // exported positions belong to the LAST forward pass of the step (what `data.xipos` holds after
     // mj_step): for Euler that is the state before the integration (SURVEY 3.3), for RK4 the fourth stage.
     // Taken now because xipos is recycled by the solver scratch below
-    const DevModel& dm = *c.dm;
+    const DM& dm = *c.dm;
     MJB_NOUNROLL
     for (int p = c.lane; p < dm.nprobe; p += 32) {
       int kind = CI(probe_kind)[p], id = CI(probe_id)[p];
@@ -1922,7 +1929,7 @@ MJB_DEV int forward(const Ctx& c, bool sensors, bool probes, int* iters_out, int
 
 // qpos += h * qvel-like `v` (lane = joint)
 MJB_DEV void integrate_pos(const Ctx& c, float* qpos, const float* v, float h) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   MJB_NOUNROLL
   for (int j = c.lane; j < dm.njnt; j += 32) {
     int qa = CI(jnt_qposadr)[j], da = CI(jnt_dofadr)[j];
@@ -1949,7 +1956,7 @@ MJB_DEV void integrate_pos(const Ctx& c, float* qpos, const float* v, float h) {
 // runs, since a row may hold damping where the model has none.
 template <bool PRM = false>
 MJB_DEV int substep(const Ctx& c, bool sensors, bool integrate, int* iters_out, int* dropped) {
-  const DevModel& dm = *c.dm;
+  const DM& dm = *c.dm;
   const int nv = dm.nv, lane = c.lane;
   float *qpos = SF(qpos), *qvel = SF(qvel), *qacc = SF(qacc);
   const float h = dm.timestep;

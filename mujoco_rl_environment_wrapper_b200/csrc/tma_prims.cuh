@@ -1,6 +1,8 @@
 // tma_prims.cuh — mbarrier + 1-D TMA bulk copy (cp.async.bulk, SASS UBLKCP / SYNCS) helpers shared by the kernels.
 #pragma once
+#if !defined(__CUDACC_RTC__)
 #include <stdint.h>
+#endif
 
 namespace mjb {
 

@@ -4,9 +4,11 @@
 // sync / shuffle) so the device code can be debugged in a container without a GPU.  The emulator
 // is test tooling; the product only ever runs the nvcc build.
 #pragma once
+#if !defined(__CUDACC_RTC__)
 #include <math.h>
 #include <stdint.h>
 #include <string.h>
+#endif
 
 #if defined(MJB_HOST_EMU)
 #include "../../tests/emu/simt_emu.h"
