@@ -172,6 +172,11 @@ typedef struct mjb_env_spec {
    * non-finite ranges, lo > hi, lo < 0 (lo <= 0 for family 0), and a table with skip_frames = 0. */
   float* params;
   float param_lo[4], param_hi[4];
+  /* MJB_SPEC_AUTORESET only (ignored otherwise), optional: device buffer [N, qpos_stride] that receives the qpos row of
+   * every env whose episode mjb_step ends, as the finishing step left it (the state its final_obs row describes), before
+   * the reset overwrites buffers.qpos.  Rows of other envs are not written.  NULL: not written.  mjb_render_ex renders
+   * the last frame of those episodes from it (mjb_render_args.qpos). */
+  float* final_qpos;
 } mjb_env_spec;
 
 /* mjb_env_spec.flags */
@@ -286,6 +291,27 @@ int mjb_set_env_subset(mjb_batch* b, const int32_t* env_ids_dev, int32_t count);
  * Image formation: first geom hit per pixel, two-sided head-light shading of the geom's rgba (render_kernel.cuh);
  * the OpenGL pipeline's lights / materials / shadows are not modelled. */
 int mjb_render(mjb_batch* b, const int32_t* cam_ids, int32_t ncams, int32_t width, int32_t height, uint8_t* rgb_dev);
+/* mjb_render with more channels, another qpos source and an env mask.  All three channels come from the same primary ray
+ * and the same first hit (a geom with alpha 0 is invisible to all three); rows are bottom-up in each:
+ *   rgb          u8 [num_envs, ncams, height, width, 3]: the bytes mjb_render writes
+ *   depth        f32 [num_envs, ncams, height, width]: distance from the camera origin to the hit along the camera's
+ *                optical axis (its -z), in metres (MuJoCo's linearised depth, not the OpenGL z-buffer); 0 where nothing
+ *                is hit
+ *   segmentation i32 [num_envs, ncams, height, width]: MuJoCo geom id of the hit, -1 where nothing is hit
+ * Each output may be NULL (not written), but not all three.  `qpos`: the rows rendered, NULL or buffers.qpos (the current
+ * state) or the batch's mjb_env_spec.final_qpos (the last state of the episodes the last mjb_step ended).  `mask`: u8
+ * [num_envs] device, NULL = all envs; entries of envs whose byte is 0 are not written.  MJB_ERR_ARG: every output NULL,
+ * the camera / size refusals of mjb_render, or any other qpos pointer (final_qpos included when the batch has none). */
+typedef struct mjb_render_args {
+  const int32_t* cam_ids;  /* host array [ncams] */
+  int32_t ncams, width, height;
+  uint8_t* rgb;
+  float* depth;
+  int32_t* segmentation;
+  const float* qpos;
+  const uint8_t* mask;
+} mjb_render_args;
+int mjb_render_ex(mjb_batch* b, const mjb_render_args* args);
 /* launch geometry chosen at creation: CTAs, env-warps per CTA, dynamic shared memory per CTA */
 int mjb_batch_geometry(const mjb_batch* b, int32_t* grid, int32_t* warps_per_cta, int64_t* smem_bytes);
 /* The physics step of mjb_step runs a kernel compiled at mjb_batch_create for the model's shape (sizes, strides and

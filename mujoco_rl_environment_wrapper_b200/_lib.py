@@ -59,6 +59,7 @@ class EnvSpec(ctypes.Structure):
         ("act_low", ctypes.c_float * 64), ("act_high", ctypes.c_float * 64), ("final_obs", ctypes.c_void_p),
         ("start_qpos", ctypes.c_void_p), ("start_qvel", ctypes.c_void_p), ("n_start", ctypes.c_int32),
         ("params", ctypes.c_void_p), ("param_lo", ctypes.c_float * 4), ("param_hi", ctypes.c_float * 4),
+        ("final_qpos", ctypes.c_void_p),
     ]
 
 
@@ -76,6 +77,12 @@ class Buffers(ctypes.Structure):
     _fields_ = [(n, ctypes.c_void_p) for n in
                 ("qpos", "qvel", "ctrl", "warmstart", "sensordata", "probe", "actions", "obs", "reward", "term",
                  "trunc", "timestep", "store_i", "store_f", "ncon", "contact_geom", "contact_dist", "niter", "nreset", "probe_quat", "ncon_dropped")]
+
+
+class RenderArgs(ctypes.Structure):
+    _fields_ = [("cam_ids", ctypes.POINTER(ctypes.c_int32)), ("ncams", ctypes.c_int32), ("width", ctypes.c_int32),
+                ("height", ctypes.c_int32), ("rgb", ctypes.c_void_p), ("depth", ctypes.c_void_p),
+                ("segmentation", ctypes.c_void_p), ("qpos", ctypes.c_void_p), ("mask", ctypes.c_void_p)]
 
 
 _LIB = None
@@ -148,6 +155,7 @@ def load(build_if_missing=True):
     lib.mjb_kernel_time_ms.argtypes = [vp, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(i64)]
     lib.mjb_set_env_subset.argtypes = [vp, vp, ctypes.c_int32]
     lib.mjb_render.argtypes = [vp, ctypes.POINTER(ctypes.c_int32), ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, vp]
+    lib.mjb_render_ex.argtypes = [vp, ctypes.POINTER(RenderArgs)]
     lib.mjb_batch_geometry.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(i32), ctypes.POINTER(i64)]
     lib.mjb_batch_spec_info.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(ctypes.c_double), ctypes.c_char_p, i32]
     lib.mjb_spec_compile.argtypes = [vp, ctypes.POINTER(EnvSpec), i32, ctypes.POINTER(ctypes.c_double), vp, ctypes.POINTER(i64)]

@@ -14,13 +14,15 @@ from . import _lib as L
 
 class Batch:
     def __init__(self, model: "L.Model", spec: "L.EnvSpec", num_envs: int, device=None, keepalive=(), share=None, probe_quat=False,
-                 start_states=None, params=False, param_ranges=None):
+                 start_states=None, params=False, param_ranges=None, final_qpos=False):
         """`share`: another Batch whose tensors this handle steps as well (level variants, see set_subset);
         the two models must produce the same buffer layout.  `start_states`: (qpos [P, nq], qvel [P, nv]) float32 CUDA
         tensors, a pool every reset draws its start state from (include/mjb.h, mjb_env_spec.start_qpos).
         `params`: give every env its own physical parameters, the table `self.params` [N, n_params] (include/mjb.h,
         mjb_env_spec.params), filled with the model's values (or `share`'s table).  `param_ranges`: four (lo, hi) scale
-        ranges, one per family of L.PARAM_FAMILIES: every reset then draws the env's row (MJB_SPEC_RANDOMIZE)."""
+        ranges, one per family of L.PARAM_FAMILIES: every reset then draws the env's row (MJB_SPEC_RANDOMIZE).
+        `final_qpos` (with MJB_SPEC_AUTORESET): keep the qpos row of every episode a step ends in `self.final_qpos`
+        [N, qpos_stride] (include/mjb.h, mjb_env_spec.final_qpos), to render its last frame (render_ex(final=True))."""
         self._lib = L.load()
         if not torch.cuda.is_available():
             raise RuntimeError("mujoco_rl_environment_wrapper_b200: no CUDA device — the step path is CUDA-only "
@@ -57,6 +59,9 @@ class Batch:
             self.final_obs = z((N, max(1, A), lay.obs_stride), f32)
             spec = L.EnvSpec.from_buffer_copy(spec)   # the caller's spec stays as it was
             spec.final_obs = self.final_obs.data_ptr()
+            if final_qpos:
+                self.final_qpos = z((N, lay.qpos_stride), f32)
+                spec.final_qpos = self.final_qpos.data_ptr()
         if start_states is not None:
             qp, qv = (t.to(device=dev, dtype=f32).contiguous() for t in start_states)
             if qp.dim() != 2 or qv.dim() != 2 or qp.shape[0] < 1 or qv.shape[0] != qp.shape[0] or \
@@ -148,6 +153,36 @@ class Batch:
             out = torch.empty((self.num_envs, n, height, width, 3), dtype=torch.uint8, device=self.device)
         ids = (ctypes.c_int32 * n)(*cam_ids)
         L.check(self._lib.mjb_render(self._h, ids, n, int(width), int(height), ctypes.c_void_p(out.data_ptr())), "render")
+        return out
+
+    def render_ex(self, cam_ids, width=64, height=64, rgb=True, depth=False, segmentation=False, final=False, mask=None, out=None):
+        """Images of the listed fixed cameras (include/mjb.h, mjb_render_ex): a dict with the requested channels, rgb u8
+        [N, n, height, width, 3], depth f32 and segmentation i32 [N, n, height, width], all from the same ray and hit.
+        `final`: render the rows of self.final_qpos (the last state of the episodes the last step ended) instead of the
+        current qpos.  `mask` (bool / u8 [N]): only these envs are written.  `out`: a dict of tensors to write into (missing
+        entries are allocated, zero-filled when a mask is given).  Asynchronous on self.stream."""
+        n, N = len(cam_ids), self.num_envs
+        if final and getattr(self, "final_qpos", None) is None:
+            raise Exception("render_ex(final=True) needs a batch created with MJB_SPEC_AUTORESET and final_qpos=True")
+        out = dict(out or {})
+        new = torch.zeros if mask is not None else torch.empty
+        shapes = {"rgb": ((N, n, height, width, 3), torch.uint8), "depth": ((N, n, height, width), torch.float32),
+                  "segmentation": ((N, n, height, width), torch.int32)}
+        for k, on in (("rgb", rgb), ("depth", depth), ("segmentation", segmentation)):
+            if on and k not in out:
+                out[k] = new(shapes[k][0], dtype=shapes[k][1], device=self.device)
+        a = L.RenderArgs()
+        ids = (ctypes.c_int32 * max(1, n))(*cam_ids)
+        a.cam_ids, a.ncams, a.width, a.height = ctypes.cast(ids, ctypes.POINTER(ctypes.c_int32)), n, int(width), int(height)
+        for k in ("rgb", "depth", "segmentation"):
+            if k in out:
+                t = out[k]
+                if tuple(t.shape) != shapes[k][0] or t.dtype != shapes[k][1] or not t.is_contiguous() or t.device != self.device:
+                    raise Exception(f"render_ex: out['{k}'] must be a contiguous {shapes[k][1]} tensor of shape {shapes[k][0]} on {self.device}")
+                setattr(a, k, t.data_ptr())
+        a.qpos = self.final_qpos.data_ptr() if final else None
+        a.mask = self._mask_ptr(mask)
+        L.check(self._lib.mjb_render_ex(self._h, ctypes.byref(a)), "render")
         return out
 
     def physics(self, skip_frames=1):

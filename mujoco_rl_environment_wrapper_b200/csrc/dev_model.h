@@ -176,9 +176,12 @@ struct DevModel {
   int n_params, prm_n;
   int randomize, prm_soff, off_prm_map, off_prm_nominal;
   float prm_lo[4], prm_hi[4];
-  // frame, velocity and joint sensors (DESIGN §5f): 16 bytes, padded like the fields above.  off_sens_obj: image word
-  // offset of one SO_STRIDE record per sensor, present only when ext_sensors is set.
-  int ext_sensors, off_sens_obj, ext_pad[2];
+  // frame, velocity and joint sensors (DESIGN §5f): 8 bytes.  off_sens_obj: image word offset of one SO_STRIDE record per
+  // sensor, present only when ext_sensors is set.
+  int ext_sensors, off_sens_obj;
+  // MJB_SPEC_AUTORESET: [N, qpos_stride] rows of the episodes a step ends (mjb_env_spec.final_qpos), null: not written.
+  // It takes the 8 padding bytes that ended the struct, so the size and every kernel parameter offset stay as they were.
+  float* final_qpos;
 };
 // Object record of a frame / velocity sensor: the kernel body the object rides on (-1: static) and the object's pose in
 // that body's frame (in the world frame when static).  jointpos / jointvel keep their qpos / dof address in sensor_site.

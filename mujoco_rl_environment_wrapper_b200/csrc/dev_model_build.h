@@ -464,6 +464,7 @@ inline void build_dev_model(const ModelView& m, const mjb_env_spec& spec, DevIma
   for (int i = 0; i < spec.n_dynamics; i++) cp(dm.dynamics[i], spec.dynamics[i]);
   dm.autoreset = (spec.flags & MJB_SPEC_AUTORESET) ? 1 : 0;
   dm.final_obs = dm.autoreset ? spec.final_obs : nullptr;
+  dm.final_qpos = dm.autoreset ? spec.final_qpos : nullptr;
   for (int i = 0; i < spec.n_dynamics; i++) {
     const int d = spec.dynamics[i].act_lo;
     if (dm.autoreset && spec.dynamics[i].act_hi > d) {

@@ -638,6 +638,11 @@ pass:
       const size_t o = (size_t)env * A1 * dm.obs_stride;
       MJB_NOUNROLL
       for (int i = lane; i < A1 * dm.obs_stride; i += 32) dm.final_obs[o + i] = B.obs[o + i];
+      // ... and the state it describes (the copy's qpos as stored above; the reset pass has not run yet), for the last frame
+      if (dm.final_qpos) {
+        MJB_NOUNROLL
+        for (int j = lane; j < dm.nq1; j += 32) dm.final_qpos[(size_t)env * dm.qpos_stride + j] = qpos[k * dm.nq1 + j];
+      }
     }
   }
   MJB_PH(c, PH_EPILOGUE);

@@ -477,6 +477,22 @@ int mjb_kernel_time_ms(mjb_batch* b, double* total_ms, int64_t* launches) {
 
 int mjb_render(mjb_batch* b, const int32_t* cam_ids, int32_t ncams, int32_t width, int32_t height, uint8_t* rgb_dev) {
   if (!b || !cam_ids || !rgb_dev) { mjb::set_error("mjb_render: null argument"); return MJB_ERR_ARG; }
+  mjb_render_args a{};
+  a.cam_ids = cam_ids; a.ncams = ncams; a.width = width; a.height = height; a.rgb = rgb_dev;
+  return mjb_render_ex(b, &a);
+}
+
+int mjb_render_ex(mjb_batch* b, const mjb_render_args* args) {
+  if (!b || !args || !args->cam_ids) { mjb::set_error("mjb_render: null argument"); return MJB_ERR_ARG; }
+  const mjb_render_args& a = *args;
+  const int32_t ncams = a.ncams, width = a.width, height = a.height;
+  if (!a.rgb && !a.depth && !a.segmentation) { mjb::set_error("mjb_render_ex: rgb, depth and segmentation are all NULL"); return MJB_ERR_ARG; }
+  const float* qpos = (a.qpos == nullptr || a.qpos == b->B.qpos) ? b->B.qpos : a.qpos;
+  if (qpos != b->B.qpos && (qpos != b->img.dm.final_qpos || !b->img.dm.final_qpos)) {
+    mjb::set_error(b->img.dm.final_qpos ? "mjb_render_ex: qpos must be NULL, buffers.qpos or the batch's spec.final_qpos"
+                                        : "mjb_render_ex: qpos must be NULL or buffers.qpos (the batch has no spec.final_qpos)");
+    return MJB_ERR_ARG;
+  }
   const mjb::RenderHdr& rh = b->rimg.rhdr;
   if (rh.ncam == 0) { mjb::set_error("mjb_render: the model has no <camera>"); return MJB_ERR_ARG; }
   if (ncams < 1 || ncams > RENDER_MAX_CAMS || width < 1 || height < 1 || width > 4096 || height > 4096) {
@@ -486,12 +502,12 @@ int mjb_render(mjb_batch* b, const int32_t* cam_ids, int32_t ncams, int32_t widt
   mjb::RenderCams cams{};
   cams.n = ncams;
   for (int k = 0; k < ncams; k++) {
-    if (cam_ids[k] < 0 || cam_ids[k] >= rh.ncam) { mjb::set_error("mjb_render: camera id out of range"); return MJB_ERR_ARG; }
-    if (b->rimg.render[rh.off_cam + cam_ids[k] * mjb::CAM_STRIDE + mjb::CAM_MODE] != 0) {
+    if (a.cam_ids[k] < 0 || a.cam_ids[k] >= rh.ncam) { mjb::set_error("mjb_render: camera id out of range"); return MJB_ERR_ARG; }
+    if (b->rimg.render[rh.off_cam + a.cam_ids[k] * mjb::CAM_STRIDE + mjb::CAM_MODE] != 0) {
       mjb::set_error("mjb_render: only mode=\"fixed\" cameras can be rendered");
       return MJB_ERR_ARG;
     }
-    cams.id[k] = cam_ids[k];
+    cams.id[k] = a.cam_ids[k];
   }
   CUDA_TRY(cudaSetDevice(b->device));
   const mjb::DevModel& dm = b->rimg.dm;
@@ -502,13 +518,17 @@ int mjb_render(mjb_batch* b, const int32_t* cam_ids, int32_t ncams, int32_t widt
     CUDA_TRY(cudaMalloc(&b->d_rtab, b->rimg.render.size() * 4));
     CUDA_TRY(cudaMemcpy(b->d_rimage, b->rimg.words.data(), b->rimg.words.size() * 4, cudaMemcpyHostToDevice));
     CUDA_TRY(cudaMemcpy(b->d_rtab, b->rimg.render.data(), b->rimg.render.size() * 4, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaFuncSetAttribute(mjb::k_render, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_TRY(cudaFuncSetAttribute(mjb::k_render<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_TRY(cudaFuncSetAttribute(mjb::k_render<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   }
   int sms = 148;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device);
   const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (smem + 1024)));
   const int grid = std::min(b->num_envs, sms * per_sm);
-  mjb::k_render<<<grid, 256, smem, b->stream>>>(dm, b->d_rimage, rh, b->d_rtab, b->B.qpos, b->num_envs, cams, width, height, rgb_dev);
+  // depth or segmentation requested: the instantiation that keeps each pixel's hit (the colour-only one runs without it)
+  auto kern = (a.depth || a.segmentation) ? mjb::k_render<true> : mjb::k_render<false>;
+  kern<<<grid, 256, smem, b->stream>>>(dm, b->d_rimage, rh, b->d_rtab, qpos, a.mask, b->num_envs, cams, width, height, a.rgb, a.depth,
+                                       a.segmentation);
   CUDA_TRY(cudaGetLastError());
   b->launches++;
   return MJB_OK;

@@ -12,6 +12,11 @@
 // broadcast-friendly list in shared memory and culls them per 16 x 8 pixel tile (bounding sphere against the
 // tile's view cone, conservative, so the image is unchanged), then one warp shades one tile: every lane takes
 // 4 neighbouring pixels, walks the tile's short geom list (warp-uniform) and writes three 32-bit words.
+//
+// Depth and segmentation (mjb_render_ex) come from the same ray and the same first hit as the colour: depth is the hit
+// distance along the camera's optical axis (-z), t / |(u, v, -1)| for the ray through image-plane point (u, v), 0 where
+// nothing is hit; segmentation is the hit's geom id, -1 where nothing is hit.  They are a separate instantiation (CH), so
+// the colour-only launch keeps its registers, local arrays and stores.
 #pragma once
 #include "step_kernel.cuh"
 
@@ -86,8 +91,11 @@ MJB_DEV float hit_cosine(int type, const float* size, f3 lp, f3 lv, float t) {
 }
 
 // colours of the first geom along 4 rays that share the origin `o` (unit directions d[4]); geom-outer loop: one
-// geom record load and one local origin serve all four rays.  Packed 0x00BBGGRR each.
-MJB_DEV_NOINLINE void shade_rays4(const float* GL, const uint16_t* list, int nlist, f3 o, const f3* d, uint32_t* col) {
+// geom record load and one local origin serve all four rays.  Packed 0x00BBGGRR each.  CH: also the hit distance along
+// each ray (t_hit) and the hit geom (g_hit, -1: none).
+template <bool CH = false>
+MJB_DEV_NOINLINE void shade_rays4(const float* GL, const uint16_t* list, int nlist, f3 o, const f3* d, uint32_t* col,
+                                  float* t_hit = nullptr, int* g_hit = nullptr) {
   float best[4] = {MJB_BIG, MJB_BIG, MJB_BIG, MJB_BIG};
   int bi[4] = {-1, -1, -1, -1};
   MJB_NOUNROLL
@@ -114,6 +122,7 @@ MJB_DEV_NOINLINE void shade_rays4(const float* GL, const uint16_t* list, int nli
   }
 #pragma unroll
   for (int j = 0; j < 4; j++) {
+    if (CH) { t_hit[j] = best[j]; g_hit[j] = bi[j]; }
     if (bi[j] < 0) { col[j] = 0u; continue; }
     const float* G = GL + bi[j] * GL_STRIDE;
     const int type = __float_as_int(G[GL_TYPE]);
@@ -130,18 +139,25 @@ MJB_DEV_NOINLINE void shade_rays4(const float* GL, const uint16_t* list, int nli
 #define RENDER_TILE_H 8
 #define RENDER_TILE_BATCH 128   // tiles whose geom lists are resident at once
 
-// direction of the ray through image-plane point (fx, fy) in pixels (pixel centres are at +0.5)
-MJB_DEV f3 pixel_dir(const float* cw, float th, float fx, float fy, int width, int height) {
+// direction of the ray through image-plane point (fx, fy) in pixels (pixel centres are at +0.5); `axial`: the cosine of
+// the ray with the optical axis, 1 / |(u, v, -1)| (distance along the ray x axial = depth)
+MJB_DEV f3 pixel_dir(const float* cw, float th, float fx, float fy, int width, int height, float* axial = nullptr) {
   float u = (fx / width * 2.f - 1.f) * th * ((float)width / (float)height), v = (fy / height * 2.f - 1.f) * th;
   f3 dl = mk3(u, v, -1.f);   // camera frame: looks along -z, +y up
-  return mulv(cw + 3, dl * MJB_RSQRT(dot(dl, dl)));
+  const float s = MJB_RSQRT(dot(dl, dl));
+  if (axial) *axial = s;
+  return mulv(cw + 3, dl * s);
 }
 
-// out: u8 [num_envs, cams.n, height, width, 3]
+// out: u8 [num_envs, cams.n, height, width, 3] of the rows qpos_g [num_envs, qpos_stride]; envs whose mask byte is 0 are
+// skipped (mask null: every env).  CH: also depth (f32) and seg (i32) [num_envs, cams.n, height, width]; each of the
+// three outputs may be null then.
+template <bool CH>
 __global__ void __launch_bounds__(256) k_render(const __grid_constant__ DevModel dm, const uint32_t* __restrict__ image,
                                                 const RenderHdr rh, const uint32_t* __restrict__ rtab,
-                                                const float* __restrict__ qpos_g, int num_envs, const RenderCams cams, int width,
-                                                int height, uint8_t* __restrict__ out) {
+                                                const float* __restrict__ qpos_g, const uint8_t* __restrict__ mask, int num_envs,
+                                                const RenderCams cams, int width, int height, uint8_t* __restrict__ out,
+                                                float* __restrict__ depth, int32_t* __restrict__ seg) {
   extern __shared__ __align__(128) uint32_t smem[];
   uint32_t* img = smem;
   float* scratch = reinterpret_cast<float*>(img + dm.image_words);
@@ -159,7 +175,10 @@ __global__ void __launch_bounds__(256) k_render(const __grid_constant__ DevModel
   const int tiles_x = (width + RENDER_TILE_W - 1) / RENDER_TILE_W, tiles_y = (height + RENDER_TILE_H - 1) / RENDER_TILE_H;
   const int tiles_cam = tiles_x * tiles_y, ntiles = tiles_cam * cams.n;
   const bool words = (width & 3) == 0;   // 4-pixel groups never straddle the right edge: 12-byte stores
+  // ... and one 16-byte store each of depth and segmentation
+  const bool quads = CH && words && ((reinterpret_cast<uintptr_t>(depth) | reinterpret_cast<uintptr_t>(seg)) & 15u) == 0;
   for (int env = blockIdx.x; env < num_envs; env += gridDim.x) {
+    if (mask && !mask[env]) continue;   // CTA-uniform
     if (tid < 32) {
       float* qpos = SF(qpos);
       for (int i = lane; i < dm.nq; i += 32) qpos[i] = qpos_g[(size_t)env * dm.qpos_stride + i];
@@ -239,10 +258,29 @@ __global__ void __launch_bounds__(256) k_render(const __grid_constant__ DevModel
         const int nl = L[0];
         uint32_t col[4];
         f3 d[4];
+        float axial[4], t_hit[4];
+        int g_hit[4];
 #pragma unroll
-        for (int j = 0; j < 4; j++) d[j] = pixel_dir(cw, th, ix0 + j + 0.5f, iy + 0.5f, width, height);   // columns past the edge are not stored
-        shade_rays4(GL, L + 1, nl, o, d, col);
-        uint8_t* dst = out + ((((size_t)env * cams.n + k) * height + iy) * width + ix0) * 3;
+        for (int j = 0; j < 4; j++)   // columns past the edge are not stored
+          d[j] = pixel_dir(cw, th, ix0 + j + 0.5f, iy + 0.5f, width, height, CH ? &axial[j] : nullptr);
+        shade_rays4<CH>(GL, L + 1, nl, o, d, col, CH ? t_hit : nullptr, CH ? g_hit : nullptr);
+        const size_t px = (((size_t)env * cams.n + k) * height + iy) * width + ix0;
+        if (CH) {
+          float z[4];
+#pragma unroll
+          for (int j = 0; j < 4; j++) z[j] = g_hit[j] < 0 ? 0.f : t_hit[j] * axial[j];
+          if (quads) {
+            if (depth) *reinterpret_cast<float4*>(depth + px) = make_float4(z[0], z[1], z[2], z[3]);
+            if (seg) *reinterpret_cast<int4*>(seg + px) = make_int4(g_hit[0], g_hit[1], g_hit[2], g_hit[3]);
+          } else {
+            for (int j = 0; j < 4 && ix0 + j < width; j++) {
+              if (depth) depth[px + j] = z[j];
+              if (seg) seg[px + j] = g_hit[j];
+            }
+          }
+          if (!out) continue;
+        }
+        uint8_t* dst = out + px * 3;
         if (words) {  // 12 bytes = three aligned words
           uint32_t* d32 = reinterpret_cast<uint32_t*>(dst);
           d32[0] = col[0] | (col[1] << 24);

@@ -297,7 +297,8 @@ class MuJoCoRL:
             with torch.cuda.device(self.device):
                 lv["batch"] = Batch(self.model, spec, self.num_envs, device=self.device, keepalive=keep,
                                     share=self._levels[0]["batch"] if lid else None, probe_quat=self.export_orientation,
-                                    start_states=self._start_states, params=self._per_env_params, param_ranges=self._param_ranges)
+                                    start_states=self._start_states, params=self._per_env_params, param_ranges=self._param_ranges,
+                                    final_qpos=self.auto_reset and bool(self.agent_cameras))
         self._use_level(0)
         self._spec, self._batch = self._levels[0]["spec"], self._levels[0]["batch"]
         self.params = self.__param_views() if self._per_env_params else None
@@ -686,6 +687,63 @@ class MuJoCoRL:
         if squeeze:
             img = img[:, 0]
         return img if self.num_envs > 1 else img[0].cpu().numpy()
+
+    def get_camera_images(self, cam_object, depth=True, segmentation=True, final=False):
+        """get_camera_data with more channels: a dict with `rgb` (u8 [N, n_cams, H, W, 3]), and on request `depth` (f32
+        [N, n_cams, H, W], metres along the camera's optical axis, 0 where nothing is hit) and `segmentation` (i32
+        [N, n_cams, H, W], MuJoCo geom id, -1 where nothing is hit), all from the same ray and hit (include/mjb.h,
+        mjb_render_ex).  Agents, camera names, squeezing and num_envs = 1 as in get_camera_data.
+
+        `final=True` (needs `autoReset`): the last frame of the episodes the last step() ended, rendered from the state
+        their `final_observation` describes; the images of other envs are zero, and the dict also holds `mask` (bool [N],
+        the last step's `_final_observation`)."""
+        if not self.agent_cameras:
+            raise Exception("get_camera_images needs config 'agentCameras': True")
+        if final and not self.auto_reset:
+            raise Exception("get_camera_images(final=True) needs config 'autoReset': True (without it no step ends an "
+                            "episode inside the kernel, and the last state of every episode is the current one)")
+        w, h = self.sensor_resolution
+        names, squeeze = self.__camera_names(cam_object)
+        ids = [self.__camera_id(n) for n in names]
+        N = self.num_envs
+        chans = dict(rgb=True, depth=bool(depth), segmentation=bool(segmentation))
+        mask = None
+        if final:
+            A = len(self.agents)
+            mask = (self._batch.term[:, A] | self._batch.trunc[:, A]).view(torch.bool).clone()
+        if not ids:
+            shapes = {"rgb": ((N, 0, h, w, 3), torch.uint8), "depth": ((N, 0, h, w), torch.float32),
+                      "segmentation": ((N, 0, h, w), torch.int32)}
+            out = {k: torch.zeros(shapes[k][0], dtype=shapes[k][1], device=self.device) for k, on in chans.items() if on}
+        elif len(self._levels) == 1:
+            out = self._batch.render_ex(ids, w, h, final=final, mask=mask, **chans)
+        else:   # as get_camera_data: each env keeps the geometry / colours of its own level (no autoReset here, so no final)
+            out = self._levels[0]["batch"].render_ex(ids, w, h, **chans)
+            for lid, lv in enumerate(self._levels[1:], 1):
+                sel = self.level_id == lid
+                if bool(sel.any()):
+                    other = lv["batch"].render_ex(ids, w, h, **chans)
+                    for k in out:
+                        out[k][sel] = other[k][sel]
+        if squeeze:
+            out = {k: v[:, 0] for k, v in out.items()}
+        if N == 1:
+            out = {k: v[0].cpu().numpy() for k, v in out.items()}
+        if final:
+            out["mask"] = mask if N > 1 else bool(mask[0].item())
+        return out
+
+    def __camera_names(self, cam_object):
+        """(camera names, squeeze): all cameras of an agent, or one named camera"""
+        if cam_object in self._tables.rgb_sensors:
+            return self._tables.rgb_sensors[cam_object], False
+        return [cam_object], True
+
+    def __camera_id(self, name):
+        cid = self.model.name2id(L.OBJ_CAMERA, name)
+        if cid < 0:
+            raise KeyError(f"Invalid name '{name}'. Valid names: {[n for v in self._tables.rgb_sensors.values() for n in v]}")
+        return cid
 
     def _position(self, name_or_xyz):
         """[N, 3] position: exported probe, constant of a static object, or explicit coordinates"""
