@@ -105,7 +105,7 @@ enum ImageField {
 #define MJB_SMEM_FIELDS(X)                                                                          \
   X(qpos) X(qvel) X(qacc) X(ctrl) X(qfrc) /* state, current accel iterate, smooth force         */ \
   X(xpos) X(xquat) X(xmat) X(xipos)       /* body frames                                         */ \
-  X(cdof) X(cinert) X(crb) X(cvel) X(cacc) /* spatial quantities about the tree root origin      */ \
+  X(cdof) X(cinert) X(cfrc) X(cvel) X(cacc) /* spatial quantities about the tree root origin     */ \
   X(gpos) X(gmat) X(spos) X(smat)         /* dynamic geom / site world frames                    */ \
   X(M) X(H)                               /* joint-space inertia, Newton Hessian / factors       */ \
   X(cand)                                 /* broadphase survivors (pair indices)                 */ \

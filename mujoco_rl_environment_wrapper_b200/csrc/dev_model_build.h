@@ -616,7 +616,7 @@ inline void build_dev_model(const ModelView& m, const mjb_env_spec& spec, DevIma
   const int nv = m.nv;
   sizes[SF_qpos] = m.nq; sizes[SF_qvel] = nv; sizes[SF_qacc] = nv; sizes[SF_ctrl] = std::max(1, m.nu); sizes[SF_qfrc] = nv;
   sizes[SF_xpos] = 3 * nmb; sizes[SF_xquat] = 4 * nmb; sizes[SF_xmat] = 9 * nmb; sizes[SF_xipos] = 3 * nmb;
-  sizes[SF_cdof] = 6 * nv; sizes[SF_cinert] = 10 * nmb; sizes[SF_crb] = 10 * nmb; sizes[SF_cvel] = 6 * nmb; sizes[SF_cacc] = 6 * nmb;
+  sizes[SF_cdof] = 6 * nv; sizes[SF_cinert] = 10 * nmb; sizes[SF_cfrc] = 10 * nmb; sizes[SF_cvel] = 6 * nmb; sizes[SF_cacc] = 6 * nmb;
   sizes[SF_gpos] = 3 * std::max(1, ngdyn); sizes[SF_gmat] = 9 * std::max(1, ngdyn);
   sizes[SF_spos] = 3 * std::max(1, m.nsite); sizes[SF_smat] = 9 * std::max(1, m.nsite);
   const int tri = nv * (nv + 1) / 2;  // packed lower triangle
@@ -639,9 +639,10 @@ inline void build_dev_model(const ModelView& m, const mjb_env_spec& spec, DevIma
       if (i != SF_qpos && i != SF_qvel && i != SF_qacc && i != SF_ctrl && i != SF_qfrc && i != SF_sens && i != SF_J) sizes[i] = 0;
     sizes[SF_J] = plug_words;
   }
-  // lifetime aliasing: the Hessian lives where cinert + crb were (dead once the bias forces are known),
-  // the broad-phase candidate list where cvel + cacc are (dead between the bias pass and the sensors)
-  const bool alias_H = !lite && tri <= r4(sizes[SF_cinert]) + r4(sizes[SF_crb]);
+  // lifetime aliasing: the Hessian lives where cinert + cfrc were (composite inertias and body forces, dead once
+  // dyn_backward has built M and qfrc_smooth), the broad-phase candidate list where cvel + cacc are (dead between the
+  // bias pass and the sensors)
+  const bool alias_H = !lite && tri <= r4(sizes[SF_cinert]) + r4(sizes[SF_cfrc]);
   if (dm.maxcand > r4(sizes[SF_cvel]) + r4(sizes[SF_cacc])) dm.maxcand = std::max(32, r4(sizes[SF_cvel]) + r4(sizes[SF_cacc]) - 4);
   const bool alias_cand = !lite && dm.maxcand <= r4(sizes[SF_cvel]) + r4(sizes[SF_cacc]);
   // without acceleration-stage sensors nothing touches cvel / cacc after the bias pass: the contact

@@ -247,59 +247,13 @@ MJB_DEV void fk(const Ctx& c) {
   MJB_SYNC();
 }
 
-// composite rigid body inertias and the joint-space inertia matrix (packed lower triangle)
-MJB_DEV void crb_mass(const Ctx& c) {
-  const DM& dm = *c.dm;
-  const int* level_adr = CI(level_adr);
-  float *cinert = SF(cinert), *crb = SF(crb), *M = SF(M), *cdof = SF(cdof);
-  MJB_NOUNROLL
-  for (int i = c.lane; i < 10 * dm.nmb; i += 32) crb[i] = cinert[i];
-  MJB_NOUNROLL
-  for (int i = c.lane; i < (dm.nv * (dm.nv + 1)) / 2; i += 32) M[i] = 0.f;
-  MJB_SYNC();
-  MJB_NOUNROLL
-  for (int l = dm.nlevel - 2; l >= 0; l--) {
-    MJB_NOUNROLL
-    for (int b = level_adr[l] + c.lane; b < level_adr[l + 1]; b += 32) {
-      int ca = CI(mb_childadr)[b], ce = CI(mb_childadr)[b + 1];
-      if (ce > ca) {
-        float acc[10];
-#pragma unroll
-        for (int i = 0; i < 10; i++) acc[i] = crb[10 * b + i];
-        MJB_NOUNROLL
-        for (int k = ca; k < ce; k++) {
-          int ch = CI(mb_child)[k];
-#pragma unroll
-          for (int i = 0; i < 10; i++) acc[i] += crb[10 * ch + i];
-        }
-#pragma unroll
-        for (int i = 0; i < 10; i++) crb[10 * b + i] = acc[i];
-      }
-    }
-    MJB_SYNC();
-  }
-  MJB_NOUNROLL
-  for (int i = c.lane; i < dm.nv; i += 32) {
-    int b = CI(dof_mb)[i];
-    f3 n, f;
-    inertia_mul(crb + 10 * b, ld3(cdof + 6 * i), ld3(cdof + 6 * i + 3), n, f);
-    for (int j = i; j >= 0; j = CI(dof_parent)[j]) {
-      float v = dot(ld3(cdof + 6 * j), n) + dot(ld3(cdof + 6 * j + 3), f);
-      if (j == i) v += CF(dof_armature)[i];
-      M[tri(i, j)] = v;  // j is an ancestor dof: j <= i
-    }
-  }
-  MJB_SYNC();
-}
-
-// velocity-dependent bias forces (Coriolis, centrifugal, gravity) by recursive Newton-Euler, then
-// qfrc_smooth = passive - bias + actuation.  With `with_acc` the pass includes qacc (post-constraint
-// body accelerations for the accelerometer) and only fills cvel / cacc.
-MJB_DEV void rne_pass(const Ctx& c, bool with_acc) {
+// accelerometer walk: velocity and acceleration of every body (about the tree root's origin), the outward loop of the
+// recursive Newton-Euler algorithm with the solved qacc added; fills cvel / cacc.  A loop of its own, not kin_forward's:
+// that one takes a root free joint in closed form, which rounds differently from the generic dof loop.
+MJB_DEV void acc_walk(const Ctx& c) {
   const DM& dm = *c.dm;
   const int* level_adr = CI(level_adr);
   float *cdof = SF(cdof), *cvel = SF(cvel), *cacc = SF(cacc), *qvel = SF(qvel), *qacc = SF(qacc);
-  float *cinert = SF(cinert), *cfrc = SF(crb);  // crb is dead after crb_mass: reuse as body force
   MJB_NOUNROLL
   for (int l = 0; l < dm.nlevel; l++) {
     MJB_NOUNROLL
@@ -322,69 +276,31 @@ MJB_DEV void rne_pass(const Ctx& c, bool with_acc) {
           aw = aw + cross(uw, sw) * qd;
           av = av + (cross(uw, sv) + cross(uv, sw)) * qd;
         }
-        if (with_acc) { aw = aw + sw * qacc[d]; av = av + sv * qacc[d]; }
+        aw = aw + sw * qacc[d]; av = av + sv * qacc[d];
         w = w + sw * qd; v = v + sv * qd;
       }
       st3(cvel + 6 * b, w); st3(cvel + 6 * b + 3, v);
       st3(cacc + 6 * b, aw); st3(cacc + 6 * b + 3, av);
-      if (!with_acc) {
-        f3 n1, f1, n2, f2;
-        inertia_mul(cinert + 10 * b, aw, av, n1, f1);
-        inertia_mul(cinert + 10 * b, w, v, n2, f2);
-        // v x* (I v) = [w x n + v x f ; w x f]
-        st3(cfrc + 10 * b, n1 + cross(w, n2) + cross(v, f2));
-        st3(cfrc + 10 * b + 3, f1 + cross(w, f2));
-      }
     }
     MJB_SYNC();
   }
-  if (with_acc) return;
-  MJB_NOUNROLL
-  for (int l = dm.nlevel - 2; l >= 0; l--) {
-    MJB_NOUNROLL
-    for (int b = level_adr[l] + c.lane; b < level_adr[l + 1]; b += 32) {
-      int ca = CI(mb_childadr)[b], ce = CI(mb_childadr)[b + 1];
-      MJB_NOUNROLL
-      for (int k = ca; k < ce; k++) {
-        int ch = CI(mb_child)[k];
-#pragma unroll
-        for (int i = 0; i < 6; i++) cfrc[10 * b + i] += cfrc[10 * ch + i];
-      }
-    }
-    MJB_SYNC();
-  }
-  float *qfrc = SF(qfrc), *ctrl = SF(ctrl);
-  MJB_NOUNROLL
-  for (int d = c.lane; d < dm.nv; d += 32) {
-    int b = CI(dof_mb)[d];
-    float bias = dot(ld3(cdof + 6 * d), ld3(cfrc + 10 * b)) + dot(ld3(cdof + 6 * d + 3), ld3(cfrc + 10 * b + 3));
-    float f = -CF(dof_damping)[d] * qvel[d] - bias;
-    MJB_NOUNROLL
-    for (int k = CI(dof_actadr)[d]; k < CI(dof_actadr)[d] + CI(dof_actnum)[d]; k++) {
-      int u = CI(act_list)[k];
-      const float* ap = CF(act_param) + 4 * u;
-      float cv = ctrl[u];
-      if (ap[1] != 0.f) cv = fminf(ap[3], fmaxf(ap[2], cv));
-      f += ap[0] * cv;
-    }
-    qfrc[d] = f;
-  }
-  MJB_SYNC();
 }
 
 // ---- fused passes of the step proper -------------------------------------------------------------------------------
-// kin_forward = fk + the outward half of rne_pass in ONE walk over the tree levels: per body its frame, motion subspaces
-// (about the tree root's origin), spatial inertia, velocity, bias acceleration and its own inertial force
-// I a + v x* I v.  Composite inertias later accumulate IN PLACE in SF_cinert; SF_crb holds the body forces.
-// dyn_backward = the inward halves of crb_mass and rne_pass in one walk (16 words per body), then one loop over the dofs
-// for the rows of M and qfrc_smooth.  (fk / crb_mass / rne_pass stay for the renderer and the accelerometer pass.)
+// kin_forward = kinematics and the outward half of the recursive Newton-Euler algorithm in ONE walk over the tree
+// levels: per body its frame, motion subspaces (about the tree root's origin), spatial inertia, velocity, bias
+// acceleration and its own inertial force I a + v x* I v; then the dynamic geom and site frames.  Composite inertias
+// later accumulate IN PLACE in SF_cinert; SF_cfrc holds the body forces.
+// dyn_backward = the inward half in one walk (composite inertias and body forces, 16 words per body), then one loop
+// over the dofs for the rows of M and qfrc_smooth.  (fk stays for the renderer: a frames-only instantiation of this walk
+// compiles to frames that round differently in the last bits and so renders different images, DESIGN §5b.)
 template <bool PRM = false>
 MJB_DEV void kin_forward(const Ctx& c) {
   const DM& dm = *c.dm;
   const int* level_adr = CI(level_adr);
   float *qpos = SF(qpos), *qvel = SF(qvel);
   float *xpos = SF(xpos), *xquat = SF(xquat), *xmat = SF(xmat), *xipos = SF(xipos), *cdof = SF(cdof);
-  float *cinert = SF(cinert), *cfrc = SF(crb), *cvel = SF(cvel), *cacc = SF(cacc);
+  float *cinert = SF(cinert), *cfrc = SF(cfrc), *cvel = SF(cvel), *cacc = SF(cacc);
   MJB_NOUNROLL
   for (int l = 0; l < dm.nlevel; l++) {
     MJB_NOUNROLL
@@ -542,7 +458,7 @@ template <bool PRM = false>
 MJB_DEV void dyn_backward(const Ctx& c) {
   const DM& dm = *c.dm;
   const int* level_adr = CI(level_adr);
-  float *crb = SF(cinert), *cfrc = SF(crb), *M = SF(M), *cdof = SF(cdof), *qvel = SF(qvel);
+  float *crb = SF(cinert), *cfrc = SF(cfrc), *M = SF(M), *cdof = SF(cdof), *qvel = SF(qvel);
   MJB_NOUNROLL
   for (int l = dm.nlevel - 2; l >= 0; l--) {
     MJB_NOUNROLL
@@ -1206,18 +1122,6 @@ MJB_DEV void make_constraints(const Ctx& c, int ncon) {
 // dense helpers (nv <= 32: lane = row / dof).  M is block diagonal over kinematic trees and so is the
 // Hessian unless a contact couples two trees, so everything works per block [t0, t1) of the lane and the
 // blocks of different trees proceed in parallel on their own lanes.
-// out = sum_j A(row, j) x[j] over the row's block, A symmetric packed
-MJB_DEV float matvec_row(const float* A, const float* x, int row, int t0, int t1) {
-  float s0 = 0.f, s1 = 0.f;
-  int j = t0;
-  MJB_NOUNROLL
-  for (; j + 1 <= row && j + 1 < t1; j += 2) { s0 += A[tri(row, j)] * x[j]; s1 += A[tri(row, j + 1)] * x[j + 1]; }
-  MJB_NOUNROLL
-  for (; j <= row && j < t1; j++) s0 += A[tri(row, j)] * x[j];
-  MJB_NOUNROLL
-  for (; j < t1; j++) s1 += A[tri(j, row)] * x[j];
-  return s0 + s1;
-}
 // in-place Cholesky of the packed lower triangle, block by block; lane i owns row i.  `nb` = the largest
 // block size (warp-uniform).  Returns 1 / L_ii of the lane's row.
 MJB_DEV float cholesky(float* A, int lane, int t0, int t1, int nb) {
@@ -1774,7 +1678,7 @@ MJB_DEV void sensors_acc(const Ctx& c, int ncon) {
   const DM& dm = *c.dm;
   if (!dm.need_acc_sensors) return;
   float* sens = SF(sens);
-  bool did_rne = false;
+  bool did_acc = false;
   const uint32_t* pairs = CU(pair_pack);
   const int base = 2 * dm.nlim;
   MJB_NOUNROLL
@@ -1803,7 +1707,7 @@ MJB_DEV void sensors_acc(const Ctx& c, int ncon) {
       total = wsum(total);
       if (c.lane == 0) sens[adr] = cutoff(c, i, total);
     } else if (type == MJB_SENS_ACCELEROMETER) {
-      if (!did_rne) { rne_pass(c, true); did_rne = true; }
+      if (!did_acc) { acc_walk(c); did_acc = true; }
       int b = CI(site_mb)[t];
       if (c.lane == 0) {
         f3 acc = mk3(-dm.gravity[0], -dm.gravity[1], -dm.gravity[2]);
